@@ -26,6 +26,12 @@ its own games (weak scaling); there is no collective inside a simulation.
 `roofline`: the fused network kernel (tcgen05), sampled with CUDA events inside the timed region.
 `cpu_baseline`: the restated reference (oracle C search + libtorch-CPU f32 forward, 128 games in lock-step like
            selfplay/src/main.rs:37) on this box's host cores, bounded sample.
+
+--dump-outputs DIR writes what the last timed step of the `value` leg computed as DIR/<name>.npy (float32, float64 for
+integers wider than 16 bits, so every value is exact), rank 0's games only, for comparing two builds output for output: after a
+self-play move the games' new positions and the children of their new roots (the subtree the search grew), after a
+reanalyze batch the targets tz_reanalyze_read returns.  Per-game arrays keep a fixed, seeded sample of DUMP_GAMES games
+(`games.npy` lists them); the inputs are seeded, so the same arguments give the same inputs on every run.
 """
 from __future__ import annotations
 
@@ -143,6 +149,67 @@ def workload_config(wl: dict, name: str, n_gpus: int) -> dict:
         cfg["sharding"] = (f"buffer positions sharded over {n_gpus} GPU(s) by contiguous index range, "
                            f"no data-path collective")
     return cfg
+
+
+# ---------------------------------------------------------------------------------------- --dump-outputs
+
+DUMP_GAMES = 1024  # at a move stride of 1024 this keeps a dump near 40 MB
+DUMP_LIMIT = 64 << 20
+
+
+def dump_games(G: int):
+    """The games a dump keeps: all of them up to DUMP_GAMES, else the same seeded sample on every run."""
+    import numpy as np
+
+    if G <= DUMP_GAMES:
+        return np.arange(G)
+    return np.sort(np.random.default_rng(0).choice(G, size=DUMP_GAMES, replace=False))
+
+
+def write_dump(directory: str, arrays: dict) -> None:
+    """DIR/<name>.npy per array: floats as float32, integers as float32 when they have at most 16 bits (exact) and as
+    float64 otherwise (exact up to 32 bits; 64-bit words are split into 32-bit halves before they get here)."""
+    import numpy as np
+
+    out = {}
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        wide = a.dtype.kind in "iu" and a.dtype.itemsize > 2
+        out[name] = np.ascontiguousarray(a, dtype=np.float64 if wide else np.float32)
+    total = sum(a.nbytes for a in out.values())
+    if total > DUMP_LIMIT:
+        raise SystemExit(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT}-byte limit")
+    os.makedirs(directory, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(directory, f"{name}.npy"), a)
+
+
+def selfplay_outputs(m, rows) -> dict:
+    """After tz_selfplay_move: the new positions (tz_get_positions) and the children of the new roots
+    (tz_root_children), rows `rows`."""
+    import numpy as np
+
+    pos = m.positions()[rows]
+    out = {"games": rows}
+    # the 64-bit stack words as (low, high) 32-bit halves: exact in float64
+    out["position_stack"] = np.ascontiguousarray(pos["stack"]).view(np.uint32)
+    for f in ("height", "top", "to_move", "stones", "caps", "ply", "reversible_plies"):
+        out[f"position_{f}"] = pos[f]
+    tbl = m.root_children()
+    tag, bits = tbl["eval_tag"][rows], tbl["eval_bits"][rows]
+    out["root_n"] = tbl["n"][rows]
+    for f in ("moves", "visits", "logit", "prob", "std_dev"):
+        out[f"root_{f}"] = tbl[f][rows]
+    out["root_eval_tag"] = tag
+    # a VALUE evaluation holds an f32, a solved one (win / loss / draw) the ply count (exact in f32)
+    out["root_eval"] = np.where(tag == 0, bits.view(np.float32), bits.astype(np.float32))
+    return out
+
+
+def reanalyze_outputs(m, rows) -> dict:
+    """After tz_reanalyze_batch: the targets tz_reanalyze_read returns, rows `rows`."""
+    t = m.reanalyze_read()
+    return {"games": rows, **{f"target_{k}": v[rows] for k, v in t.items()}}
 
 
 # ---------------------------------------------------------------------------------- restated reference (CPU)
@@ -377,6 +444,8 @@ def run_selfplay(args, wl, emit):
     clocks.start()
     every = timed_selfplay(run, params, args.steps, 1, profile=True)
     clock_info = clocks.stop()
+    if args.dump_outputs and run.rank == 0:
+        write_dump(args.dump_outputs, selfplay_outputs(m, dump_games(G)))
     # the same with ONE generation in the region (the amortised cadence: a new model every >= --steps moves) and none
     fresh_games()
     sparse = timed_selfplay(run, params, args.steps, args.steps, profile=False)
@@ -545,6 +614,8 @@ def run_reanalyze(args, wl, emit):
     if m.status():
         raise SystemExit(f"device search error bits 0x{m.status():x} during the timed region")
     c1 = m.counters()
+    if args.dump_outputs and run.rank == 0:
+        write_dump(args.dump_outputs, reanalyze_outputs(m, dump_games(G)))
     (ms,), (sims, evals, known, targets, launches) = run.reduce(
         [ms], [c1.simulations - c0.simulations, c1.evaluations - c0.evaluations, c1.known - c0.known, G * args.steps,
                m.launch_count() - l0])
@@ -617,7 +688,13 @@ def main():
     ap.add_argument("--workload", default="6x6_selfplay", choices=sorted(WORKLOADS))
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's outputs as DIR/<name>.npy (see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the CUDA library's outputs: it needs --impl ours")
     wl = WORKLOADS[args.workload]
     # stdout carries exactly ONE line, the JSON result: anything a library prints on the way (NCCL's version
     # banner, torchrun notices) goes to stderr
