@@ -8,7 +8,7 @@ import pytest
 from oracle import oracle as O
 from takzero_b200 import capi
 
-from helpers import games_to_states, host_agent_from_oracle, oracle_children
+from helpers import assert_tree_equal, games_to_states, host_agent_from_oracle
 
 pytestmark = pytest.mark.gpu
 
@@ -18,21 +18,6 @@ def _device_matching_math():
     O.lib().tk_set_exact_math(1)
     yield
     O.lib().tk_set_exact_math(0)
-
-
-def assert_tree_equal(m, tree, what):
-    node = tree.node
-    st = m.root_stats()[0]
-    tbl = m.root_children()
-    assert st["n_children"] == node.n_children, what
-    assert st["visit_count"] == node.visit_count, what
-    assert (st["eval_tag"], st["eval_bits"]) == (node.evaluation.tag, node.evaluation.u.ply), what
-    oc = oracle_children(node)
-    n = node.n_children
-    for key in ("moves", "visits", "eval_tag", "eval_bits"):
-        assert np.array_equal(tbl[key][0, :n], oc[key]), f"{what}: {key}"
-    for key in ("logit", "prob", "std_dev"):
-        assert np.array_equal(tbl[key][0, :n].view(np.uint32), oc[key].view(np.uint32)), f"{what}: {key}"
 
 
 def oracle_pv(tree):

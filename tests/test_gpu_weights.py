@@ -9,40 +9,9 @@ from oracle import net_ref
 from oracle import oracle as O
 from takzero_b200 import capi, network
 
-from helpers import games_to_states
+from helpers import folded_layer, games_to_states
 
 pytestmark = pytest.mark.gpu
-
-FILTERS = 256
-
-
-def to_bf16_bits(x: np.ndarray) -> np.ndarray:
-    u = x.astype(np.float32).view(np.uint32)
-    return ((u + np.uint32(0x7FFF) + ((u >> np.uint32(16)) & np.uint32(1))) >> np.uint32(16)).astype(np.uint16)
-
-
-def folded_layer(w, bn, conv_bias, cin_pad, f16):
-    """The host restatement: conv [cout][cin][3][3] (+ BN, eval mode, eps 1e-5) -> the 16-bit blocks
-    [cin_pad/64][9 taps, centre first][2 halves][8 k-chunks][128 n][8] and 256 f32 biases."""
-    cout, cin = w.shape[:2]
-    one, eps = np.float32(1.0), np.float32(1e-5)
-    scale = np.ones(cout, np.float32)
-    bias = np.zeros(FILTERS, np.float32)
-    if bn is not None:
-        bw, bb, bm, bv = bn
-        scale = (bw * (one / np.sqrt(bv + eps, dtype=np.float32))).astype(np.float32)
-        bias[:cout] = bb - bm * scale
-    if conv_bias is not None:
-        bias[:cout] = bias[:cout] + conv_bias * scale
-    full = np.zeros((FILTERS, cin_pad, 9), np.float32)
-    full[:cout, :cin] = (w.reshape(cout, cin, 9) * scale[:, None, None]).astype(np.float32)
-    taps = [4, 0, 1, 2, 3, 5, 6, 7, 8]
-    blk = full[:, :, taps]                                  # [co][ci][ti]
-    blk = blk.reshape(2, 128, cin_pad // 64, 8, 8, 9)        # [half][nrow][kb][kc][e][ti]
-    blk = blk.transpose(2, 5, 0, 3, 1, 4)                    # [kb][ti][half][kc][nrow][e]
-    flat = np.ascontiguousarray(blk).reshape(-1)
-    bits = flat.astype(np.float16).view(np.uint16) if f16 else to_bf16_bits(flat)
-    return bits, bias
 
 
 @pytest.mark.parametrize("dtype", [network.DTYPE_F16, network.DTYPE_BF16])
