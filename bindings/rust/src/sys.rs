@@ -28,6 +28,7 @@ pub const TZ_STATUS_SET_EMPTY: u32 = 64;
 pub const TZ_STATUS_REPLAY_FULL: u32 = 128;
 pub const TZ_STATUS_NETWORK_STALL: u32 = 256;
 pub const TZ_STATUS_WEIGHTS_MISMATCH: u32 = 512;
+pub const TZ_STATUS_TARGETS_FULL: u32 = 1024;
 pub const TZ_AGENT_SYNTHETIC: u32 = 0;
 pub const TZ_AGENT_HOST: u32 = 1;
 pub const TZ_AGENT_NETWORK: u32 = 2;
@@ -102,6 +103,35 @@ pub struct tz_selfplay_t {
 }
 #[repr(C)]
 #[derive(Clone, Copy)]
+pub struct tz_selfplay_data_t {
+    pub target_cap: usize,
+    pub policy_cap: usize,
+    pub replay_cap: usize,
+    pub move_cap: usize,
+    pub target_env: *mut tz_state_t,
+    pub target_value: *mut f32,
+    pub target_ube: *mut f32,
+    pub target_n: *mut c_int,
+    pub target_offset: *mut u64,
+    pub target_game: *mut c_int,
+    pub policy_moves: *mut tz_move_t,
+    pub policy_probs: *mut f32,
+    pub replay_start: *mut tz_state_t,
+    pub replay_result: *mut c_int,
+    pub replay_terminal: *mut c_int,
+    pub replay_length: *mut c_int,
+    pub replay_offset: *mut u64,
+    pub replay_game: *mut c_int,
+    pub replay_exploration: *mut u8,
+    pub replay_moves: *mut tz_move_t,
+    pub n_targets: usize,
+    pub n_policy: usize,
+    pub n_replays: usize,
+    pub n_moves: usize,
+    pub high_water_bytes: usize,
+}
+#[repr(C)]
+#[derive(Clone, Copy)]
 pub struct tz_reanalyze_t {
     pub sampled_actions: c_int,
     pub search_budget: u32,
@@ -157,6 +187,8 @@ extern "C" {
     pub fn tz_set_root_priors(h: *mut tz_handle, stride: c_int, prob: *const f32, logit: *const f32) -> c_int;
     pub fn tz_selfplay_move(h: *mut tz_handle, params: *const tz_selfplay_t) -> c_int;
     pub fn tz_launch_count(h: *mut tz_handle, out: *mut u64) -> c_int;
+    pub fn tz_selfplay_record(h: *mut tz_handle, enable: c_int, bytes_per_game: usize, output_bytes: usize) -> c_int;
+    pub fn tz_selfplay_read(h: *mut tz_handle, io: *mut tz_selfplay_data_t) -> c_int;
     pub fn tz_stage_positions(h: *mut tz_handle, states: *const tz_state_t, count: usize) -> c_int;
     pub fn tz_reanalyze_batch(h: *mut tz_handle, pool_indices: *const u32, params: *const tz_reanalyze_t) -> c_int;
     pub fn tz_reanalyze_read(h: *mut tz_handle, stride: c_int, out_policy: *mut f32, out_ube: *mut f32, out_value: *mut f32, out_n: *mut c_int, out_moves: *mut tz_move_t) -> c_int;

@@ -11,6 +11,11 @@
 // `buffer_lengths.txt` throttle with its checksum (main.rs:93-104,371-387) is honoured when that file exists;
 // the loop stops after --moves iterations.  Several GPUs: one process per GPU with `--device d --game-base d*games`,
 // all appending to the same files like the reference's independent processes (README.md:128-130).
+//
+// --resident runs the same loop with tz_selfplay_move and the library's on-device training-data records
+// (tz_selfplay_record / tz_selfplay_read): one asynchronous call per move instead of five blocking ones and no
+// full-stride target table on the host; the text of one move is formatted while the device searches the next.
+// Both modes write byte-identical files.  --record-bytes sets the record region per game (0: the library default).
 #include <chrono>
 #include <cstdio>
 #include <cstdlib>
@@ -41,7 +46,9 @@ struct Args {
     unsigned long long seed = 1;
     float beta = 0.25f;
     bool exploration = false;
+    bool resident = false;
     unsigned arena_slots = 0;
+    unsigned long long record_bytes = 0;
 };
 
 static Args parse(int argc, char** argv) {
@@ -69,6 +76,8 @@ static Args parse(int argc, char** argv) {
         else if (k == "--seed") a.seed = std::strtoull(val(), nullptr, 10);
         else if (k == "--arena-slots") a.arena_slots = (unsigned)std::atoi(val());
         else if (k == "--exploration") a.exploration = true;
+        else if (k == "--resident") a.resident = true;
+        else if (k == "--record-bytes") a.record_bytes = std::strtoull(val(), nullptr, 10);
         else {
             std::fprintf(stderr, "unknown flag %s\n", k.c_str());
             std::exit(2);
@@ -116,16 +125,75 @@ int main(int argc, char** argv) {
         while ((2u << log_sampled) <= (unsigned)args.sampled_actions) log_sampled++;
         const unsigned visitations = args.budget / log_sampled / (unsigned)args.sampled_actions * ((1u << log_sampled) - 1);
 
-        std::vector<std::vector<IncompleteTarget>> policy_targets(G);
-        std::vector<tz_state_t> cur = mcts.envs();
-        for (int step = 0; step < args.moves; step++) {
-            // wait while the trainer's exploitation buffer is full (main.rs:93-104)
+        // wait while the trainer's exploitation buffer is full (main.rs:93-104)
+        auto throttle = [&]() {
             for (;;) {
                 const BufferLengths lengths = read_buffer_lengths(args.directory);
                 if (lengths.status == -1 || (lengths.status == 0 && lengths.selfplay <= MAX_SELFPLAY_BUFFER_LEN)) break;
                 if (lengths.status == -2) std::fprintf(stderr, "Could not read buffer lengths: wrong checksum or missing component\n");
                 std::this_thread::sleep_for(std::chrono::seconds(1));
             }
+        };
+
+        if (args.resident) {
+            mcts.selfplay_record(true, (size_t)args.record_bytes);
+            tz_selfplay_t sp{};
+            sp.sampled_actions = args.sampled_actions;
+            sp.search_budget = args.budget;
+            sp.beta = args.exploration ? args.beta : 0.0f;
+            sp.weighted_random_plies = args.weighted_random_plies;
+            sp.sample_threshold = 32;
+            sp.allowed_eval_drop = 0.5f;
+            sp.target_visitations = (float)visitations;
+            sp.target_beta = args.beta;
+            sp.seed = args.seed;
+            bool warned_full = false;
+            // restart_envs_and_complete_targets' file output (main.rs:263-329) of one move's data
+            auto write = [&](const BatchedMCTS::SelfplayData& data) {
+                std::string targets_txt, replays_txt, exploration_txt;
+                for (const BatchedMCTS::FinishedGame& f : data.games) {
+                    if (args.exploration && f.exploration) {
+                        Replay head = f.replay;
+                        if ((int)head.actions.size() > args.weighted_random_plies) head.actions.resize(args.weighted_random_plies);
+                        exploration_txt += head.to_string(n, head.actions.size() == f.replay.actions.size() ? f.result : 0);
+                    }
+                    replays_txt += f.replay.to_string(n, f.result);
+                }
+                for (const Target& t : data.targets) targets_txt += t.to_string(n);
+                if (!targets_txt.empty()) append(args.directory + "/targets-selfplay.txt", targets_txt);
+                if (!replays_txt.empty()) append(args.directory + "/replays.txt", replays_txt);
+                if (!exploration_txt.empty()) append(args.directory + "/replays-exploration.txt", exploration_txt);
+            };
+            BatchedMCTS::SelfplayData prev;
+            bool have_prev = false;
+            for (int step = 0; step < args.moves; step++) {
+                throttle();
+                reload_model();
+                mcts.selfplay_move(sp);
+                if (have_prev) write(prev);  // formatted while the device searches this move
+                prev = mcts.selfplay_read();
+                have_prev = true;
+                uint32_t bits = 0;
+                check(tz_status(mcts.handle(), &bits));
+                if (bits & TZ_STATUS_TARGETS_FULL) {
+                    if (!warned_full)
+                        std::fprintf(stderr, "selfplay: training data dropped (record region or queue full, high-water "
+                                             "mark %zu bytes per game); raise --record-bytes\n", prev.high_water_bytes);
+                    warned_full = true;
+                    check(tz_clear_status(mcts.handle()));
+                }
+            }
+            if (have_prev) write(prev);
+            const tz_counters_t c = mcts.counters();
+            std::printf("selfplay: %d moves of %d games, %llu simulations, %llu evaluations\n", args.moves, G,
+                        (unsigned long long)c.simulations, (unsigned long long)c.evaluations);
+            return 0;
+        }
+
+        std::vector<std::vector<IncompleteTarget>> policy_targets(G);
+        std::vector<tz_state_t> cur = mcts.envs();
+        for (int step = 0; step < args.moves; step++) {
+            throttle();
             reload_model();
             std::vector<Move> selected =
                 mcts.gumbel_sequential_halving(betas, args.sampled_actions, args.budget, args.seed);

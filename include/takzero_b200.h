@@ -55,6 +55,9 @@ enum {
                                       tile (never seen; the watchdog turns a would-be hang into this error) */
     TZ_STATUS_WEIGHTS_MISMATCH = 512, /* a broadcast weight set describes another network (board size, residual
                                          blocks or 16-bit type differ between the ranks) */
+    TZ_STATUS_TARGETS_FULL = 1024, /* resident self-play recording ran out of room: a game's record region (its
+                                      recorded prefix is still emitted) or the output queue (whole games that do not
+                                      fit are dropped); the search is not affected.  See tz_selfplay_record. */
 };
 
 /* Move (takparse `Move`, 2 bytes):
@@ -218,6 +221,60 @@ typedef struct tz_selfplay_t {
 } tz_selfplay_t;
 TZ_API int tz_selfplay_move(tz_handle* h, const tz_selfplay_t* params);
 TZ_API int tz_launch_count(tz_handle* h, uint64_t* out);             /* kernels launched so far */
+
+/* Training data of tz_selfplay_move, kept on the device (take_a_step + restart_envs_and_complete_targets,
+ * selfplay/src/main.rs:238-329).  With recording on, every tz_selfplay_move appends one pending record per game (root
+ * position, replay index, improved policy in child order, UBE target) to the game's region of `bytes_per_game` bytes
+ * (a record takes 400 + 6 * children bytes, rounded up to 16), and when a game ends it emits, into the output queue,
+ * the game's replay and its targets from the last ply to the first with the value completed from the result
+ * (exploration half, beta != 0 and game < n_games / 2: only plies > weighted_random_plies).  Finished games come in
+ * ascending game order; the order does not depend on timing.
+ *   bytes_per_game 0: a quarter of the free HBM divided among the games, at least 64 KiB and at most the worst case
+ *     TZ_MAX_PLIES * (400 + 6 * move_stride); tz_selfplay_read reports the most any game has used.
+ *   output_bytes 0: half the size of all regions, at most an eighth of the free HBM, at least 16 MiB.  The queue is
+ *     split: 1/16 replays, 1/16 replay moves, the rest targets and policy entries sized for a mean of move_stride / 4
+ *     children per target.
+ * A full region stops that game's recording (its prefix is still emitted with correct values); whole games that do
+ * not fit the queue are dropped; both raise TZ_STATUS_TARGETS_FULL and never disturb the search.  Pending records
+ * belong to consecutive tz_selfplay_move calls: tz_step, tz_restart_terminal, tz_new_openings, tz_set_positions,
+ * tz_random_steps, tz_reset_roots, tz_reanalyze_batch with indices and the tz_tree_* calls drop them at the next
+ * recording move.  enable = 0 frees everything; enabling again starts empty.  Recording off (the default) leaves
+ * tz_selfplay_move's launches exactly as they are. */
+TZ_API int tz_selfplay_record(tz_handle* h, int enable, size_t bytes_per_game, size_t output_bytes);
+
+/* Caller buffers of tz_selfplay_read.  The caller sets the four capacities (entries) and any of the pointers (NULL
+ * skips that field); the call sets the counts. */
+typedef struct tz_selfplay_data_t {
+    size_t target_cap;
+    size_t policy_cap;
+    size_t replay_cap;
+    size_t move_cap;
+    tz_state_t* target_env;       /* [targets] position before the move */
+    float* target_value;          /* [targets] value target */
+    float* target_ube;            /* [targets] UBE target */
+    int* target_n;                /* [targets] policy entries */
+    uint64_t* target_offset;      /* [targets] first entry in policy_moves / policy_probs */
+    int* target_game;             /* [targets] global game id (game_base + game) */
+    tz_move_t* policy_moves;      /* [policy] */
+    float* policy_probs;          /* [policy] improved policy */
+    tz_state_t* replay_start;     /* [replays] start position */
+    int* replay_result;           /* [replays] tz_game_result code of the final position */
+    int* replay_terminal;         /* [replays] tz_result code of the final position */
+    int* replay_length;           /* [replays] moves */
+    uint64_t* replay_offset;      /* [replays] first move in replay_moves */
+    int* replay_game;             /* [replays] global game id */
+    uint8_t* replay_exploration;  /* [replays] 1 for the exploration half */
+    tz_move_t* replay_moves;      /* [moves] */
+    size_t n_targets;             /* out: entries returned, or needed when a capacity is too small */
+    size_t n_policy;
+    size_t n_replays;
+    size_t n_moves;
+    size_t high_water_bytes;      /* out: most bytes one game's region has held since tz_selfplay_record */
+} tz_selfplay_data_t;
+/* Waits for the handle's stream, copies the queue out (cudaMemcpyAsync on the handle's stream) and empties it.  A
+ * capacity below its count returns TZ_EINVAL with the counts set and consumes nothing; TZ_ESEARCH on a device search
+ * error (TZ_STATUS_TARGETS_FULL is not one). */
+TZ_API int tz_selfplay_read(tz_handle* h, tz_selfplay_data_t* io);
 
 /* The loop body of `reanalyze` (reanalyze/src/main.rs:147-235) without per-batch host buffers.  tz_stage_positions
  * uploads the positions of the replay buffer once (position_buffer, main.rs:60-75); tz_reanalyze_batch makes the

@@ -513,6 +513,84 @@ class BatchedMCTS {
         check(tz_reanalyze_read(h_, stride_, t.policy.data(), t.ube.data(), t.value.data(), t.n.data(), t.moves.data()));
         return t;
     }
+    // ---- resident self-play (selfplay/src/main.rs:138-153,238-329 on the device) ----------------------------------------
+    // one whole move of every game, asynchronous; with recording on, its training data stays on the device
+    void selfplay_move(const tz_selfplay_t& params) { check(tz_selfplay_move(h_, &params)); }
+    void selfplay_record(bool enable, size_t bytes_per_game = 0, size_t output_bytes = 0) {
+        check(tz_selfplay_record(h_, enable ? 1 : 0, bytes_per_game, output_bytes));
+    }
+    struct FinishedGame {
+        Replay replay;
+        int result = 0;     // tz_game_result code of the final position
+        int terminal = 0;   // tz_result code of the final position
+        int game = 0;       // global game id
+        bool exploration = false;
+    };
+    struct SelfplayData {
+        std::vector<Target> targets;  // finished games in ascending order, each from its last ply to its first
+        std::vector<int> target_games;
+        std::vector<FinishedGame> games;
+        size_t high_water_bytes = 0;
+    };
+    // completed targets and finished replays since the last read (waits for the device, empties the queue)
+    SelfplayData selfplay_read() {
+        tz_selfplay_data_t io{};
+        const int rc = tz_selfplay_read(h_, &io);  // capacities 0: the counts
+        if (rc != TZ_EINVAL || (io.n_targets | io.n_policy | io.n_replays | io.n_moves) == 0) check(rc);
+        std::vector<tz_state_t> t_env(io.n_targets), r_start(io.n_replays);
+        std::vector<float> t_value(io.n_targets), t_ube(io.n_targets), probs(io.n_policy);
+        std::vector<int> t_n(io.n_targets), t_game(io.n_targets), r_result(io.n_replays), r_term(io.n_replays),
+            r_len(io.n_replays), r_game(io.n_replays);
+        std::vector<uint64_t> t_off(io.n_targets), r_off(io.n_replays);
+        std::vector<Move> moves(io.n_policy), r_moves(io.n_moves);
+        std::vector<uint8_t> r_expl(io.n_replays);
+        if (rc != TZ_OK) {
+            io.target_cap = io.n_targets;
+            io.policy_cap = io.n_policy;
+            io.replay_cap = io.n_replays;
+            io.move_cap = io.n_moves;
+            io.target_env = t_env.data();
+            io.target_value = t_value.data();
+            io.target_ube = t_ube.data();
+            io.target_n = t_n.data();
+            io.target_offset = t_off.data();
+            io.target_game = t_game.data();
+            io.policy_moves = moves.data();
+            io.policy_probs = probs.data();
+            io.replay_start = r_start.data();
+            io.replay_result = r_result.data();
+            io.replay_terminal = r_term.data();
+            io.replay_length = r_len.data();
+            io.replay_offset = r_off.data();
+            io.replay_game = r_game.data();
+            io.replay_exploration = r_expl.data();
+            io.replay_moves = r_moves.data();
+            check(tz_selfplay_read(h_, &io));
+        }
+        SelfplayData out;
+        out.high_water_bytes = io.high_water_bytes;
+        out.targets.resize(io.n_targets);
+        out.target_games = t_game;
+        for (size_t i = 0; i < io.n_targets; i++) {
+            Target& t = out.targets[i];
+            t.env = t_env[i];
+            t.value = t_value[i];
+            t.ube = t_ube[i];
+            t.policy.reserve((size_t)t_n[i]);
+            for (int j = 0; j < t_n[i]; j++) t.policy.emplace_back(moves[t_off[i] + j], probs[t_off[i] + j]);
+        }
+        out.games.resize(io.n_replays);
+        for (size_t i = 0; i < io.n_replays; i++) {
+            FinishedGame& f = out.games[i];
+            f.replay.env = r_start[i];
+            f.replay.actions.assign(r_moves.begin() + (ptrdiff_t)r_off[i], r_moves.begin() + (ptrdiff_t)(r_off[i] + r_len[i]));
+            f.result = r_result[i];
+            f.terminal = r_term[i];
+            f.game = r_game[i];
+            f.exploration = r_expl[i] != 0;
+        }
+        return out;
+    }
     void set_agent(int kind, tz_agent_fn fn = nullptr, void* ctx = nullptr) { check(tz_set_agent(h_, kind, fn, ctx)); }
     void new_openings(uint64_t seed) { check(tz_new_openings(h_, nullptr, nullptr, nullptr, seed)); }
     void set_positions(const std::vector<tz_state_t>& envs) { check(tz_set_positions(h_, envs.data(), nullptr)); }

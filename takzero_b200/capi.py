@@ -94,6 +94,35 @@ class ReanalyzeParams(C.Structure):
                 ("seed", C.c_uint64)]
 
 
+class SelfplayData(C.Structure):
+    """tz_selfplay_data_t: caller buffers of tz_selfplay_read."""
+
+    _fields_ = [("target_cap", C.c_size_t), ("policy_cap", C.c_size_t), ("replay_cap", C.c_size_t),
+                ("move_cap", C.c_size_t),
+                ("target_env", C.c_void_p), ("target_value", C.c_void_p), ("target_ube", C.c_void_p),
+                ("target_n", C.c_void_p), ("target_offset", C.c_void_p), ("target_game", C.c_void_p),
+                ("policy_moves", C.c_void_p), ("policy_probs", C.c_void_p),
+                ("replay_start", C.c_void_p), ("replay_result", C.c_void_p), ("replay_terminal", C.c_void_p),
+                ("replay_length", C.c_void_p), ("replay_offset", C.c_void_p), ("replay_game", C.c_void_p),
+                ("replay_exploration", C.c_void_p), ("replay_moves", C.c_void_p),
+                ("n_targets", C.c_size_t), ("n_policy", C.c_size_t), ("n_replays", C.c_size_t),
+                ("n_moves", C.c_size_t), ("high_water_bytes", C.c_size_t)]
+
+
+# tz_selfplay_data_t arrays: name -> (count field, dtype)
+SELFPLAY_FIELDS = {
+    "target_env": ("n_targets", STATE_DTYPE), "target_value": ("n_targets", np.float32),
+    "target_ube": ("n_targets", np.float32), "target_n": ("n_targets", np.int32),
+    "target_offset": ("n_targets", np.uint64), "target_game": ("n_targets", np.int32),
+    "policy_moves": ("n_policy", np.uint16), "policy_probs": ("n_policy", np.float32),
+    "replay_start": ("n_replays", STATE_DTYPE), "replay_result": ("n_replays", np.int32),
+    "replay_terminal": ("n_replays", np.int32), "replay_length": ("n_replays", np.int32),
+    "replay_offset": ("n_replays", np.uint64), "replay_game": ("n_replays", np.int32),
+    "replay_exploration": ("n_replays", np.uint8), "replay_moves": ("n_moves", np.uint16),
+}
+STATUS_TARGETS_FULL = 1024
+
+
 class Profile(C.Structure):
     _fields_ = [("ms", C.c_double * 8), ("launches", C.c_uint64 * 8), ("locksteps", C.c_uint64),
                 ("positions", C.c_uint64)]
@@ -168,6 +197,8 @@ def lib():
         "tz_tree_principal_variation": ([vp, vp, i32], i32),
         "tz_selfplay_move": ([vp, P(SelfplayParams)], i32),
         "tz_launch_count": ([vp, P(u64)], i32),
+        "tz_selfplay_record": ([vp, i32, C.c_size_t, C.c_size_t], i32),
+        "tz_selfplay_read": ([vp, P(SelfplayData)], i32),
         "tz_stage_positions": ([vp, vp, C.c_size_t], i32),
         "tz_reanalyze_batch": ([vp, vp, P(ReanalyzeParams)], i32),
         "tz_reanalyze_read": ([vp, i32, vp, vp, vp, vp, vp], i32),
@@ -234,6 +265,7 @@ class BatchedMCTS:
         self.n = board_n
         self.half_komi = half_komi
         self.G = n_games
+        self.game_base = game_base
         ms, slots, ic, oc = C.c_int(), C.c_uint32(), C.c_int(), C.c_int()
         _check(lib().tz_info(self._h, C.byref(ms), C.byref(slots), C.byref(ic), C.byref(oc)))
         self.move_stride, self.arena_slots = ms.value, slots.value
@@ -455,6 +487,45 @@ class BatchedMCTS:
     def selfplay_move(self, params: SelfplayParams) -> None:
         """One whole self-play move on the device, asynchronous (see tz_selfplay_move)."""
         _check(lib().tz_selfplay_move(self._h, C.byref(params)))
+
+    def selfplay_record(self, enable: bool = True, bytes_per_game: int = 0, output_bytes: int = 0) -> None:
+        """Keep the training data of selfplay_move on the device (0 = default sizes; see tz_selfplay_record)."""
+        _check(lib().tz_selfplay_record(self._h, 1 if enable else 0, int(bytes_per_game), int(output_bytes)))
+
+    def selfplay_read(self, capacity: Optional[dict] = None) -> dict:
+        """Completed targets and finished replays since the last read, as numpy arrays (empties the queue).
+
+        Targets come per finished game in ascending game order, each game's from its last ply to its first; target i
+        has policy entries policy_moves / policy_probs[target_offset[i] : + target_n[i]], replay j its moves
+        replay_moves[replay_offset[j] : + replay_length[j]].  `capacity` = {"n_targets": .., "n_policy": ..,
+        "n_replays": .., "n_moves": ..} reads with fixed buffers (TakzeroError when too small); None sizes them from
+        the queue.  Also returns "high_water_bytes"."""
+        io = SelfplayData()
+        if capacity is None:
+            rc = lib().tz_selfplay_read(self._h, C.byref(io))  # capacities 0: reports the counts
+            if rc == 0:
+                return self._selfplay_arrays(io, {k: 0 for k in ("n_targets", "n_policy", "n_replays", "n_moves")})
+            if rc != -1 or not (io.n_targets or io.n_policy or io.n_replays or io.n_moves):
+                _check(rc)
+            capacity = {k: getattr(io, k) for k in ("n_targets", "n_policy", "n_replays", "n_moves")}
+        out = {name: np.zeros(capacity[cnt], dtype=dt) for name, (cnt, dt) in SELFPLAY_FIELDS.items()}
+        io = SelfplayData()
+        io.target_cap, io.policy_cap = capacity["n_targets"], capacity["n_policy"]
+        io.replay_cap, io.move_cap = capacity["n_replays"], capacity["n_moves"]
+        for name, a in out.items():
+            setattr(io, name, a.ctypes.data_as(C.c_void_p).value if a.size else None)
+        _check(lib().tz_selfplay_read(self._h, C.byref(io)))
+        return self._selfplay_arrays(io, capacity, out)
+
+    @staticmethod
+    def _selfplay_arrays(io, capacity, out=None) -> dict:
+        res = {}
+        for name, (cnt, dt) in SELFPLAY_FIELDS.items():
+            n = getattr(io, cnt)
+            res[name] = out[name][:n].copy() if out is not None else np.zeros(0, dtype=dt)
+        for k in ("n_targets", "n_policy", "n_replays", "n_moves", "high_water_bytes"):
+            res[k] = int(getattr(io, k))
+        return res
 
     # ---- reanalyze (reanalyze/src/main.rs:147-235) ---------------------------------------------------------
     def stage_positions(self, states: np.ndarray) -> None:

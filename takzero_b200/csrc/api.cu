@@ -95,6 +95,8 @@ static int first_invalid_state(const tz_state_t* states, int count, int n, const
         if (bad_ >= 0) return fail(TZ_EINVAL, "state %d is not a possible position of this board", bad_); \
     } while (0)
 
+static void rec_free(tz_handle* h);
+
 static int default_stride(int n) { return n <= 3 ? 128 : n == 4 ? 256 : n == 5 ? 512 : 1024; }
 
 extern "C" TZ_API int tz_create(const tz_config_t* cfg, tz_handle** out) {
@@ -255,6 +257,7 @@ extern "C" TZ_API void tz_destroy(tz_handle* h) {
     if (h->stream) cudaStreamSynchronize(h->stream);
     nn_free(h);
     comm_destroy(h);
+    rec_free(h);
     for (void* p : h->allocs) cudaFree(p);
     if (h->pool) cudaFree(h->pool);
     if (h->pin_small) cudaFreeHost(h->pin_small);
@@ -280,9 +283,10 @@ extern "C" TZ_API int tz_sync(tz_handle* h) {
 
 static const char* status_text(uint32_t bits, char* buf, size_t len) {
     static const char* names[] = {"arena_full", "depth",       "no_child",      "too_many_moves",  "bad_move",
-                                  "nan",        "set_empty",   "replay_full",   "network_stall",   "weights_mismatch"};
+                                  "nan",        "set_empty",   "replay_full",   "network_stall",   "weights_mismatch",
+                                  "targets_full"};
     buf[0] = 0;
-    for (int i = 0; i < 10; i++)
+    for (int i = 0; i < 11; i++)
         if (bits & (1u << i)) {
             strncat(buf, names[i], len - strlen(buf) - 1);
             strncat(buf, " ", len - strlen(buf) - 1);
@@ -441,6 +445,7 @@ static int upload_mask(tz_handle* h, const uint8_t* mask, const uint8_t** dmask)
 
 extern "C" TZ_API int tz_set_positions(tz_handle* h, const tz_state_t* states, const uint8_t* mask) {
     CHECK_H(h);
+    h->rec_stale = true;
     if (!states) return fail(TZ_EINVAL, "null states");
     CHECK_STATES(states, h->d.G, mask);
     const uint8_t* dmask;
@@ -477,6 +482,7 @@ static int upload_openings(tz_handle* h, const int* sym, const int* adj, const i
 
 extern "C" TZ_API int tz_new_openings(tz_handle* h, const uint8_t* mask, const int* sym, const int* adj, uint64_t seed) {
     CHECK_H(h);
+    h->rec_stale = true;
     const uint8_t* dmask;
     const int *dsym, *dadj;
     int rc = upload_mask(h, mask, &dmask);
@@ -491,6 +497,7 @@ extern "C" TZ_API int tz_new_openings(tz_handle* h, const uint8_t* mask, const i
 
 extern "C" TZ_API int tz_random_steps(tz_handle* h, const uint8_t* mask, int steps, uint64_t seed) {
     CHECK_H(h);
+    h->rec_stale = true;
     if (steps < 0) return fail(TZ_EINVAL, "steps must be >= 0");
     const uint8_t* dmask;
     int rc = upload_mask(h, mask, &dmask);
@@ -501,6 +508,7 @@ extern "C" TZ_API int tz_random_steps(tz_handle* h, const uint8_t* mask, int ste
 
 extern "C" TZ_API int tz_reset_roots(tz_handle* h, const uint8_t* mask) {
     CHECK_H(h);
+    h->rec_stale = true;
     const uint8_t* dmask;
     int rc = upload_mask(h, mask, &dmask);
     if (rc) return rc;
@@ -684,6 +692,7 @@ extern "C" TZ_API int tz_last_gumbel(tz_handle* h, float* out, int stride) {
 
 extern "C" TZ_API int tz_step(tz_handle* h, const tz_move_t* moves) {
     CHECK_H(h);
+    h->rec_stale = true;
     if (!moves) return fail(TZ_EINVAL, "null moves");
     CU(cudaMemcpyAsync(h->moves, moves, (size_t)h->d.G * sizeof(uint16_t), cudaMemcpyHostToDevice, h->stream));
     launch_step(h->d, h->moves, h->stream);
@@ -693,6 +702,7 @@ extern "C" TZ_API int tz_step(tz_handle* h, const tz_move_t* moves) {
 
 extern "C" TZ_API int tz_restart_terminal(tz_handle* h, const int* sym, const int* adj, uint64_t seed, int* out_terminal) {
     CHECK_H(h);
+    h->rec_stale = true;
     if (!out_terminal) return fail(TZ_EINVAL, "null out_terminal");
     const int *dsym, *dadj;
     int rc = upload_openings(h, sym, adj, &dsym, &dadj);
@@ -1047,14 +1057,185 @@ extern "C" TZ_API int tz_selfplay_move(tz_handle* h, const tz_selfplay_t* sp) {
     if (rc) return rc;
     // targets of this position (selfplay/src/main.rs:243-256) stay on the device
     launch_targets(d, sp->target_visitations, sp->target_beta, d.M, h->tbl_f32a, h->ube, h->tbl_n, nullptr, h->stream);
+    const bool recording = h->rec.store != nullptr;
+    if (recording) {
+        if (h->rec_stale) {  // the pending records describe positions that were moved or replaced since
+            CU(cudaMemsetAsync(h->rec.used, 0, 3 * (size_t)d.G * sizeof(uint32_t), h->stream));
+            h->rec_stale = false;
+        }
+        launch_record(d, h->rec, h->tbl_f32a, h->ube, h->tbl_n, d.M, h->stream);
+    }
     // plies < weighted_random_plies sample proportionally to visits, the rest keep the halving winner
     launch_select_actions(d, sp->weighted_random_plies, sp->sample_threshold, sp->allowed_eval_drop, nullptr, sp->seed,
                           h->move_counter, h->tbl_moves, h->stream);
     launch_merge_moves(d, sp->weighted_random_plies, h->tbl_moves, h->moves, h->stream);
     launch_step(d, h->moves, h->stream);
     launch_restart(d, nullptr, nullptr, sp->seed, h->opening_counter++, h->terminal, h->fin_start, h->fin_replay,
-                   h->fin_len, h->stream);
+                   h->fin_len, h->stream, recording ? h->rec.result : nullptr);
     h->launches += 6;
+    if (recording) {
+        // restart_envs_and_complete_targets (main.rs:263-329): the exploration half is the first G/2 games
+        launch_emit(d, h->rec, h->terminal, h->fin_len, h->fin_start, h->fin_replay, sp->weighted_random_plies,
+                    sp->beta != 0.0f ? d.G / 2 : 0, h->stream);
+        h->launches += 4;
+    }
+    CU(cudaGetLastError());
+    return TZ_OK;
+}
+
+// ---- training data of resident self-play ------------------------------------------------------------------
+
+static void rec_free(tz_handle* h) {
+    for (void* p : h->rec_allocs) cudaFree(p);
+    h->rec_allocs.clear();
+    memset(&h->rec, 0, sizeof(h->rec));
+    h->rec_stale = false;
+}
+
+// bytes of one queued target (env, value, ube, n, policy offset, game id) / replay (start, result, terminal, length,
+// move offset, game id, exploration flag)
+static const size_t TZ_TARGET_BYTES = sizeof(TzState) + 4 + 4 + 4 + 8 + 4;
+static const size_t TZ_REPLAY_BYTES = sizeof(TzState) + 4 + 4 + 4 + 8 + 4 + 1;
+
+extern "C" TZ_API int tz_selfplay_record(tz_handle* h, int enable, size_t bytes_per_game, size_t output_bytes) {
+    CHECK_H(h);
+    CU(cudaStreamSynchronize(h->stream));
+    rec_free(h);
+    if (!enable) return TZ_OK;
+    const size_t G = (size_t)h->d.G, M = (size_t)h->d.M;
+    const size_t worst = (size_t)TZ_MAX_PLIES * (sizeof(TzRecHead) + ((6 * M + 15) & ~(size_t)15));
+    size_t free_b = 0, total_b = 0;
+    CU(cudaMemGetInfo(&free_b, &total_b));
+    size_t bpg = bytes_per_game;
+    if (bpg == 0) {  // a quarter of the free HBM, at least 64 KiB and at most the worst case, per game
+        bpg = free_b / 4 / G;
+        if (bpg > worst) bpg = worst;
+        if (bpg < (64 << 10)) bpg = 64 << 10;
+    }
+    bpg &= ~(size_t)15;  // records are 16-byte aligned
+    if (bpg == 0) return fail(TZ_EINVAL, "bytes_per_game must be 0 (default) or >= 16");
+    size_t out = output_bytes;
+    if (out == 0) {  // half of the whole store, at most an eighth of the free HBM, at least 16 MiB
+        out = G * bpg / 2;
+        if (out > free_b / 8) out = free_b / 8;
+        if (out < (16 << 20)) out = 16 << 20;
+    }
+    // the queue's split: 1/16 replay records, 1/16 replay moves, the rest targets and policy entries for a mean of
+    // move_stride / 4 children per target
+    const size_t mean_n = M / 4 > 0 ? M / 4 : 1;
+    const size_t tp = out - out / 8;
+    unsigned long long cap[TZ_Q_KINDS];
+    cap[TZ_Q_TARGETS] = tp / (TZ_TARGET_BYTES + 6 * mean_n);
+    cap[TZ_Q_POLICY] = (tp - cap[TZ_Q_TARGETS] * TZ_TARGET_BYTES) / 6;
+    cap[TZ_Q_REPLAYS] = out / 16 / TZ_REPLAY_BYTES;
+    cap[TZ_Q_MOVES] = out / 16 / 2;
+    for (int q = 0; q < TZ_Q_KINDS; q++)
+        if (cap[q] == 0) return fail(TZ_EINVAL, "output_bytes %zu cannot hold one replay", out);
+    TzRecorder& r = h->rec;
+    uint32_t* cursors = nullptr;
+    cudaError_t e = cudaSuccess;
+#define RM(ptr, count)                                                                  \
+    if (e == cudaSuccess) {                                                             \
+        void* v_ = nullptr;                                                             \
+        e = cudaMalloc(&v_, (size_t)(count) * sizeof(*(ptr)));                         \
+        if (e == cudaSuccess) {                                                         \
+            h->rec_allocs.push_back(v_);                                                \
+            (ptr) = (decltype(ptr))v_;                                                  \
+        }                                                                               \
+    }
+    RM(r.store, G * bpg);
+    RM(r.rec_off, G * TZ_MAX_PLIES);
+    RM(cursors, 3 * G);
+    RM(r.high_water, 1);
+    RM(r.fill, TZ_Q_KINDS);
+    RM(r.result, G);
+    RM(r.g_count, G * TZ_Q_KINDS);
+    RM(r.g_base, G * TZ_Q_KINDS);
+    RM(r.t_env, cap[TZ_Q_TARGETS]);
+    RM(r.t_value, cap[TZ_Q_TARGETS]);
+    RM(r.t_ube, cap[TZ_Q_TARGETS]);
+    RM(r.t_n, cap[TZ_Q_TARGETS]);
+    RM(r.t_off, cap[TZ_Q_TARGETS]);
+    RM(r.t_game, cap[TZ_Q_TARGETS]);
+    RM(r.p_moves, cap[TZ_Q_POLICY]);
+    RM(r.p_probs, cap[TZ_Q_POLICY]);
+    RM(r.r_start, cap[TZ_Q_REPLAYS]);
+    RM(r.r_result, cap[TZ_Q_REPLAYS]);
+    RM(r.r_terminal, cap[TZ_Q_REPLAYS]);
+    RM(r.r_len, cap[TZ_Q_REPLAYS]);
+    RM(r.r_off, cap[TZ_Q_REPLAYS]);
+    RM(r.r_game, cap[TZ_Q_REPLAYS]);
+    RM(r.r_exploration, cap[TZ_Q_REPLAYS]);
+    RM(r.r_moves, cap[TZ_Q_MOVES]);
+#undef RM
+    if (e != cudaSuccess) {
+        rec_free(h);
+        return fail(TZ_ENOMEM, "cudaMalloc of the self-play record store (%zu B per game) / queue (%zu B): %s", bpg, out,
+                    cudaGetErrorString(e));
+    }
+    r.used = cursors;
+    r.count = cursors + G;
+    r.full = cursors + 2 * G;
+    r.bytes_per_game = bpg;
+    for (int q = 0; q < TZ_Q_KINDS; q++) r.cap[q] = cap[q];
+    int rc = TZ_OK;
+    if (cudaMemsetAsync(cursors, 0, 3 * G * sizeof(uint32_t), h->stream) != cudaSuccess ||
+        cudaMemsetAsync(r.high_water, 0, sizeof(uint32_t), h->stream) != cudaSuccess ||
+        cudaMemsetAsync(r.fill, 0, TZ_Q_KINDS * sizeof(unsigned long long), h->stream) != cudaSuccess ||
+        cudaStreamSynchronize(h->stream) != cudaSuccess)
+        rc = fail(TZ_ECUDA, "tz_selfplay_record: %s", cudaGetErrorString(cudaGetLastError()));
+    if (rc) rec_free(h);
+    return rc;
+}
+
+extern "C" TZ_API int tz_selfplay_read(tz_handle* h, tz_selfplay_data_t* io) {
+    CHECK_H(h);
+    if (!io) return fail(TZ_EINVAL, "null io");
+    const TzRecorder& r = h->rec;
+    if (!r.store) return fail(TZ_EINVAL, "recording is off: tz_selfplay_record first");
+    unsigned long long* fill = (unsigned long long*)(h->pin_small + 256);
+    uint32_t* hw = (uint32_t*)(h->pin_small + 256 + 8 * TZ_Q_KINDS);
+    uint32_t* bits = hw + 1;
+    CU(cudaMemcpyAsync(fill, r.fill, TZ_Q_KINDS * sizeof(unsigned long long), cudaMemcpyDeviceToHost, h->stream));
+    CU(cudaMemcpyAsync(hw, r.high_water, sizeof(uint32_t), cudaMemcpyDeviceToHost, h->stream));
+    CU(cudaMemcpyAsync(bits, h->d.status, sizeof(uint32_t), cudaMemcpyDeviceToHost, h->stream));
+    CU(cudaStreamSynchronize(h->stream));
+    CU(cudaGetLastError());
+    if (*bits & ~(uint32_t)TZ_ERR_TARGETS_FULL) {
+        char buf[160];
+        return fail(TZ_ESEARCH, "device search error bits 0x%x: %s", *bits, status_text(*bits, buf, sizeof(buf)));
+    }
+    io->n_targets = (size_t)fill[TZ_Q_TARGETS];
+    io->n_policy = (size_t)fill[TZ_Q_POLICY];
+    io->n_replays = (size_t)fill[TZ_Q_REPLAYS];
+    io->n_moves = (size_t)fill[TZ_Q_MOVES];
+    io->high_water_bytes = (size_t)*hw;
+    if (io->target_cap < io->n_targets || io->policy_cap < io->n_policy || io->replay_cap < io->n_replays ||
+        io->move_cap < io->n_moves)
+        return fail(TZ_EINVAL, "capacity too small: the queue holds %zu targets, %zu policy entries, %zu replays, %zu moves",
+                    io->n_targets, io->n_policy, io->n_replays, io->n_moves);
+#define OUT(dst, src, count)                                                                                    \
+    if ((dst) && (count) > 0)                                                                                   \
+    CU(cudaMemcpyAsync((dst), (src), (size_t)(count) * sizeof(*(dst)), cudaMemcpyDeviceToHost, h->stream))
+    OUT(io->target_env, (const tz_state_t*)r.t_env, io->n_targets);
+    OUT(io->target_value, r.t_value, io->n_targets);
+    OUT(io->target_ube, r.t_ube, io->n_targets);
+    OUT(io->target_n, r.t_n, io->n_targets);
+    OUT(io->target_offset, (const uint64_t*)r.t_off, io->n_targets);
+    OUT(io->target_game, r.t_game, io->n_targets);
+    OUT(io->policy_moves, r.p_moves, io->n_policy);
+    OUT(io->policy_probs, r.p_probs, io->n_policy);
+    OUT(io->replay_start, (const tz_state_t*)r.r_start, io->n_replays);
+    OUT(io->replay_result, r.r_result, io->n_replays);
+    OUT(io->replay_terminal, r.r_terminal, io->n_replays);
+    OUT(io->replay_length, r.r_len, io->n_replays);
+    OUT(io->replay_offset, (const uint64_t*)r.r_off, io->n_replays);
+    OUT(io->replay_game, r.r_game, io->n_replays);
+    OUT(io->replay_exploration, r.r_exploration, io->n_replays);
+    OUT(io->replay_moves, r.r_moves, io->n_moves);
+#undef OUT
+    CU(cudaMemsetAsync(r.fill, 0, TZ_Q_KINDS * sizeof(unsigned long long), h->stream));
+    CU(cudaStreamSynchronize(h->stream));
     CU(cudaGetLastError());
     return TZ_OK;
 }
@@ -1101,6 +1282,7 @@ extern "C" TZ_API int tz_reanalyze_batch(tz_handle* h, const uint32_t* pool_indi
         CU(cudaMemcpyAsync(h->pool_idx, pool_indices, (size_t)d.G * sizeof(uint32_t), cudaMemcpyHostToDevice, h->stream));
         launch_gather_positions(d, h->pool, h->pool_idx, h->stream);  // *node = Node::default(); *env = replay_env
         h->launches += 1;
+        h->rec_stale = true;
     }
     launch_gumbel_noise(d, h->gumbel, d.M, rp->seed, h->move_counter, h->stream);
     h->gumbel_stride = d.M;
@@ -1305,6 +1487,7 @@ extern "C" TZ_API int tz_read_novelty_set(tz_handle* h, uint8_t* out, size_t cap
 
 static int tree_simulate(tz_handle* h, float beta, int batch_size, int max_forwards) {
     const TzDev& d = h->d;
+    h->rec_stale = true;
     if (batch_size <= 0 || batch_size > d.Q)
         return fail(TZ_EINVAL, "batch_size must be 1..max(n_games, tree_batch) (%d)", d.Q);
     h->prof_active = false;
@@ -1328,6 +1511,7 @@ extern "C" TZ_API int tz_tree_simulate_batch(tz_handle* h, float beta, int batch
 
 extern "C" TZ_API int tz_tree_descend(tz_handle* h, tz_move_t move) {
     CHECK_H(h);
+    h->rec_stale = true;
     std::vector<uint16_t> mv((size_t)h->d.G, 0);
     mv[0] = move;
     CU(cudaMemcpyAsync(h->moves, mv.data(), mv.size() * sizeof(uint16_t), cudaMemcpyHostToDevice, h->stream));

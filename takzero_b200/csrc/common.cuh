@@ -75,6 +75,7 @@ enum {
     TZ_ERR_REPLAY_FULL = 128,
     TZ_ERR_NETWORK_STALL = 256,
     TZ_ERR_WEIGHTS_MISMATCH = 512,
+    TZ_ERR_TARGETS_FULL = 1024,
 };
 
 // Device-side view of one handle, passed by value to every kernel.
@@ -117,4 +118,54 @@ struct TzDev {
     int* set_len;         // [G]
     unsigned long long* counters;  // [G][4] simulations, evaluations, known, expansions
     uint32_t* status;              // [1] sticky error bits
+};
+
+// Training data of resident self-play (tz_selfplay_record / tz_selfplay_read).
+// Pending records: every game owns `bytes_per_game` bytes of `store`; a record is a TzRecHead followed by n f32
+// improved-policy probabilities and n u16 moves (child order), padded to 16 bytes.  When a game ends its records are
+// completed with their value and emitted, with the game's replay, into the output queue: struct-of-arrays with one
+// array per field of tz_selfplay_data_t, so that tz_selfplay_read is one copy per array.
+struct __align__(16) TzRecHead {
+    TzState env;  // the root position before the move
+    int p;        // replay index of the move (replay_len at that moment)
+    int n;        // children of the root
+    float ube;    // UBE target
+    int pad;
+};
+static_assert(sizeof(TzRecHead) == 400, "record header is 400 bytes");
+
+enum { TZ_Q_TARGETS = 0, TZ_Q_POLICY, TZ_Q_REPLAYS, TZ_Q_MOVES, TZ_Q_KINDS };
+
+struct TzRecorder {
+    // pending records; used / count / full are one allocation [3][G] (one memset clears every cursor)
+    unsigned char* store;       // [G][bytes_per_game]
+    uint32_t* rec_off;          // [G][TZ_MAX_PLIES] byte offset of each record inside the game's region
+    uint32_t* used;             // [G] bytes in use
+    uint32_t* count;            // [G] records
+    uint32_t* full;             // [G] the region ran out: no more records until the game ends
+    uint32_t* high_water;       // [1] most bytes one game has used
+    unsigned long long bytes_per_game;
+    // output queue
+    TzState* t_env;
+    float* t_value;
+    float* t_ube;
+    int* t_n;
+    unsigned long long* t_off;  // first policy entry of the target
+    int* t_game;                // global game id
+    uint16_t* p_moves;
+    float* p_probs;
+    TzState* r_start;
+    int* r_result;              // tz_game_result code of the final position
+    int* r_terminal;            // tz_result code of the final position (side to move)
+    int* r_len;
+    unsigned long long* r_off;  // first move of the replay in r_moves
+    int* r_game;
+    uint8_t* r_exploration;
+    uint16_t* r_moves;
+    unsigned long long cap[TZ_Q_KINDS];  // entries of targets, policy, replays, moves
+    unsigned long long* fill;            // [TZ_Q_KINDS] entries in the queue
+    // emission of one move
+    int* result;                // [G] tz_game_result of every game k_restart finished
+    unsigned long long* g_count;  // [G][TZ_Q_KINDS] what each finished game emits
+    unsigned long long* g_base;   // [G][TZ_Q_KINDS] where it goes; g_base[g][0] = ~0 when it does not fit
 };

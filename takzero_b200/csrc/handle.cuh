@@ -59,6 +59,10 @@ struct tz_handle {
     float* pin_logits = nullptr;
     float* pin_value = nullptr;
     float* pin_variance = nullptr;
+    // resident self-play training data (tz_selfplay_record); rec.store == nullptr: recording is off
+    TzRecorder rec{};
+    std::vector<void*> rec_allocs;
+    bool rec_stale = false;  // positions were moved or replaced since the last recording move: drop pending records
     // bookkeeping
     unsigned long long move_counter = 0;
     unsigned long long opening_counter = 0;

@@ -1172,11 +1172,11 @@ __global__ void k_reset_roots(TzDev d, const uint8_t* mask) {
 }
 
 // batched.rs:185-203.  A finished game's replay is parked in fin_* before the reset so the
-// host can still read it.
+// host can still read it; out_result (optional) receives the absolute result of the final position.
 __global__ void __launch_bounds__(32 * WPB) k_restart(TzDev d, const int* sym, const int* adj,
                                                       unsigned long long seed, unsigned long long counter,
                                                       int* out_terminal, TzState* fin_start, uint16_t* fin_replay,
-                                                      int* fin_len) {
+                                                      int* fin_len, int* out_result) {
     __shared__ TzState s_state[WPB];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int g = blockIdx.x * WPB + warp;
@@ -1186,6 +1186,10 @@ __global__ void __launch_bounds__(32 * WPB) k_restart(TzDev d, const int* sym, c
     const int term = warp_terminal(st, d.n, d.half_komi, d.rev_limit, lane);
     if (lane == 0) out_terminal[g] = term;
     if (term == TZ_T_NONE) return;
+    if (out_result) {
+        const int res = warp_game_result(st, d.n, d.half_komi, d.rev_limit, lane);
+        if (lane == 0) out_result[g] = res;
+    }
     const int rl = d.replay_len[g];
     for (int i = lane; i < rl; i += 32)
         fin_replay[(size_t)g * TZ_MAX_PLIES + i] = d.replay[(size_t)g * TZ_MAX_PLIES + i];
@@ -1559,9 +1563,246 @@ __global__ void k_debug_expf(const float* in, int count, float* out) {
     if (i < count) out[i] = expf_libm(in[i]);
 }
 
+// ---- resident self-play training data (selfplay/src/main.rs:238-329 on the device) ------------------
+
+__device__ __forceinline__ uint32_t record_bytes(int n) {
+    return (uint32_t)sizeof(TzRecHead) + (((uint32_t)n * 6u + 15u) & ~15u);
+}
+
+// selfplay/src/main.rs:173: the exploration half keeps only targets past the weighted-random plies
+__device__ __forceinline__ bool record_kept(int g, int exploration_games, int ply, int weighted_random_plies) {
+    return g >= exploration_games || ply > weighted_random_plies;
+}
+
+// take_a_step (main.rs:238-258): append one pending record per game -- the root position, its replay index, the
+// improved policy / UBE target k_targets left in `policy` [G][stride] / `ube` / `tbl_n`, the root's moves in child
+// order.  A game whose region is full records nothing more until it ends.
+__global__ void __launch_bounds__(32 * WPB) k_record(TzDev d, TzRecorder r, const float* policy, const float* ube,
+                                                     const int* tbl_n, int stride) {
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int g = blockIdx.x * WPB + warp;
+    if (g >= d.G || r.full[g]) return;
+    int n = tbl_n[g];
+    if (n > stride) n = stride;
+    const uint32_t size = record_bytes(n);
+    const uint32_t cnt = r.count[g], used = r.used[g];
+    if (cnt >= TZ_MAX_PLIES || (unsigned long long)used + size > r.bytes_per_game) {
+        if (lane == 0) {
+            r.full[g] = 1;
+            atomicOr(d.status, TZ_ERR_TARGETS_FULL);
+        }
+        return;
+    }
+    unsigned char* rec = r.store + (size_t)g * r.bytes_per_game + used;
+    TzRecHead* head = reinterpret_cast<TzRecHead*>(rec);
+    warp_load_state(&head->env, &d.env[g], lane);
+    if (lane == 0) {
+        head->p = d.replay_len[g];
+        head->n = n;
+        head->ube = ube[g];
+        head->pad = 0;
+    }
+    float* probs = reinterpret_cast<float*>(rec + sizeof(TzRecHead));
+    uint16_t* moves = reinterpret_cast<uint16_t*>(probs + n);
+    const GameTree t = game_tree(d.arena, g);
+    const uint32_t first = t.first[0];
+    for (int i = lane; i < n; i += 32) {
+        probs[i] = policy[(size_t)g * stride + i];
+        moves[i] = (uint16_t)tz_meta_move(t.meta[first + i]);
+    }
+    if (lane == 0) {
+        r.rec_off[(size_t)g * TZ_MAX_PLIES + cnt] = used;
+        r.count[g] = cnt + 1;
+        r.used[g] = used + size;
+        atomicMax(r.high_water, used + size);
+    }
+}
+
+// what every game k_restart finished emits: kept targets, their policy entries, one replay, its moves
+__global__ void __launch_bounds__(32 * WPB) k_emit_count(TzDev d, TzRecorder r, const int* terminal, const int* fin_len,
+                                                         int weighted_random_plies, int exploration_games) {
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int g = blockIdx.x * WPB + warp;
+    if (g >= d.G) return;
+    unsigned long long* c = r.g_count + (size_t)g * TZ_Q_KINDS;
+    if (terminal[g] == TZ_T_NONE) {
+        if (lane < TZ_Q_KINDS) c[lane] = 0;
+        return;
+    }
+    const int cnt = (int)r.count[g];
+    const unsigned char* region = r.store + (size_t)g * r.bytes_per_game;
+    unsigned long long kept = 0, entries = 0;
+    for (int j = lane; j < cnt; j += 32) {
+        const TzRecHead* h = reinterpret_cast<const TzRecHead*>(region + r.rec_off[(size_t)g * TZ_MAX_PLIES + j]);
+        if (record_kept(g, exploration_games, (int)h->env.ply, weighted_random_plies)) {
+            kept++;
+            entries += (unsigned long long)h->n;
+        }
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        kept += __shfl_xor_sync(FULL_MASK, kept, o);
+        entries += __shfl_xor_sync(FULL_MASK, entries, o);
+    }
+    if (lane == 0) {
+        c[TZ_Q_TARGETS] = kept;
+        c[TZ_Q_POLICY] = entries;
+        c[TZ_Q_REPLAYS] = 1;
+        c[TZ_Q_MOVES] = (unsigned long long)fin_len[g];
+    }
+}
+
+// exclusive scan of the per-game counts over games in index order (one block): game g's data goes to
+// fill + (sum over games < g).  The games that fit form a prefix (the sums only grow); the first game that does not
+// fit and every later one are dropped (their records are lost), TZ_ERR_TARGETS_FULL is raised, and the queue fill
+// advances past the games that fit only.
+__global__ void __launch_bounds__(1024) k_emit_scan(TzDev d, TzRecorder r) {
+    __shared__ unsigned long long s_warp[32][TZ_Q_KINDS];
+    __shared__ unsigned long long s_carry[TZ_Q_KINDS], s_fill[TZ_Q_KINDS];
+    __shared__ int s_dropped;
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    if (tid < TZ_Q_KINDS) {
+        s_carry[tid] = 0;
+        s_fill[tid] = r.fill[tid];
+    }
+    if (tid == 0) s_dropped = 0;
+    __syncthreads();
+    for (int base = 0; base < d.G; base += 1024) {
+        const int g = base + tid;
+        unsigned long long v[TZ_Q_KINDS], incl[TZ_Q_KINDS];
+#pragma unroll
+        for (int q = 0; q < TZ_Q_KINDS; q++) {
+            v[q] = g < d.G ? r.g_count[(size_t)g * TZ_Q_KINDS + q] : 0ull;
+            incl[q] = v[q];
+        }
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1)
+#pragma unroll
+            for (int q = 0; q < TZ_Q_KINDS; q++) {
+                const unsigned long long y = __shfl_up_sync(FULL_MASK, incl[q], o);
+                if (lane >= o) incl[q] += y;
+            }
+        if (lane == 31)
+            for (int q = 0; q < TZ_Q_KINDS; q++) s_warp[warp][q] = incl[q];
+        __syncthreads();
+        if (warp == 0) {
+#pragma unroll
+            for (int q = 0; q < TZ_Q_KINDS; q++) {
+                unsigned long long x = s_warp[lane][q];
+#pragma unroll
+                for (int o = 1; o < 32; o <<= 1) {
+                    const unsigned long long y = __shfl_up_sync(FULL_MASK, x, o);
+                    if (lane >= o) x += y;
+                }
+                s_warp[lane][q] = x;
+            }
+        }
+        __syncthreads();
+        if (g < d.G && v[TZ_Q_REPLAYS] != 0) {
+            unsigned long long at[TZ_Q_KINDS];
+            bool fits = true;
+#pragma unroll
+            for (int q = 0; q < TZ_Q_KINDS; q++) {
+                const unsigned long long before = s_carry[q] + (warp ? s_warp[warp - 1][q] : 0ull) + incl[q] - v[q];
+                at[q] = r.fill[q] + before;
+                fits = fits && at[q] + v[q] <= r.cap[q];
+            }
+            unsigned long long* b = r.g_base + (size_t)g * TZ_Q_KINDS;
+            if (fits) {
+#pragma unroll
+                for (int q = 0; q < TZ_Q_KINDS; q++) {
+                    b[q] = at[q];
+                    atomicMax(&s_fill[q], at[q] + v[q]);
+                }
+            } else {
+                b[0] = ~0ull;
+                s_dropped = 1;
+            }
+        }
+        __syncthreads();
+        if (tid < TZ_Q_KINDS) s_carry[tid] += s_warp[31][tid];
+        __syncthreads();
+    }
+    if (tid < TZ_Q_KINDS) r.fill[tid] = s_fill[tid];
+    if (tid == 0 && s_dropped) atomicOr(d.status, TZ_ERR_TARGETS_FULL);
+}
+
+// restart_envs_and_complete_targets (main.rs:263-329): the finished game's replay, then its targets from the last ply
+// to the first with value = Eval::from(terminal) negated L - p times (L = replay length, p = the record's replay
+// index), the exploration half filtered by ply; every finished game's cursor is reset
+__global__ void __launch_bounds__(32 * WPB) k_emit_write(TzDev d, TzRecorder r, const int* terminal, const int* fin_len,
+                                                         const TzState* fin_start, const uint16_t* fin_replay,
+                                                         int weighted_random_plies, int exploration_games) {
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int g = blockIdx.x * WPB + warp;
+    if (g >= d.G) return;
+    const int term = terminal[g];
+    if (term == TZ_T_NONE) return;
+    const unsigned long long* b = r.g_base + (size_t)g * TZ_Q_KINDS;
+    if (b[TZ_Q_TARGETS] != ~0ull) {
+        const unsigned long long ri = b[TZ_Q_REPLAYS], mo = b[TZ_Q_MOVES];
+        const int L = fin_len[g];
+        warp_load_state(&r.r_start[ri], &fin_start[g], lane);
+        if (lane == 0) {
+            r.r_result[ri] = r.result[g];
+            r.r_terminal[ri] = term;
+            r.r_len[ri] = L;
+            r.r_off[ri] = mo;
+            r.r_game[ri] = d.game_base + g;
+            r.r_exploration[ri] = g < exploration_games ? 1 : 0;
+        }
+        for (int i = lane; i < L; i += 32) r.r_moves[mo + i] = fin_replay[(size_t)g * TZ_MAX_PLIES + i];
+        unsigned long long ti = b[TZ_Q_TARGETS], po = b[TZ_Q_POLICY];
+        const unsigned char* region = r.store + (size_t)g * r.bytes_per_game;
+        Ev e = ev_from_terminal(term);
+        int pc = L;
+        for (int j = (int)r.count[g] - 1; j >= 0; j--) {
+            const unsigned char* rec = region + r.rec_off[(size_t)g * TZ_MAX_PLIES + j];
+            const TzRecHead* h = reinterpret_cast<const TzRecHead*>(rec);
+            const int p = h->p, n = h->n;
+            for (; pc > p; pc--) e = ev_negate(e);
+            if (!record_kept(g, exploration_games, (int)h->env.ply, weighted_random_plies)) continue;
+            warp_load_state(&r.t_env[ti], &h->env, lane);
+            if (lane == 0) {
+                r.t_value[ti] = ev_to_f32(e);
+                r.t_ube[ti] = h->ube;
+                r.t_n[ti] = n;
+                r.t_off[ti] = po;
+                r.t_game[ti] = d.game_base + g;
+            }
+            const float* probs = reinterpret_cast<const float*>(rec + sizeof(TzRecHead));
+            const uint16_t* moves = reinterpret_cast<const uint16_t*>(probs + n);
+            for (int i = lane; i < n; i += 32) {
+                r.p_probs[po + i] = probs[i];
+                r.p_moves[po + i] = moves[i];
+            }
+            ti++;
+            po += (unsigned long long)n;
+        }
+    }
+    __syncwarp();
+    if (lane == 0) {
+        r.count[g] = 0;
+        r.used[g] = 0;
+        r.full[g] = 0;
+    }
+}
+
 // ---- launchers -------------------------------------------------------------------------------
 
 static inline int blocks_for(int items) { return (items + WPB - 1) / WPB; }
+
+void launch_record(const TzDev& d, const TzRecorder& r, const float* policy, const float* ube, const int* n, int stride,
+                   cudaStream_t st) {
+    k_record<<<blocks_for(d.G), 32 * WPB, 0, st>>>(d, r, policy, ube, n, stride);
+}
+void launch_emit(const TzDev& d, const TzRecorder& r, const int* terminal, const int* fin_len, const TzState* fin_start,
+                 const uint16_t* fin_replay, int weighted_random_plies, int exploration_games, cudaStream_t st) {
+    k_emit_count<<<blocks_for(d.G), 32 * WPB, 0, st>>>(d, r, terminal, fin_len, weighted_random_plies, exploration_games);
+    k_emit_scan<<<1, 1024, 0, st>>>(d, r);
+    k_emit_write<<<blocks_for(d.G), 32 * WPB, 0, st>>>(d, r, terminal, fin_len, fin_start, fin_replay,
+                                                       weighted_random_plies, exploration_games);
+}
 
 void launch_select(const TzDev& d, int phase, int halving_i, const float* betas, cudaStream_t st) {
     k_select<<<blocks_for(d.G), 32 * WPB, 0, st>>>(d, phase, halving_i, betas);
@@ -1625,9 +1866,10 @@ void launch_reset_roots(const TzDev& d, const uint8_t* mask, cudaStream_t st) {
     k_reset_roots<<<(d.G + 127) / 128, 128, 0, st>>>(d, mask);
 }
 void launch_restart(const TzDev& d, const int* sym, const int* adj, unsigned long long seed, unsigned long long counter,
-                    int* out_terminal, TzState* fin_start, uint16_t* fin_replay, int* fin_len, cudaStream_t st) {
+                    int* out_terminal, TzState* fin_start, uint16_t* fin_replay, int* fin_len, cudaStream_t st,
+                    int* out_result) {
     k_restart<<<blocks_for(d.G), 32 * WPB, 0, st>>>(d, sym, adj, seed, counter, out_terminal, fin_start, fin_replay,
-                                                    fin_len);
+                                                    fin_len, out_result);
 }
 void launch_root_table(const TzDev& d, int stride, int* out_n, uint16_t* moves, uint32_t* visits, uint32_t* eval_tag,
                        uint32_t* eval_bits, float* logit, float* prob, float* std_dev, cudaStream_t st) {

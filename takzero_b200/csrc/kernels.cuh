@@ -19,7 +19,14 @@ void launch_new_openings(const TzDev& d, const uint8_t* mask, const int* sym, co
 void launch_set_positions(const TzDev& d, const TzState* states, const uint8_t* mask, cudaStream_t st);
 void launch_reset_roots(const TzDev& d, const uint8_t* mask, cudaStream_t st);
 void launch_restart(const TzDev& d, const int* sym, const int* adj, unsigned long long seed, unsigned long long counter,
-                    int* out_terminal, TzState* fin_start, uint16_t* fin_replay, int* fin_len, cudaStream_t st);
+                    int* out_terminal, TzState* fin_start, uint16_t* fin_replay, int* fin_len, cudaStream_t st,
+                    int* out_result = nullptr);
+// resident self-play training data: one pending record per game (after launch_targets), and after launch_restart
+// the finished games' completed targets and replays into the output queue (three launches)
+void launch_record(const TzDev& d, const TzRecorder& r, const float* policy, const float* ube, const int* n, int stride,
+                   cudaStream_t st);
+void launch_emit(const TzDev& d, const TzRecorder& r, const int* terminal, const int* fin_len, const TzState* fin_start,
+                 const uint16_t* fin_replay, int weighted_random_plies, int exploration_games, cudaStream_t st);
 void launch_root_table(const TzDev& d, int stride, int* out_n, uint16_t* moves, uint32_t* visits, uint32_t* eval_tag,
                        uint32_t* eval_bits, float* logit, float* prob, float* std_dev, cudaStream_t st);
 void launch_root_stats(const TzDev& d, uint32_t* out, cudaStream_t st);

@@ -38,6 +38,9 @@ __device__ __forceinline__ Ev ev_negate(Ev e) {  // eval.rs:40-47
     }
 }
 
+// Eval::from(terminal) (eval.rs:118-126): tz_result codes 1 win, 2 loss, 3 draw are the tags Win / Loss / Draw at ply 0
+__device__ __forceinline__ Ev ev_from_terminal(int terminal) { return ev_make((uint32_t)terminal, 0u); }
+
 // compiler-rt __powisf2(0.997f, ply): what Rust's f32::powi lowers to (eval.rs:97)
 __device__ __forceinline__ float powi_discount(int b) {
     float a = 0.997f, r = 1.0f;
