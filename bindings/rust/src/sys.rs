@@ -200,6 +200,9 @@ extern "C" {
     pub fn tz_tree_simulate_batch(h: *mut tz_handle, beta: f32, batch_size: c_int) -> c_int;
     pub fn tz_tree_descend(h: *mut tz_handle, move_: tz_move_t) -> c_int;
     pub fn tz_tree_principal_variation(h: *mut tz_handle, out_moves: *mut tz_move_t, cap: c_int) -> c_int;
+    pub fn tz_trees_simulate_batch(h: *mut tz_handle, mask: *const u8, beta: f32, batch_size: c_int) -> c_int;
+    pub fn tz_trees_descend(h: *mut tz_handle, mask: *const u8, moves: *const tz_move_t) -> c_int;
+    pub fn tz_trees_principal_variation(h: *mut tz_handle, mask: *const u8, cap: c_int, out_moves: *mut tz_move_t, out_len: *mut c_int) -> c_int;
     pub fn tz_set_weights(h: *mut tz_handle, tensors: *const tz_tensor_t, count: c_int) -> c_int;
     pub fn tz_comm_unique_id(out_id128: *mut c_void) -> c_int;
     pub fn tz_comm_init(h: *mut tz_handle, id128: *const c_void, nranks: c_int, rank: c_int) -> c_int;

@@ -3,12 +3,18 @@
 // (`env.play` + `Node::descend`: the explored sub-tree is kept); any other line runs `simulate_batch(agent, env,
 // BETA = 0, BATCH_SIZE = 128)`; after either, the root is printed with `impl Display for Node` (node/debug.rs).
 // `--example` plays a whole game against itself: simulate, `select_best_action`, descend (main.rs:33-42).
+// `--positions FILE --batches K` analyses a list of positions instead (one TPS per line; blank lines are skipped): each
+// position is the tree of one game of a single handle, all trees get K simulate_batch calls side by side
+// (tz_trees_simulate_batch, one network batch for all of them), then, in file order, every position prints its TPS, its
+// root as the REPL would and its principal variation.
 // Differences at the process boundary: --model-path may be omitted (deterministic synthetic agent, for tests);
 // board size and komi are flags; end of input ends the program.
 #include <cstdio>
 #include <cstdlib>
+#include <fstream>
 #include <iostream>
 #include <string>
+#include <vector>
 
 #include "../include/takzero_b200.hpp"
 
@@ -16,10 +22,55 @@ using namespace takzero;
 
 static const float BETA = 0.0f;
 
+// one position per non-blank line; false (with the line number on stderr) at the first line that is not TPS
+static bool read_positions(const std::string& path, int board, std::vector<tz_state_t>* out) {
+    std::ifstream in(path);
+    if (!in) {
+        std::fprintf(stderr, "analysis: cannot read %s\n", path.c_str());
+        return false;
+    }
+    std::string line;
+    for (int no = 1; std::getline(in, line); no++) {
+        const size_t a = line.find_first_not_of(" \t\r\n"), b = line.find_last_not_of(" \t\r\n");
+        if (a == std::string::npos) continue;
+        tz_state_t env;
+        if (!parse_tps(line.substr(a, b - a + 1), board, &env)) {
+            std::fprintf(stderr, "analysis: %s line %d is not valid TPS\n", path.c_str(), no);
+            return false;
+        }
+        out->push_back(env);
+    }
+    if (out->empty()) {
+        std::fprintf(stderr, "analysis: %s holds no position\n", path.c_str());
+        return false;
+    }
+    return true;
+}
+
+static int analyse_positions(const std::vector<tz_state_t>& envs, int board, int half_komi, int device,
+                             unsigned arena_slots, int batch_size, int batches, const std::string& model_path) {
+    const int count = (int)envs.size();
+    BatchedMCTS mcts(board, half_komi, count, device, 0, arena_slots, count * batch_size);
+    if (!model_path.empty()) {
+        mcts.load_model(model_path);
+        mcts.set_agent(TZ_AGENT_NETWORK);
+    }
+    mcts.set_positions(envs);
+    for (int k = 0; k < batches; k++) mcts.trees_simulate_batch(BETA, batch_size);
+    const std::vector<std::vector<Move>> pv = mcts.trees_principal_variation();
+    for (int g = 0; g < count; g++) {
+        std::cout << "tps: " << tps(envs[g], board) << "\n" << node_display(mcts, g) << "pv:";
+        for (Move m : pv[g]) std::cout << ' ' << move_to_string(m);
+        std::cout << "\n";
+    }
+    return 0;
+}
+
 int main(int argc, char** argv) {
     int board = 6, half_komi = 4, device = 0, batch_size = 128;
     unsigned arena_slots = 1u << 22;
-    std::string model_path, tps_text;
+    std::string model_path, tps_text, positions_path;
+    int batches = -1;
     bool example = false;
     for (int i = 1; i < argc; i++) {
         const std::string k = argv[i];
@@ -39,9 +90,29 @@ int main(int argc, char** argv) {
         else if (k == "--device") device = std::atoi(v);
         else if (k == "--batch-size") batch_size = std::atoi(v);
         else if (k == "--arena-slots") arena_slots = (unsigned)std::atoi(v);
+        else if (k == "--positions") positions_path = v;
+        else if (k == "--batches") batches = std::atoi(v);
         else {
             std::fprintf(stderr, "unknown flag %s\n", k.c_str());
             return 2;
+        }
+    }
+    if (!positions_path.empty() || batches >= 0) {
+        if (positions_path.empty() || batches < 1 || example || !tps_text.empty()) {
+            std::fprintf(stderr, "analysis: --positions FILE needs --batches K >= 1 and neither --example nor --tps\n");
+            return 2;
+        }
+        if (board < 3 || board > 6 || batch_size < 1) {
+            std::fprintf(stderr, "analysis: --board must be 3..6 and --batch-size >= 1\n");
+            return 2;
+        }
+        std::vector<tz_state_t> envs;
+        if (!read_positions(positions_path, board, &envs)) return 2;
+        try {
+            return analyse_positions(envs, board, half_komi, device, arena_slots, batch_size, batches, model_path);
+        } catch (const std::exception& e) {
+            std::fprintf(stderr, "analysis: %s\n", e.what());
+            return 1;
         }
     }
     try {

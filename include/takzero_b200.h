@@ -90,7 +90,7 @@ typedef struct tz_config_t {
     int reversible_limit;  /* reversible-ply draw threshold; 0 = default 100 (unpinned, see DESIGN.md) */
     int move_stride;       /* row stride of per-game move/logit tables; 0 = default for board_n */
     uint32_t arena_slots;  /* node slots per game per arena half; 0 = sized from free HBM */
-    int tree_batch;        /* single-tree use (tz_tree_*): leaves per network batch; 0 = n_games */
+    int tree_batch;        /* search trees (tz_tree_*, tz_trees_*): leaves per network batch, all trees; 0 = n_games */
 } tz_config_t;
 
 typedef struct tz_handle tz_handle;
@@ -310,12 +310,24 @@ TZ_API int tz_timer_start(tz_handle* h);
 TZ_API int tz_timer_stop(tz_handle* h, double* out_ms);
 
 /* ---- single tree (tei/src/main.rs:139-290, analysis/src/main.rs): the tree and position are game 0 of the
- * handle (tz_set_positions / tz_reset_roots); batch_size <= n_games. ------------------------------------------ */
+ * handle (tz_set_positions / tz_reset_roots); batch_size <= max(n_games, tree_batch). -------------------------- */
 TZ_API int tz_tree_simulate_simple(tz_handle* h, float beta);                 /* Node::simulate_simple (mcts.rs:235-266) */
 TZ_API int tz_tree_simulate_batch(tz_handle* h, float beta, int batch_size);  /* Node::simulate_batch (mcts.rs:268-328) */
 TZ_API int tz_tree_descend(tz_handle* h, tz_move_t move);                     /* Node::descend + env.step (tree reuse) */
 /* Node::principal_variation (node/mod.rs:40-62); returns the length written to out_moves */
 TZ_API int tz_tree_principal_variation(tz_handle* h, tz_move_t* out_moves, int cap);
+
+/* ---- many single trees at once: the tree of every selected game (mask [n_games], NULL = every game), each with the
+ * single-tree semantics above, searched side by side.  A mask that selects no game is a no-op.  Like tz_tree_*,
+ * these calls make pending self-play records stale. ---------------------------------------------------------------- */
+/* Node::simulate_batch (mcts.rs:268-328) on every selected game's tree at once: each tree gets up to batch_size leaves
+ * (4 * batch_size forwards), one network batch for all of them.  Selected games * batch_size <= max(n_games, tree_batch). */
+TZ_API int tz_trees_simulate_batch(tz_handle* h, const uint8_t* mask, float beta, int batch_size);
+/* Node::descend + env.step per selected game (moves [n_games]; entries of unselected games are ignored) */
+TZ_API int tz_trees_descend(tz_handle* h, const uint8_t* mask, const tz_move_t* moves);
+/* Node::principal_variation per game: out_moves [n_games][cap], out_len [n_games] (0 for unselected games); entries of
+ * out_moves past a game's length are left as they were */
+TZ_API int tz_trees_principal_variation(tz_handle* h, const uint8_t* mask, int cap, tz_move_t* out_moves, int* out_len);
 
 /* ---- network (takzero/src/network/{net4_simhash,net5,net6_simhash,residual,repr}.rs) ----------- */
 /* Net::load (network/mod.rs:16-35): f32 tensors in PyTorch layout, named

@@ -744,6 +744,23 @@ class BatchedMCTS {
         pv.resize(len);
         return pv;
     }
+    // ---- many single trees at once: the tree of every game with mask[g] != 0 (all: empty mask) ----
+    void trees_simulate_batch(float beta, int batch_size, const std::vector<uint8_t>& mask = {}) {
+        check(tz_trees_simulate_batch(h_, mask.empty() ? nullptr : mask.data(), beta, batch_size));
+    }
+    // moves [n_games]; unselected games' entries are ignored
+    void trees_descend(const std::vector<Move>& moves, const std::vector<uint8_t>& mask = {}) {
+        check(tz_trees_descend(h_, mask.empty() ? nullptr : mask.data(), moves.data()));
+    }
+    // one principal variation per game (empty for unselected games)
+    std::vector<std::vector<Move>> trees_principal_variation(int cap = 64, const std::vector<uint8_t>& mask = {}) {
+        std::vector<Move> buf((size_t)games_ * cap);
+        std::vector<int> len(games_);
+        check(tz_trees_principal_variation(h_, mask.empty() ? nullptr : mask.data(), cap, buf.data(), len.data()));
+        std::vector<std::vector<Move>> pv(games_);
+        for (int g = 0; g < games_; g++) pv[g].assign(buf.begin() + (size_t)g * cap, buf.begin() + (size_t)g * cap + len[g]);
+        return pv;
+    }
     tz_counters_t counters() {
         tz_counters_t c;
         check(tz_counters(h_, &c));

@@ -195,6 +195,9 @@ def lib():
         "tz_debug_tree_warps": ([vp, i32], i32),
         "tz_tree_descend": ([vp, C.c_uint16], i32),
         "tz_tree_principal_variation": ([vp, vp, i32], i32),
+        "tz_trees_simulate_batch": ([vp, vp, f32, i32], i32),
+        "tz_trees_descend": ([vp, vp, vp], i32),
+        "tz_trees_principal_variation": ([vp, vp, i32, vp, vp], i32),
         "tz_selfplay_move": ([vp, P(SelfplayParams)], i32),
         "tz_launch_count": ([vp, P(u64)], i32),
         "tz_selfplay_record": ([vp, i32, C.c_size_t, C.c_size_t], i32),
@@ -483,6 +486,27 @@ class BatchedMCTS:
         out = np.zeros(cap, dtype=np.uint16)
         n = _check(lib().tz_tree_principal_variation(self._h, _ptr(out), cap))
         return out[:n].copy()
+
+    # ---- many single trees at once: the tree of every selected game (mask [G], None = every game) ----
+    def trees_simulate_batch(self, beta: float, batch_size: int, mask=None) -> None:
+        """Node::simulate_batch on every selected game's tree, one network batch for all of them
+        (selected games * batch_size <= max(n_games, tree_batch))."""
+        m = None if mask is None else _arr(mask, np.uint8, (self.G,))
+        _check(lib().tz_trees_simulate_batch(self._h, _ptr(m), beta, batch_size))
+
+    def trees_descend(self, moves, mask=None) -> None:
+        """Node::descend + env.step of every selected game (moves [G]; unselected games' entries are ignored)."""
+        mv = _arr(moves, np.uint16, (self.G,))
+        m = None if mask is None else _arr(mask, np.uint8, (self.G,))
+        _check(lib().tz_trees_descend(self._h, _ptr(m), _ptr(mv)))
+
+    def trees_principal_variation(self, cap: int = 64, mask=None):
+        """Per game: (moves [G][cap] uint16, lengths [G] int32); length 0 for unselected games."""
+        m = None if mask is None else _arr(mask, np.uint8, (self.G,))
+        out = np.zeros((self.G, cap), dtype=np.uint16)
+        n = np.zeros(self.G, dtype=np.int32)
+        _check(lib().tz_trees_principal_variation(self._h, _ptr(m), cap, _ptr(out), _ptr(n)))
+        return out, n
 
     def selfplay_move(self, params: SelfplayParams) -> None:
         """One whole self-play move on the device, asynchronous (see tz_selfplay_move)."""

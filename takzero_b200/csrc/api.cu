@@ -8,6 +8,7 @@
 #include <stdlib.h>
 #include <string.h>
 
+#include <algorithm>
 #include <vector>
 
 #include "../../include/takzero_b200.h"
@@ -172,6 +173,9 @@ extern "C" TZ_API int tz_create(const tz_config_t* cfg, tz_handle** out) {
     DM(d.logits, Q * d.M);
     DM(d.value, Q);
     DM(d.variance, Q);
+    DM(d.tree_game, G);
+    DM(d.tree_fill, G);
+    DM(d.tree_slot, Q);
     float* ln_table = nullptr;
     DM(ln_table, (size_t)TZ_LN_TABLE);
     DM(d.set_child, G * TZ_MAX_K);
@@ -1482,58 +1486,130 @@ extern "C" TZ_API int tz_read_novelty_set(tz_handle* h, uint8_t* out, size_t cap
     return TZ_OK;
 }
 
-// ---- single tree (tei / analysis): Node::simulate_simple, simulate_batch, descend, principal_variation ----
-// The tree is game 0 of the handle; batch_size <= n_games because the per-leaf paths reuse the per-game buffers.
+// ---- search trees (tei / analysis): Node::simulate_simple, simulate_batch, descend, principal_variation ----
+// The trees of a call are its selected games, tree t the t-th of them in game order; one CTA (one warp for the PV) per
+// tree.  The tz_tree_* calls are the same code with game 0 selected.
 
-static int tree_simulate(tz_handle* h, float beta, int batch_size, int max_forwards) {
+static std::vector<int> selected_games(const tz_handle* h, const uint8_t* mask) {
+    std::vector<int> games;
+    for (int g = 0; g < h->d.G; g++)
+        if (!mask || mask[g]) games.push_back(g);
+    return games;
+}
+
+// d.tree_game = games (copied only when it changed: the one-tree calls select game 0 every time)
+static int upload_trees(tz_handle* h, const std::vector<int>& games) {
+    if (games == h->tree_games) return TZ_OK;
+    h->tree_games.clear();  // stays empty if the copy fails
+    CU(cudaMemcpyAsync(h->d.tree_game, games.data(), games.size() * sizeof(int), cudaMemcpyHostToDevice, h->stream));
+    h->tree_games = games;
+    return TZ_OK;
+}
+
+static int trees_simulate(tz_handle* h, const std::vector<int>& games, float beta, int batch_size, int max_forwards) {
     const TzDev& d = h->d;
+    const int trees = (int)games.size();
+    if (batch_size <= 0) return fail(TZ_EINVAL, "batch_size must be >= 1");
+    if ((long long)trees * batch_size > d.Q)
+        return fail(TZ_EINVAL, "selected games (%d) x batch_size (%d) must be <= max(n_games, tree_batch) (%d): raise tree_batch",
+                    trees, batch_size, d.Q);
+    if (trees == 0) return TZ_OK;
     h->rec_stale = true;
-    if (batch_size <= 0 || batch_size > d.Q)
-        return fail(TZ_EINVAL, "batch_size must be 1..max(n_games, tree_batch) (%d)", d.Q);
-    h->prof_active = false;
-    launch_tree_forward(d, beta, batch_size, max_forwards, h->dbg_tree_warps, h->stream);
-    int rc = run_agent(h);
+    int rc = upload_trees(h, games);
     if (rc) return rc;
-    launch_tree_backward(d, h->dbg_tree_warps, h->stream);
+    h->prof_active = false;
+    CU(cudaMemsetAsync(d.nn_count, 0, sizeof(int), h->stream));  // the trees append their leaves
+    launch_tree_forward(d, trees, beta, batch_size, max_forwards, h->dbg_tree_warps, h->stream);
+    rc = run_agent(h);
+    if (rc) return rc;
+    launch_tree_backward(d, trees, batch_size, h->dbg_tree_warps, h->stream);
     h->launches += 2;
     return finish(h);
 }
 
 extern "C" TZ_API int tz_tree_simulate_simple(tz_handle* h, float beta) {
     CHECK_H(h);
-    return tree_simulate(h, beta, 1, 1);  // mcts.rs:235-266
+    return trees_simulate(h, {0}, beta, 1, 1);  // mcts.rs:235-266
 }
 
 extern "C" TZ_API int tz_tree_simulate_batch(tz_handle* h, float beta, int batch_size) {
     CHECK_H(h);
-    return tree_simulate(h, beta, batch_size, 4 * batch_size);  // mcts.rs:268-328
+    return trees_simulate(h, {0}, beta, batch_size, 4 * batch_size);  // mcts.rs:268-328
+}
+
+extern "C" TZ_API int tz_trees_simulate_batch(tz_handle* h, const uint8_t* mask, float beta, int batch_size) {
+    CHECK_H(h);
+    return trees_simulate(h, selected_games(h, mask), beta, batch_size, 4 * batch_size);
+}
+
+extern "C" TZ_API int tz_trees_descend(tz_handle* h, const uint8_t* mask, const tz_move_t* moves) {
+    CHECK_H(h);
+    if (!moves) return fail(TZ_EINVAL, "null moves");
+    if (selected_games(h, mask).empty()) return TZ_OK;
+    h->rec_stale = true;
+    const uint8_t* dmask;
+    int rc = upload_mask(h, mask, &dmask);
+    if (rc) return rc;
+    CU(cudaMemcpyAsync(h->moves, moves, (size_t)h->d.G * sizeof(uint16_t), cudaMemcpyHostToDevice, h->stream));
+    launch_step(h->d, h->moves, h->stream, dmask);
+    h->launches += 1;
+    return finish(h);
 }
 
 extern "C" TZ_API int tz_tree_descend(tz_handle* h, tz_move_t move) {
     CHECK_H(h);
-    h->rec_stale = true;
     std::vector<uint16_t> mv((size_t)h->d.G, 0);
+    std::vector<uint8_t> mask((size_t)h->d.G, 0);
     mv[0] = move;
-    CU(cudaMemcpyAsync(h->moves, mv.data(), mv.size() * sizeof(uint16_t), cudaMemcpyHostToDevice, h->stream));
-    launch_step(h->d, h->moves, h->stream, 0);
-    h->launches += 1;
-    return finish(h);
+    mask[0] = 1;
+    return tz_trees_descend(h, mask.data(), mv.data());
+}
+
+// principal variations of the trees of `games`: moves [trees][cap] (cap <= move_stride), lens [trees]
+static int trees_pv(tz_handle* h, const std::vector<int>& games, int cap, std::vector<uint16_t>* moves, std::vector<int>* lens) {
+    const int trees = (int)games.size();
+    int rc = upload_trees(h, games);
+    if (rc) return rc;
+    launch_tree_pv(h->d, trees, h->tbl_moves, cap, h->tbl_n, h->stream);
+    moves->resize((size_t)trees * cap);
+    lens->resize(trees);
+    CU(cudaMemcpyAsync(moves->data(), h->tbl_moves, moves->size() * sizeof(uint16_t), cudaMemcpyDeviceToHost, h->stream));
+    CU(cudaMemcpyAsync(lens->data(), h->tbl_n, (size_t)trees * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+    CU(cudaStreamSynchronize(h->stream));
+    CU(cudaGetLastError());
+    return TZ_OK;
 }
 
 extern "C" TZ_API int tz_tree_principal_variation(tz_handle* h, tz_move_t* out_moves, int cap) {
     CHECK_H(h);
     if (!out_moves || cap <= 0) return fail(TZ_EINVAL, "bad argument");
     if (cap > h->d.M) cap = h->d.M;
-    launch_tree_pv(h->d, h->tbl_moves, cap, h->tbl_n, h->stream);
-    int* len = (int*)(h->pin_small + 192);
-    CU(cudaMemcpyAsync(len, h->tbl_n, sizeof(int), cudaMemcpyDeviceToHost, h->stream));
-    CU(cudaStreamSynchronize(h->stream));
-    if (*len > 0) {
-        CU(cudaMemcpyAsync(out_moves, h->tbl_moves, (size_t)*len * sizeof(uint16_t), cudaMemcpyDeviceToHost, h->stream));
-        CU(cudaStreamSynchronize(h->stream));
+    std::vector<uint16_t> moves;
+    std::vector<int> lens;
+    const int rc = trees_pv(h, {0}, cap, &moves, &lens);
+    if (rc) return rc;
+    std::copy(moves.begin(), moves.begin() + lens[0], out_moves);
+    return lens[0];
+}
+
+extern "C" TZ_API int tz_trees_principal_variation(tz_handle* h, const uint8_t* mask, int cap, tz_move_t* out_moves,
+                                                   int* out_len) {
+    CHECK_H(h);
+    if (!out_moves || !out_len || cap <= 0) return fail(TZ_EINVAL, "bad argument");
+    const std::vector<int> games = selected_games(h, mask);
+    std::fill(out_len, out_len + h->d.G, 0);
+    if (games.empty()) return TZ_OK;
+    const int dcap = cap < h->d.M ? cap : h->d.M;
+    std::vector<uint16_t> moves;
+    std::vector<int> lens;
+    const int rc = trees_pv(h, games, dcap, &moves, &lens);
+    if (rc) return rc;
+    for (size_t t = 0; t < games.size(); t++) {
+        const int g = games[t];
+        std::copy(moves.begin() + t * dcap, moves.begin() + t * dcap + lens[t], out_moves + (size_t)g * cap);
+        out_len[g] = lens[t];
     }
-    CU(cudaGetLastError());
-    return *len;
+    return TZ_OK;
 }
 
 // BatchedMCTS::apply_noise (batched.rs:146-151) support: store host-computed priors / logits of the roots

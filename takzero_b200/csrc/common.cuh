@@ -91,8 +91,8 @@ struct TzDev {
     uint16_t* replay;    // [G][TZ_MAX_PLIES] moves played since start_env
     int* replay_len;     // [G]
     // one lock-step simulation
-    uint32_t* traj;      // [G][TZ_MAX_DEPTH] node slots of the selection path
-    int* traj_len;       // [G]
+    uint32_t* traj;      // [Q][TZ_MAX_DEPTH] node slots of the selection path: by game (k_select), by queue slot (k_tree_*)
+    int* traj_len;       // [Q] same index
     int* nn_queue;       // [G] evaluation-queue slot -> game
     int* nn_count;       // [1] queue length
     TzState* leaf_state; // [G] leaf positions, by queue slot
@@ -112,6 +112,10 @@ struct TzDev {
     const uint32_t* nn_novelty_idx;  // [Q] hash index of every queued position
     const float* nn_rnd_unc;         // [Q] normalized RND uncertainty of every queued position (net5), or null
     const float* ln_table;  // exploration_rate(n), n < TZ_LN_TABLE (host libm logf)
+    // search trees (k_tree_*, one CTA per tree)
+    int* tree_game;  // [G] game of tree t
+    int* tree_fill;  // [G] leaves tree t queued in the last forward
+    int* tree_slot;  // [Q] queue slot of tree t's i-th leaf (commit order) at t * batch_size + i
     // sequential halving
     uint16_t* set_child;  // [G][TZ_MAX_K] candidate set (root child index)
     float* set_key;       // [G][TZ_MAX_K] logit + gumbel

@@ -27,7 +27,8 @@ struct tz_handle {
     int dbg_per_layer = 0;     // one launch per convolution instead of the fused launch
     int dbg_chunk_tiles = -1;  // minimum pair tiles per chunk (-1: default 150, 0: one chunk)
     int dbg_drop_progress = 0; // CTA pair 0 withholds its tiles (watchdog test)
-    int dbg_tree_warps = 0;    // warps of the single-tree wavefront kernels (0: default)
+    int dbg_tree_warps = 0;    // warps of the search-tree wavefront kernels (0: default)
+    std::vector<int> tree_games;  // what d.tree_game holds (the games of the last tz_tree* call)
     // device staging of host-facing arguments / results
     float* betas = nullptr;
     float* gumbel = nullptr;

@@ -346,11 +346,15 @@ __global__ void __launch_bounds__(32 * WPB) k_expand(TzDev d) {
     warp_expand(d, g, q, d.traj + (size_t)g * TZ_MAX_DEPTH, d.traj_len[g], s_p[warp], lane);
 }
 
-// ---- single tree: Node::simulate_simple / simulate_batch (mcts.rs:235-328) on game 0 -------------------------
+// ---- search trees: Node::simulate_simple / simulate_batch (mcts.rs:235-328), one CTA per tree ------------------
 
 // Up to `max_forwards` descents of ONE tree with the reference's SEQUENTIAL semantics: the visit increments of earlier
-// descents steer later ones (its only "virtual loss"), known results are backed up at once, leaves that need the
-// network fill queue slots 0..batch_size-1 in order, their paths go to traj[q].
+// descents steer later ones (its only "virtual loss"), known results are backed up at once, up to batch_size leaves
+// need the network.  CTA t searches the tree of game d.tree_game[t]; the trees of one launch share nothing but the
+// evaluation queue.  Each leaf takes a queue slot q of its own (atomicAdd on nn_count, after its commit, so the queue
+// is dense over all trees in some order), its path goes to traj[q], and d.tree_slot[t * batch_size + i] = q records
+// the tree's i-th leaf in commit order, d.tree_fill[t] how many there are: k_tree_backward walks them in that order.
+// Which slot a leaf lands in does not change its network outputs (DESIGN §5), so neither does the order across trees.
 //
 // One warp doing them one after the other is bound by the latency of its own dependent loads (~12 us per descent), so
 // TREE_WARPS warps of one CTA run consecutive descents as a wavefront, speculatively, and commit them in order:
@@ -534,6 +538,7 @@ struct TreeForwardSmem {
 };
 
 __global__ void __launch_bounds__(32 * TREE_WARPS) k_tree_forward(TzDev d, float beta, int batch_size, int max_forwards) {
+    const int tree = blockIdx.x, g = d.tree_game[tree];
     extern __shared__ __align__(128) unsigned char tree_smem[];
     TreeForwardSmem& sm = *reinterpret_cast<TreeForwardSmem*>(tree_smem);
     TzState* s_state = sm.state;
@@ -554,10 +559,10 @@ __global__ void __launch_bounds__(32 * TREE_WARPS) k_tree_forward(TzDev d, float
     c.stop = s_ctl + 5;
     if (threadIdx.x < 6) s_ctl[threadIdx.x] = 0;
     if (lane == 0) s_fprog[warp] = -1;
-    if (threadIdx.x == 0) *d.nn_count = 0;  // the committing warp that ends the batch writes the real count
+    if (threadIdx.x == 0) d.tree_fill[tree] = 0;  // the committing warp that ends the batch writes the real count
     __syncthreads();
-    const GameTree t = game_tree(d.arena, 0);
-    unsigned long long* ctr = d.counters;
+    const GameTree t = game_tree(d.arena, g);
+    unsigned long long* ctr = d.counters + (size_t)g * 4;  // only the committing warp touches the tree's counters
     TzState* st = &s_state[warp];
     uint32_t* traj = s_traj[warp];
     if (max_forwards <= 0 || batch_size <= 0) return;
@@ -596,7 +601,7 @@ __global__ void __launch_bounds__(32 * TREE_WARPS) k_tree_forward(TzDev d, float
         __threadfence_block();
         if (stopped) return;
         tree_fpublish(c, it, 0, lane);
-        warp_load_state(st, &d.env[0], lane);
+        warp_load_state(st, &d.env[g], lane);
         int len = 0;
         Ev known_ev = ev_value(0.0f);
         uint32_t err_bit = 0, undo_slot = 0xffffffffu, undo_words[3] = {0, 0, 0};
@@ -669,7 +674,7 @@ __global__ void __launch_bounds__(32 * TREE_WARPS) k_tree_forward(TzDev d, float
         if (lane == 0) {
             *c.filled = filled;
             if (stop) {
-                *d.nn_count = filled;
+                d.tree_fill[tree] = filled;
                 *c.stop = 1;
                 __threadfence_block();
                 if (res != TREE_KNOWN) *c.gen = my_gen + 1;  // whoever is still descending gives up and takes it back
@@ -680,23 +685,24 @@ __global__ void __launch_bounds__(32 * TREE_WARPS) k_tree_forward(TzDev d, float
             }
         }
         __syncwarp();
-        if (res == TREE_NEEDS) {
-            // queue entry q is this descent's alone from here on: filling it keeps nobody waiting
-            const bool too_many = cnt < 0 || cnt > d.M;  // reported, never truncated (warp_enqueue): an entry without moves
+        if (res == TREE_NEEDS && filled > q) {
+            // the tree's entry q is this descent's alone from here on: taking a queue slot and filling it keeps nobody
+            // waiting.  (A leaf with too many moves is reported, never truncated, and gets no entry: it ended the batch.)
+            int slot = 0;
             if (lane == 0) {
-                d.nn_queue[q] = 0;
-                d.n_actions[q] = too_many ? 0 : cnt;
-                d.traj_len[q] = len;
+                slot = atomicAdd(d.nn_count, 1);
+                d.tree_slot[(size_t)tree * batch_size + q] = slot;
+                d.nn_queue[slot] = g;
+                d.n_actions[slot] = cnt;
+                d.traj_len[slot] = len;
             }
-            for (int sq = lane; sq < TZ_MAX_SQ; sq += 32)
-                d.sq_ranges[(size_t)q * TZ_MAX_SQ + sq] = too_many ? 0u : s_ranges[warp][sq];
-            warp_store_state(&d.leaf_state[q], st, lane);
-            if (!too_many) {
-                uint16_t* out = d.actions + (size_t)q * d.M;
-                for (int i = lane; i < cnt; i += 32) out[i] = s_moves[warp][i];
-                uint32_t* tq = d.traj + (size_t)q * TZ_MAX_DEPTH;
-                for (int i = lane; i < len; i += 32) tq[i] = traj[i];
-            }
+            slot = __shfl_sync(FULL_MASK, slot, 0);
+            for (int sq = lane; sq < TZ_MAX_SQ; sq += 32) d.sq_ranges[(size_t)slot * TZ_MAX_SQ + sq] = s_ranges[warp][sq];
+            warp_store_state(&d.leaf_state[slot], st, lane);
+            uint16_t* out = d.actions + (size_t)slot * d.M;
+            for (int i = lane; i < cnt; i += 32) out[i] = s_moves[warp][i];
+            uint32_t* tq = d.traj + (size_t)slot * TZ_MAX_DEPTH;
+            for (int i = lane; i < len; i += 32) tq[i] = traj[i];
             __syncwarp();
         }
         if (stop) return;
@@ -704,8 +710,9 @@ __global__ void __launch_bounds__(32 * TREE_WARPS) k_tree_forward(TzDev d, float
     }
 }
 
-// backward_network_eval of the queued leaves IN QUEUE ORDER (they share one tree: every running mean and every solver
-// scan sees what the earlier leaves of the batch left), by TREE_WARPS warps of one CTA as a wavefront:
+// backward_network_eval of one tree's queued leaves IN ITS COMMIT ORDER (they share the tree: every running mean and
+// every solver scan sees what the earlier leaves of the batch left), by TREE_WARPS warps of the tree's CTA as a wavefront
+// (entry q below is the tree's q-th leaf, at queue slot d.tree_slot[t * batch_size + q]):
 //   * the heads, the softmax and the sanitising of an entry touch nothing shared and run at once for TREE_WARPS entries;
 //   * entry q works on depth e of its path (leaf step at e = len-1, then the parents up to the root at 0) in two halves:
 //     it READS the node at depth e and its children at depth e+1 once entry q-1 has finished depth e (by induction so
@@ -748,28 +755,31 @@ struct TreeBackwardSmem {
     int prog[TREE_WARPS];
 };
 
-__global__ void __launch_bounds__(32 * TREE_WARPS) k_tree_backward(TzDev d) {
+__global__ void __launch_bounds__(32 * TREE_WARPS) k_tree_backward(TzDev d, int batch_size) {
     extern __shared__ __align__(128) unsigned char tree_smem[];
     TreeBackwardSmem& sm = *reinterpret_cast<TreeBackwardSmem*>(tree_smem);
     float(*s_p)[TZ_MAX_MOVES] = sm.p;
     int* s_prog = sm.prog;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int count = *d.nn_count;
+    const int tree = blockIdx.x, g = d.tree_game[tree];
+    const int count = d.tree_fill[tree];
+    const int* slots = d.tree_slot + (size_t)tree * batch_size;
     volatile int* prog = s_prog;
     if (lane == 0) s_prog[warp] = -1;
     __syncthreads();
-    const GameTree t = game_tree(d.arena, 0);
+    const GameTree t = game_tree(d.arena, g);
     const int nw = blockDim.x >> 5;
     for (int q = warp; q < count; q += nw) {
-        const uint32_t* traj = d.traj + (size_t)q * TZ_MAX_DEPTH;
-        const int len = d.traj_len[q];
-        const LeafOutputs o = expand_outputs(d, q, s_p[warp], lane);
+        const int slot = slots[q];
+        const uint32_t* traj = d.traj + (size_t)slot * TZ_MAX_DEPTH;
+        const int len = d.traj_len[slot];
+        const LeafOutputs o = expand_outputs(d, slot, s_p[warp], lane);
         const uint32_t leaf = traj[len - 1];
         LeafUpdate u;
         bool ok = tree_wait_pred(d, prog, nw, q, len - 1, lane);  // reads at the leaf's depth
-        ok = ok && expand_leaf_children(d, 0, q, leaf, s_p[warp], o, lane, &u);
+        ok = ok && expand_leaf_children(d, g, slot, leaf, s_p[warp], o, lane, &u);
         ok = tree_wait_pred(d, prog, nw, q, len - 2, lane) && ok;  // stores at the leaf's depth
-        if (ok) expand_leaf_store(d, 0, q, leaf, u, lane);
+        if (ok) expand_leaf_store(d, g, slot, leaf, u, lane);
         Propagated pr = expand_propagated(o);
         for (int e = len - 2; ok && e >= 0; e--) {
             tree_publish(prog, nw, q, e + 1, lane);
@@ -976,12 +986,12 @@ __device__ __forceinline__ bool warp_apply_checked(TzState* st, int n, uint16_t 
     return warp_apply(st, n, mv, lane);
 }
 
-__global__ void __launch_bounds__(32 * WPB) k_step(TzDev d, const uint16_t* moves, int only_game) {
+__global__ void __launch_bounds__(32 * WPB) k_step(TzDev d, const uint16_t* moves, const uint8_t* mask) {
     __shared__ TzState s_state[WPB];
     __shared__ uint16_t s_moves[WPB][TZ_MAX_MOVES];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int g = blockIdx.x * WPB + warp;
-    if (g >= d.G || (only_game >= 0 && g != only_game)) return;
+    if (g >= d.G || (mask && !mask[g])) return;
     const int half = d.arena.half[g];
     const GameTree src = game_tree_half(d.arena, g, half);
     const uint32_t rmeta = src.meta[0];
@@ -1471,10 +1481,12 @@ __global__ void k_merge_moves(TzDev d, int weighted_random_plies, const uint16_t
     if ((int)d.env[g].ply < weighted_random_plies) moves[g] = sampled[g];
 }
 
-// Node::principal_variation (node/mod.rs:40-62) of game 0's tree
+// Node::principal_variation (node/mod.rs:40-62), one warp per tree: game d.tree_game[t] -> out_moves[t][cap], out_len[t]
 __global__ void __launch_bounds__(32) k_tree_pv(TzDev d, uint16_t* out_moves, int cap, int* out_len) {
     const int lane = threadIdx.x & 31;
-    const GameTree t = game_tree(d.arena, 0);
+    const GameTree t = game_tree(d.arena, d.tree_game[blockIdx.x]);
+    out_moves += (size_t)blockIdx.x * cap;
+    out_len += blockIdx.x;
     uint32_t slot = 0;
     int len = 0;
     while (len < cap) {
@@ -1823,28 +1835,29 @@ void launch_halve(const TzDev& d, const float* betas, float visits, int remainin
 void launch_finalize(const TzDev& d, uint16_t* out_moves, cudaStream_t st) {
     k_finalize<<<blocks_for(d.G), 32 * WPB, 0, st>>>(d, out_moves);
 }
-void launch_step(const TzDev& d, const uint16_t* moves, cudaStream_t st, int only_game) {
-    k_step<<<blocks_for(d.G), 32 * WPB, 0, st>>>(d, moves, only_game);
+void launch_step(const TzDev& d, const uint16_t* moves, cudaStream_t st, const uint8_t* mask) {
+    k_step<<<blocks_for(d.G), 32 * WPB, 0, st>>>(d, moves, mask);
 }
 static int tree_warps(int warps) { return warps >= 1 && warps <= TREE_WARPS ? warps : TREE_WARPS; }
 
-void launch_tree_forward(const TzDev& d, float beta, int batch_size, int max_forwards, int warps, cudaStream_t st) {
+void launch_tree_forward(const TzDev& d, int trees, float beta, int batch_size, int max_forwards, int warps,
+                         cudaStream_t st) {
     static const cudaError_t attr = cudaFuncSetAttribute(k_tree_forward, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                                         (int)sizeof(TreeForwardSmem));
     (void)attr;
-    k_tree_forward<<<1, 32 * tree_warps(warps), sizeof(TreeForwardSmem), st>>>(d, beta, batch_size, max_forwards);
+    k_tree_forward<<<trees, 32 * tree_warps(warps), sizeof(TreeForwardSmem), st>>>(d, beta, batch_size, max_forwards);
 }
-void launch_tree_backward(const TzDev& d, int warps, cudaStream_t st) {
+void launch_tree_backward(const TzDev& d, int trees, int batch_size, int warps, cudaStream_t st) {
     static const cudaError_t attr = cudaFuncSetAttribute(k_tree_backward, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                                         (int)sizeof(TreeBackwardSmem));
     (void)attr;
-    k_tree_backward<<<1, 32 * tree_warps(warps), sizeof(TreeBackwardSmem), st>>>(d);
+    k_tree_backward<<<trees, 32 * tree_warps(warps), sizeof(TreeBackwardSmem), st>>>(d, batch_size);
 }
 void launch_set_root_priors(const TzDev& d, int stride, const float* prob, const float* logit, cudaStream_t st) {
     k_set_root_priors<<<blocks_for(d.G), 32 * WPB, 0, st>>>(d, stride, prob, logit);
 }
-void launch_tree_pv(const TzDev& d, uint16_t* out_moves, int cap, int* out_len, cudaStream_t st) {
-    k_tree_pv<<<1, 32, 0, st>>>(d, out_moves, cap, out_len);
+void launch_tree_pv(const TzDev& d, int trees, uint16_t* out_moves, int cap, int* out_len, cudaStream_t st) {
+    k_tree_pv<<<trees, 32, 0, st>>>(d, out_moves, cap, out_len);
 }
 void launch_new_openings(const TzDev& d, const uint8_t* mask, const int* sym, const int* adj, unsigned long long seed,
                          unsigned long long counter, cudaStream_t st) {

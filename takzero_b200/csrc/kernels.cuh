@@ -10,10 +10,14 @@ void launch_gumbel_noise(const TzDev& d, float* out, int stride, unsigned long l
 void launch_gumbel_init(const TzDev& d, int k, const float* gumbel, int stride, cudaStream_t st);
 void launch_halve(const TzDev& d, const float* betas, float visits, int remaining, cudaStream_t st);
 void launch_finalize(const TzDev& d, uint16_t* out_moves, cudaStream_t st);
-void launch_step(const TzDev& d, const uint16_t* moves, cudaStream_t st, int only_game = -1);
-void launch_tree_forward(const TzDev& d, float beta, int batch_size, int max_forwards, int warps, cudaStream_t st);
-void launch_tree_backward(const TzDev& d, int warps, cudaStream_t st);
-void launch_tree_pv(const TzDev& d, uint16_t* out_moves, int cap, int* out_len, cudaStream_t st);
+// k_step on the games with mask[g] != 0 (all: null)
+void launch_step(const TzDev& d, const uint16_t* moves, cudaStream_t st, const uint8_t* mask = nullptr);
+// search trees (one CTA / warp per tree): tree t is game d.tree_game[t], t < trees.  The forward appends to the
+// evaluation queue, whose count must be zero before the first tree of a batch starts; the backward expands the leaves.
+void launch_tree_forward(const TzDev& d, int trees, float beta, int batch_size, int max_forwards, int warps,
+                         cudaStream_t st);
+void launch_tree_backward(const TzDev& d, int trees, int batch_size, int warps, cudaStream_t st);
+void launch_tree_pv(const TzDev& d, int trees, uint16_t* out_moves, int cap, int* out_len, cudaStream_t st);
 void launch_new_openings(const TzDev& d, const uint8_t* mask, const int* sym, const int* adj, unsigned long long seed,
                          unsigned long long counter, cudaStream_t st);
 void launch_set_positions(const TzDev& d, const TzState* states, const uint8_t* mask, cudaStream_t st);
