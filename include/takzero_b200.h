@@ -361,7 +361,9 @@ TZ_API int tz_comm_destroy(tz_handle* h);
  * (0 = the board's default: 20 for 5x5, else 16); every rank must use the same tz_set_network_dtype.  Tensor data in
  * pinned memory (tz_host_alloc) is uploaded from where it is, asynchronously: leave it unchanged until
  * tz_weight_generation has returned; data in pageable memory is copied into the library's own staging buffer before
- * the call returns (the same holds for tz_set_weights). */
+ * the call returns (the same holds for tz_set_weights).  The RND estimator of a 5x5 model is not part of the image: the
+ * root takes it from its tensors as tz_set_weights does (a model without it switches it off), the other ranks keep
+ * the one they had. */
 TZ_API int tz_broadcast_weights(tz_handle* h, const tz_tensor_t* tensors, int count, int res_blocks, int root);
 /* number of generations so far and the device time of the last one (upload + fold + broadcast); waits for it */
 TZ_API int tz_weight_generation(tz_handle* h, uint64_t* out_generation, double* out_ms);

@@ -848,6 +848,9 @@ int nn_broadcast_weights(tz_handle* h, const char* const* names, const float* co
     if (rank == root) {
         if ((rc = stage_raw(h, ts)) != TZ_OK) return rc;
         if ((rc = upload_and_fold(h, target)) != TZ_OK) return rc;
+        // the root takes the RND estimator as nn_set_weights does (a model without it switches it off); it is not part
+        // of the broadcast set, so the other ranks keep theirs
+        if ((rc = rnd_set_weights(h, names, data, shapes, ndims, count)) != TZ_OK) NN_FAIL(rc, "%s", rnd_last_error());
     } else {
         if (s->swap_recorded && cudaStreamWaitEvent(s->wstream, s->ev_swap, 0) != cudaSuccess) NN_FAIL(TZ_ECUDA, "cudaStreamWaitEvent");
         cudaEventRecord(s->ev_gen[0], s->wstream);
@@ -1083,7 +1086,7 @@ int nn_forward_queue(tz_handle* h) {
         h->launches += launched;
     }
     launch_novelty(h, d.leaf_state, d.nn_count, d.Q);
-    if (rnd_forward(h, d.leaf_state, d.Q) != TZ_OK) return TZ_ECUDA;
+    if (rnd_forward(h, d.leaf_state, d.nn_count, d.Q) != TZ_OK) return TZ_ECUDA;
     return cudaGetLastError() == cudaSuccess ? TZ_OK : TZ_ECUDA;
 }
 
@@ -1112,7 +1115,7 @@ int nn_forward_host(tz_handle* h, int count) {
     h->launches += 1 + launched;
     if (limit >= 0) return cudaGetLastError() == cudaSuccess ? TZ_OK : TZ_ECUDA;
     launch_novelty(h, d.leaf_state, nullptr, count);
-    if (rnd_forward(h, d.leaf_state, count) != TZ_OK) return TZ_ECUDA;
+    if (rnd_forward(h, d.leaf_state, nullptr, count) != TZ_OK) return TZ_ECUDA;
     k_heads<<<wblocks, 32 * WPB, 0, h->stream>>>(s->head_feat, reinterpret_cast<const float*>(s->wset[s->active] + s->lay.head_misc),
                                                  count, d.n, s->simhash_set, s->simhash_idx, rnd_uncertainty(h), d.value, d.variance);
     h->launches += 1;

@@ -93,16 +93,23 @@ void rnd_free(tz_handle* h) {
     h->rnd = nullptr;
 }
 
-// One warp per position: the f32 planes (game_repr order = x.view([-1, input_size])) divided by the sum of their squares
-__global__ void __launch_bounds__(32 * WPB) k_rnd_input(const TzState* states, int count, int n, int half_komi, float* out) {
+// One warp per position: the f32 planes (game_repr order = x.view([-1, input_size])) divided by the sum of their squares.
+// Slots from the device-side count (count_ptr, null = count_max) up to count_max hold no position: their row is zero,
+// so the GEMMs that run over all count_max rows read defined data there.
+__global__ void __launch_bounds__(32 * WPB) k_rnd_input(const TzState* states, const int* count_ptr, int count_max, int n,
+                                                         int half_komi, float* out) {
     __shared__ TzState s_state[WPB];
     __shared__ float s_planes[WPB][36 * 36];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int q = blockIdx.x * WPB + warp;
-    if (q >= count) return;
+    if (q >= count_max) return;
+    const int total = (2 * (2 * n + 3 + 2) + 2) * n * n;
+    if (q >= (count_ptr ? *count_ptr : count_max)) {
+        for (int i = lane; i < total; i += 32) out[(size_t)q * total + i] = 0.0f;
+        return;
+    }
     TzState* st = &s_state[warp];
     warp_load_state(st, &states[q], lane);
-    const int total = (2 * (2 * n + 3 + 2) + 2) * n * n;
     float* x = s_planes[warp];
     warp_fill_planes(x, st, n, half_komi, lane, false);
     float sq = 0.0f;
@@ -122,10 +129,10 @@ __global__ void k_rnd_bias_act(float* y, const float* bias, size_t total, int co
 // One warp per position: sum((learning - target)^2) over the 512 outputs (the final biases are added here),
 // normalized and scaled like `normalized_rnd`
 __global__ void __launch_bounds__(32 * WPB) k_rnd_finish(const float* l, const float* t, const float* bl, const float* bt,
-                                                          int count, float lo, float hi, float* unc) {
+                                                          const int* count_ptr, int count_max, float lo, float hi, float* unc) {
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int q = blockIdx.x * WPB + warp;
-    if (q >= count) return;
+    if (q >= (count_ptr ? *count_ptr : count_max)) return;
     float acc = 0.0f;
     for (int j = lane; j < RND_OUT; j += 32) {
         const float d = (l[(size_t)q * RND_OUT + j] + bl[j]) - (t[(size_t)q * RND_OUT + j] + bt[j]);
@@ -201,14 +208,14 @@ int rnd_set_weights(tz_handle* h, const char* const* names, const float* const* 
     return cudaGetLastError() == cudaSuccess ? TZ_OK : TZ_ECUDA;
 }
 
-int rnd_forward(tz_handle* h, const TzState* states, int count_max) {
+int rnd_forward(tz_handle* h, const TzState* states, const int* count_ptr, int count_max) {
     RndState* s = h->rnd;
     if (!s) return TZ_OK;
     if (count_max > s->max_positions) return TZ_EINVAL;
     const TzDev& d = h->d;
     const int wblocks = (count_max + WPB - 1) / WPB;
     g_cublas.SetStream(s->blas, h->stream);
-    k_rnd_input<<<wblocks, 32 * WPB, 0, h->stream>>>(states, count_max, d.n, d.half_komi, s->x);
+    k_rnd_input<<<wblocks, 32 * WPB, 0, h->stream>>>(states, count_ptr, count_max, d.n, d.half_komi, s->x);
     const float one = 1.0f, zero = 0.0f;
     for (int a = 0; a < 2; a++) {
         // row-major Y[B][out] = X[B][in] W^T: column-major Y(out x B) = W(in x out)^T X(in x B)
@@ -225,8 +232,8 @@ int rnd_forward(tz_handle* h, const TzState* states, int count_max) {
         act(s->h2, s->b[a][1], RND_HIDDEN);
         if (gemm(s->w[a][2], s->h2, s->out[a], RND_OUT, RND_HIDDEN) != 0) return TZ_ECUDA;
     }
-    k_rnd_finish<<<wblocks, 32 * WPB, 0, h->stream>>>(s->out[0], s->out[1], s->b[0][2], s->b[1][2], count_max, s->lo, s->hi,
-                                                      s->unc);
+    k_rnd_finish<<<wblocks, 32 * WPB, 0, h->stream>>>(s->out[0], s->out[1], s->b[0][2], s->b[1][2], count_ptr, count_max, s->lo,
+                                                      s->hi, s->unc);
     h->launches += 12;
     return cudaGetLastError() == cudaSuccess ? TZ_OK : TZ_ECUDA;
 }

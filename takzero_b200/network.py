@@ -83,7 +83,9 @@ def set_weights(mcts: capi.BatchedMCTS, tensors: Dict[str, np.ndarray], dtype: i
 def broadcast_weights(mcts: capi.BatchedMCTS, tensors: Dict[str, np.ndarray] | None, root: int = 0,
                       res_blocks: int = 0, dtype: int = DTYPE_DEFAULT) -> None:
     """One weight generation on every rank of the handle's communicator (`tz_broadcast_weights`, collective): the
-    root passes the tensors, the others None; also valid without a communicator (= set_weights)."""
+    root passes the tensors, the others None; also valid without a communicator (= set_weights).  The RND estimator
+    of a 5x5 model (`rnd_learning.*`, `rnd_target.*`, `min`, `max`) is not broadcast: the root takes it as set_weights
+    does, and the other ranks keep the one they had."""
     _declare()
     capi._check(capi.lib().tz_set_network_dtype(mcts.handle, dtype))
     if tensors is None:
