@@ -132,6 +132,22 @@ pub struct tz_selfplay_data_t {
 }
 #[repr(C)]
 #[derive(Clone, Copy)]
+pub struct tz_training_batch_t {
+    pub batch: c_int,
+    pub indices: *const u64,
+    pub symmetry: *const c_int,
+    pub augment: c_int,
+    pub seed: u64,
+    pub planes: *mut f32,
+    pub policy: *mut f32,
+    pub mask: *mut u8,
+    pub value: *mut f32,
+    pub ube: *mut f32,
+    pub out_index: *mut c_int,
+    pub out_symmetry: *mut c_int,
+}
+#[repr(C)]
+#[derive(Clone, Copy)]
 pub struct tz_reanalyze_t {
     pub sampled_actions: c_int,
     pub search_budget: u32,
@@ -189,6 +205,10 @@ extern "C" {
     pub fn tz_launch_count(h: *mut tz_handle, out: *mut u64) -> c_int;
     pub fn tz_selfplay_record(h: *mut tz_handle, enable: c_int, bytes_per_game: usize, output_bytes: usize) -> c_int;
     pub fn tz_selfplay_read(h: *mut tz_handle, io: *mut tz_selfplay_data_t) -> c_int;
+    pub fn tz_target_buffer(h: *mut tz_handle, capacity: usize, from_selfplay: c_int) -> c_int;
+    pub fn tz_target_buffer_append(h: *mut tz_handle, count: usize, env: *const tz_state_t, value: *const f32, ube: *const f32, n: *const c_int, offset: *const u64, moves: *const tz_move_t, probs: *const f32, n_policy: usize) -> c_int;
+    pub fn tz_target_buffer_info(h: *mut tz_handle, size: *mut usize, appended: *mut u64) -> c_int;
+    pub fn tz_training_batch(h: *mut tz_handle, params: *const tz_training_batch_t) -> c_int;
     pub fn tz_stage_positions(h: *mut tz_handle, states: *const tz_state_t, count: usize) -> c_int;
     pub fn tz_reanalyze_batch(h: *mut tz_handle, pool_indices: *const u32, params: *const tz_reanalyze_t) -> c_int;
     pub fn tz_reanalyze_read(h: *mut tz_handle, stride: c_int, out_policy: *mut f32, out_ube: *mut f32, out_value: *mut f32, out_n: *mut c_int, out_moves: *mut tz_move_t) -> c_int;

@@ -276,6 +276,71 @@ typedef struct tz_selfplay_data_t {
  * error (TZ_STATUS_TARGETS_FULL is not one). */
 TZ_API int tz_selfplay_read(tz_handle* h, tz_selfplay_data_t* io);
 
+/* ---- training batches on the device (the data side of `learn`: replay buffer, Augment, game_to_tensor,
+ * policy_tensor / move_mask, target.rs:32-54, repr.rs:169-244) ------------------------------------------------------
+ *
+ * Target buffer: a FIFO ring of `capacity` targets in device memory.  Every slot has a fixed stride: the position
+ * (384 B), value, UBE target and entry count (12 B) and move_stride (move, probability) pairs (6 B each), so a slot
+ * takes 396 + 6 * move_stride bytes: about 6.5 KB for the 6x6 default stride of 1024, 6.5 GB for 10^6 targets.  A
+ * root never has more than move_stride children, so a slot cannot overflow.  TZ_ENOMEM when it does not fit; capacity
+ * 0 frees the buffer; calling again replaces it with an empty one.  When the ring is full the oldest targets are
+ * overwritten.
+ *   from_selfplay = 1: while recording is on (tz_selfplay_record), every target tz_selfplay_move emits into the output
+ *     queue is also appended, device to device and in queue order (finished games ascending, each from its last ply to
+ *     its first; the exploration filter applies; games dropped under TZ_STATUS_TARGETS_FULL are in neither).  The
+ *     queue, tz_selfplay_read and the search are unchanged.  With from_selfplay = 0 or no buffer, tz_selfplay_move
+ *     launches exactly what it launches without one. */
+TZ_API int tz_target_buffer(tz_handle* h, size_t capacity, int from_selfplay);
+/* Appends `count` targets from host arrays in the layout tz_selfplay_read returns: target i is env[i], value[i],
+ * ube[i] and the n[i] entries moves / probs[offset[i] .. offset[i] + n[i]) of arrays holding n_policy entries.
+ * TZ_EINVAL, appending nothing, when n[i] < 0 or n[i] > move_stride, an entry range falls outside n_policy, a move
+ * has no move_index on this board size (square off the board, placement of a piece code above 2, spread pattern that
+ * does not fit N), a target lists the same move twice (both would land on one policy index), or a position is not one
+ * of this board.  Waits for the handle's stream. */
+TZ_API int tz_target_buffer_append(tz_handle* h, size_t count, const tz_state_t* env, const float* value,
+                                   const float* ube, const int* n, const uint64_t* offset, const tz_move_t* moves,
+                                   const float* probs, size_t n_policy);
+/* Waits for the handle's stream; *size = targets kept (at most the capacity), *appended = targets ever appended since
+ * tz_target_buffer (for replay-ratio accounting).  Either pointer may be NULL. */
+TZ_API int tz_target_buffer_info(tz_handle* h, size_t* size, uint64_t* appended);
+
+/* One training batch: `batch` examples from the target buffer, written into CALLER-OWNED DEVICE MEMORY (every
+ * non-NULL output must be device memory of the handle's device).  C = 2 * (2N + 5) + 2 input channels and
+ * OC = 3 + 4 * (2^N - 2) output channels, as tz_info reports them.
+ * Example i takes target index[i] (counted from the oldest kept target) under symmetry sym[i]:
+ *   index[i] = indices ? indices[i] : high 64 bits of (rng_hash(seed, i, 0, 0) * size)
+ *   sym[i]   = symmetry ? symmetry[i] : augment ? rng_hash(seed, i, 1, 0) & 7 : 0
+ * with rng_hash(s, a, b, c) = mix(mix(mix(mix(s ^ 0x9e3779b97f4a7c15) ^ a * 0xbf58476d1ce4e5b9) ^ b *
+ * 0x94d049bb133111eb) ^ c * 0xd6e8feb86659fd93) and mix the murmur3 64-bit finalizer (x ^= x >> 33;
+ * x *= 0xff51afd7ed558ccd; x ^= x >> 33; x *= 0xc4ceb9fe1a85ec53; x ^= x >> 33), all modulo 2^64.
+ * A symmetry maps square (row, col) by, in this order: bit 0 mirrors the column, bit 1 mirrors the row, bit 2 swaps
+ * row and column (the order of tz_new_openings).  A spread keeps its pattern byte; its direction is mapped in the same
+ * order: bit 0 swaps '<' and '>', bit 1 swaps '+' and '-', bit 2 swaps '+' with '>' and '-' with '<'.  Reserves, side
+ * to move, ply and reversible plies are kept.
+ *   planes   f32 [batch][C][N][N]  game_repr of the transformed position (the encoding of tz_encode_planes)
+ *   policy   f32 [batch][OC][N][N] zero, and each entry's probability at move_index of the transformed move
+ *   mask     u8  [batch][OC][N][N] 1 at the same places, 0 elsewhere
+ *   value, ube    f32 [batch]       the target's, unchanged
+ *   out_index, out_symmetry i32 [batch]  what was used
+ * Waits for the handle's stream (queued self-play appends land first), then validates: TZ_EINVAL for an empty
+ * buffer, batch <= 0, an index at or past the size, a symmetry above 7 or an output that is not device memory of the
+ * handle's device.  Asynchronous: returns once the kernel is enqueued on the handle's stream; tz_sync waits. */
+typedef struct tz_training_batch_t {
+    int batch;
+    const uint64_t* indices;  /* host [batch] or NULL: drawn */
+    const int* symmetry;      /* host [batch] 0..7 or NULL: drawn when augment, else 0 */
+    int augment;
+    uint64_t seed;
+    float* planes;            /* device outputs; NULL skips */
+    float* policy;
+    uint8_t* mask;
+    float* value;
+    float* ube;
+    int* out_index;           /* i32 */
+    int* out_symmetry;
+} tz_training_batch_t;
+TZ_API int tz_training_batch(tz_handle* h, const tz_training_batch_t* params);
+
 /* The loop body of `reanalyze` (reanalyze/src/main.rs:147-235) without per-batch host buffers.  tz_stage_positions
  * uploads the positions of the replay buffer once (position_buffer, main.rs:60-75); tz_reanalyze_batch makes the
  * staged positions pool_indices[g] the fresh roots of the games (`*node = Node::default(); *env = replay_env`, NULL =

@@ -591,6 +591,41 @@ class BatchedMCTS {
         }
         return out;
     }
+    // ---- training batches on the device (the data side of `learn`) --------------------------------------------------
+    // a new, empty ring of `capacity` targets (0 frees it); from_selfplay: selfplay_move's emitted targets go in too
+    void target_buffer(size_t capacity, bool from_selfplay = false) {
+        check(tz_target_buffer(h_, capacity, from_selfplay ? 1 : 0));
+    }
+    // e.g. the targets of selfplay_read, or of a targets-*.txt file through Target::parse
+    void append_targets(const std::vector<Target>& targets) {
+        std::vector<tz_state_t> env;
+        std::vector<float> value, ube, probs;
+        std::vector<int> n;
+        std::vector<uint64_t> offset;
+        std::vector<Move> moves;
+        for (const Target& t : targets) {
+            env.push_back(t.env);
+            value.push_back(t.value);
+            ube.push_back(t.ube);
+            n.push_back((int)t.policy.size());
+            offset.push_back(moves.size());
+            for (const auto& e : t.policy) {
+                moves.push_back(e.first);
+                probs.push_back(e.second);
+            }
+        }
+        check(tz_target_buffer_append(h_, targets.size(), env.data(), value.data(), ube.data(), n.data(),
+                                      offset.data(), moves.data(), probs.data(), moves.size()));
+    }
+    // (targets kept, targets ever appended)
+    std::pair<size_t, uint64_t> target_buffer_info() {
+        size_t size = 0;
+        uint64_t appended = 0;
+        check(tz_target_buffer_info(h_, &size, &appended));
+        return {size, appended};
+    }
+    // one batch into caller-owned device memory (see tz_training_batch); asynchronous, sync() waits
+    void training_batch(const tz_training_batch_t& params) { check(tz_training_batch(h_, &params)); }
     void set_agent(int kind, tz_agent_fn fn = nullptr, void* ctx = nullptr) { check(tz_set_agent(h_, kind, fn, ctx)); }
     void new_openings(uint64_t seed) { check(tz_new_openings(h_, nullptr, nullptr, nullptr, seed)); }
     void set_positions(const std::vector<tz_state_t>& envs) { check(tz_set_positions(h_, envs.data(), nullptr)); }

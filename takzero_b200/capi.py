@@ -123,6 +123,14 @@ SELFPLAY_FIELDS = {
 STATUS_TARGETS_FULL = 1024
 
 
+class TrainingBatchParams(C.Structure):
+    """tz_training_batch_t: host index / symmetry arrays (or NULL) and device output pointers (or NULL)."""
+
+    _fields_ = [("batch", C.c_int), ("indices", C.c_void_p), ("symmetry", C.c_void_p), ("augment", C.c_int),
+                ("seed", C.c_uint64), ("planes", C.c_void_p), ("policy", C.c_void_p), ("mask", C.c_void_p),
+                ("value", C.c_void_p), ("ube", C.c_void_p), ("out_index", C.c_void_p), ("out_symmetry", C.c_void_p)]
+
+
 class Profile(C.Structure):
     _fields_ = [("ms", C.c_double * 8), ("launches", C.c_uint64 * 8), ("locksteps", C.c_uint64),
                 ("positions", C.c_uint64)]
@@ -202,6 +210,10 @@ def lib():
         "tz_launch_count": ([vp, P(u64)], i32),
         "tz_selfplay_record": ([vp, i32, C.c_size_t, C.c_size_t], i32),
         "tz_selfplay_read": ([vp, P(SelfplayData)], i32),
+        "tz_target_buffer": ([vp, C.c_size_t, i32], i32),
+        "tz_target_buffer_append": ([vp, C.c_size_t, vp, vp, vp, vp, vp, vp, vp, C.c_size_t], i32),
+        "tz_target_buffer_info": ([vp, P(C.c_size_t), P(u64)], i32),
+        "tz_training_batch": ([vp, P(TrainingBatchParams)], i32),
         "tz_stage_positions": ([vp, vp, C.c_size_t], i32),
         "tz_reanalyze_batch": ([vp, vp, P(ReanalyzeParams)], i32),
         "tz_reanalyze_read": ([vp, i32, vp, vp, vp, vp, vp], i32),
@@ -267,6 +279,7 @@ class BatchedMCTS:
         _check(lib().tz_create(C.byref(cfg), C.byref(self._h)))
         self.n = board_n
         self.half_komi = half_komi
+        self.device = device
         self.G = n_games
         self.game_base = game_base
         ms, slots, ic, oc = C.c_int(), C.c_uint32(), C.c_int(), C.c_int()
@@ -550,6 +563,70 @@ class BatchedMCTS:
         for k in ("n_targets", "n_policy", "n_replays", "n_moves", "high_water_bytes"):
             res[k] = int(getattr(io, k))
         return res
+
+    # ---- training batches on the device (the data side of `learn`) ------------------------------------------
+    def target_buffer(self, capacity: int, from_selfplay: bool = False) -> None:
+        """A new, empty ring of `capacity` targets (0 frees it); from_selfplay also appends every target that
+        selfplay_move emits while recording is on (see tz_target_buffer)."""
+        _check(lib().tz_target_buffer(self._h, int(capacity), 1 if from_selfplay else 0))
+
+    def append_targets(self, data: dict) -> None:
+        """Append targets in the layout selfplay_read returns (target_env, target_value, target_ube, target_n,
+        target_offset, policy_moves, policy_probs)."""
+        env = _arr(data["target_env"], STATE_DTYPE)
+        count = len(env)
+        value = _arr(data["target_value"], np.float32, (count,))
+        ube = _arr(data["target_ube"], np.float32, (count,))
+        n = _arr(data["target_n"], np.int32, (count,))
+        offset = _arr(data["target_offset"], np.uint64, (count,))
+        moves = _arr(data["policy_moves"], np.uint16)
+        probs = _arr(data["policy_probs"], np.float32, moves.shape)
+        _check(lib().tz_target_buffer_append(self._h, count, _ptr(env), _ptr(value), _ptr(ube), _ptr(n),
+                                             _ptr(offset), _ptr(moves), _ptr(probs), len(moves)))
+
+    def target_buffer_info(self) -> tuple:
+        """(targets kept, targets ever appended)."""
+        size, appended = C.c_size_t(), C.c_uint64()
+        _check(lib().tz_target_buffer_info(self._h, C.byref(size), C.byref(appended)))
+        return int(size.value), int(appended.value)
+
+    TRAINING_FIELDS = ("planes", "policy", "mask", "value", "ube", "index", "symmetry")
+
+    def training_shapes(self, batch: int) -> dict:
+        """name -> (shape, torch dtype name) of the training_batch outputs."""
+        n, C_, OC = self.n, self.input_channels, self.output_channels
+        return {"planes": ((batch, C_, n, n), "float32"), "policy": ((batch, OC, n, n), "float32"),
+                "mask": ((batch, OC, n, n), "uint8"), "value": ((batch,), "float32"), "ube": ((batch,), "float32"),
+                "index": ((batch,), "int32"), "symmetry": ((batch,), "int32")}
+
+    def training_batch(self, batch: int, seed: int, augment: bool = True, indices=None, symmetry=None, out=None):
+        """One training batch from the target buffer as torch CUDA tensors on the handle's device: planes, policy,
+        mask, value, ube and the index / symmetry each example used (see tz_training_batch).  `out` maps any of
+        those names to preallocated contiguous tensors; with `out` only those are written.  Waits for the result."""
+        import torch
+
+        shapes = self.training_shapes(batch)
+        dev = torch.device("cuda", self.device)
+        if out is None:
+            out = {k: torch.empty(shape, dtype=getattr(torch, dt), device=dev) for k, (shape, dt) in shapes.items()}
+        for k, t in out.items():
+            if k not in shapes:
+                raise ValueError(f"unknown output {k!r}")
+            shape, dt = shapes[k]
+            if not isinstance(t, torch.Tensor) or t.device != dev:
+                raise ValueError(f"{k} must be a torch tensor on {dev}")
+            if tuple(t.shape) != shape or t.dtype != getattr(torch, dt) or not t.is_contiguous():
+                raise ValueError(f"{k} must be a contiguous {dt} tensor of shape {shape}")
+        idx = None if indices is None else _arr(indices, np.uint64, (batch,))
+        sym = None if symmetry is None else _arr(symmetry, np.int32, (batch,))
+        ptr = lambda k: out[k].data_ptr() if k in out else None
+        p = TrainingBatchParams(batch, _ptr(idx), _ptr(sym), 1 if augment else 0, seed, ptr("planes"), ptr("policy"),
+                                ptr("mask"), ptr("value"), ptr("ube"), ptr("index"), ptr("symmetry"))
+        # the library's stream does not wait for torch's: outputs allocated on torch's stream must be ready
+        torch.cuda.current_stream(dev).synchronize()
+        _check(lib().tz_training_batch(self._h, C.byref(p)))
+        self.sync()
+        return out
 
     # ---- reanalyze (reanalyze/src/main.rs:147-235) ---------------------------------------------------------
     def stage_positions(self, states: np.ndarray) -> None:

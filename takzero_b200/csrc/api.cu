@@ -97,6 +97,7 @@ static int first_invalid_state(const tz_state_t* states, int count, int n, const
     } while (0)
 
 static void rec_free(tz_handle* h);
+static void ring_free(tz_handle* h);
 
 static int default_stride(int n) { return n <= 3 ? 128 : n == 4 ? 256 : n == 5 ? 512 : 1024; }
 
@@ -262,6 +263,7 @@ extern "C" TZ_API void tz_destroy(tz_handle* h) {
     nn_free(h);
     comm_destroy(h);
     rec_free(h);
+    ring_free(h);
     for (void* p : h->allocs) cudaFree(p);
     if (h->pool) cudaFree(h->pool);
     if (h->pin_small) cudaFreeHost(h->pin_small);
@@ -1078,10 +1080,21 @@ extern "C" TZ_API int tz_selfplay_move(tz_handle* h, const tz_selfplay_t* sp) {
                    h->fin_len, h->stream, recording ? h->rec.result : nullptr);
     h->launches += 6;
     if (recording) {
+        // the queue range this move emits, [fill before, fill after), also goes to the target buffer
+        const bool to_ring = h->ring.env != nullptr && h->ring_from_selfplay;
+        const unsigned long long* fill = h->rec.fill + TZ_Q_TARGETS;
+        if (to_ring) CU(cudaMemcpyAsync(h->ring.range, fill, sizeof(*fill), cudaMemcpyDeviceToDevice, h->stream));
         // restart_envs_and_complete_targets (main.rs:263-329): the exploration half is the first G/2 games
         launch_emit(d, h->rec, h->terminal, h->fin_len, h->fin_start, h->fin_replay, sp->weighted_random_plies,
                     sp->beta != 0.0f ? d.G / 2 : 0, h->stream);
         h->launches += 4;
+        if (to_ring) {
+            CU(cudaMemcpyAsync(h->ring.range + 1, fill, sizeof(*fill), cudaMemcpyDeviceToDevice, h->stream));
+            const TzRecorder& r = h->rec;
+            launch_target_append(h->ring, r.t_env, r.t_value, r.t_ube, r.t_n, r.t_off, r.p_moves, r.p_probs, 0,
+                                 h->stream);
+            h->launches += 1;
+        }
     }
     CU(cudaGetLastError());
     return TZ_OK;
@@ -1245,6 +1258,225 @@ extern "C" TZ_API int tz_selfplay_read(tz_handle* h, tz_selfplay_data_t* io) {
 }
 
 // ---- reanalyze (reanalyze/src/main.rs:147-235) without per-batch host buffers ----------------------------------------
+
+// ---- target buffer and training batches ----------------------------------------------------------------------
+
+static void ring_free(tz_handle* h) {
+    for (void* p : h->ring_allocs) cudaFree(p);
+    h->ring_allocs.clear();
+    memset(&h->ring, 0, sizeof(h->ring));
+    h->ring_from_selfplay = false;
+    if (h->batch_idx) cudaFree(h->batch_idx);
+    if (h->batch_sym) cudaFree(h->batch_sym);
+    h->batch_idx = nullptr;
+    h->batch_sym = nullptr;
+    h->batch_cap = 0;
+}
+
+// move_index (repr.rs:49-71) exists for m on an n x n board: the square is on the board, a placement names a flat,
+// wall or cap, a spread's pattern byte is MSB-aligned to N bits and is one of the 2^N - 2 patterns of a direction
+static bool move_has_index(int n, uint16_t m) {
+    const int col = m & 7, row = (m >> 3) & 7, kd = (m >> 6) & 3, pat = m >> 8;
+    if (row >= n || col >= n) return false;
+    if (pat == 0) return kd <= 2;
+    if (pat & ((1 << (8 - n)) - 1)) return false;
+    const int p = pat >> (8 - n);
+    return p >= 1 && p <= (1 << n) - 2;
+}
+
+extern "C" TZ_API int tz_target_buffer(tz_handle* h, size_t capacity, int from_selfplay) {
+    CHECK_H(h);
+    CU(cudaStreamSynchronize(h->stream));
+    ring_free(h);
+    if (capacity == 0) return TZ_OK;
+    const size_t M = (size_t)h->d.M;
+    const size_t slot_bytes = sizeof(TzState) + 3 * 4 + 6 * M;
+    if (capacity > SIZE_MAX / slot_bytes)
+        return fail(TZ_ENOMEM, "a target buffer of %zu targets (%zu B each) does not fit", capacity, slot_bytes);
+    TzTargetRing& R = h->ring;
+    cudaError_t e = cudaSuccess;
+#define RA(ptr, count)                                                          \
+    if (e == cudaSuccess) {                                                     \
+        void* v_ = nullptr;                                                     \
+        e = cudaMalloc(&v_, (size_t)(count) * sizeof(*(ptr)));                  \
+        if (e == cudaSuccess) {                                                 \
+            h->ring_allocs.push_back(v_);                                       \
+            (ptr) = (decltype(ptr))v_;                                          \
+        }                                                                       \
+    }
+    RA(R.env, capacity);
+    RA(R.value, capacity);
+    RA(R.ube, capacity);
+    RA(R.n, capacity);
+    RA(R.moves, capacity * M);
+    RA(R.probs, capacity * M);
+    RA(R.appended, 1);
+    RA(R.range, 2);
+    RA(R.ticket, 1);
+#undef RA
+    if (e != cudaSuccess) {
+        cudaGetLastError();
+        ring_free(h);
+        return fail(TZ_ENOMEM, "cudaMalloc of a target buffer of %zu targets (%zu B): %s", capacity,
+                    capacity * slot_bytes, cudaGetErrorString(e));
+    }
+    R.cap = capacity;
+    R.stride = (int)M;
+    h->ring_from_selfplay = from_selfplay != 0;
+    if (cudaMemsetAsync(R.appended, 0, sizeof(*R.appended), h->stream) != cudaSuccess ||
+        cudaMemsetAsync(R.ticket, 0, sizeof(*R.ticket), h->stream) != cudaSuccess ||
+        cudaStreamSynchronize(h->stream) != cudaSuccess) {
+        const cudaError_t le = cudaGetLastError();
+        ring_free(h);
+        return fail(TZ_ECUDA, "tz_target_buffer: %s", cudaGetErrorString(le));
+    }
+    return TZ_OK;
+}
+
+// waits for the stream and reads the ring's counter
+static int ring_appended(tz_handle* h, unsigned long long* out) {
+    CU(cudaMemcpyAsync(out, h->ring.appended, sizeof(*out), cudaMemcpyDeviceToHost, h->stream));
+    CU(cudaStreamSynchronize(h->stream));
+    CU(cudaGetLastError());
+    return TZ_OK;
+}
+
+extern "C" TZ_API int tz_target_buffer_info(tz_handle* h, size_t* size, uint64_t* appended) {
+    CHECK_H(h);
+    if (!h->ring.env) return fail(TZ_EINVAL, "no target buffer: tz_target_buffer first");
+    unsigned long long a = 0;
+    const int rc = ring_appended(h, &a);
+    if (rc) return rc;
+    if (size) *size = (size_t)std::min<unsigned long long>(a, h->ring.cap);
+    if (appended) *appended = a;
+    return TZ_OK;
+}
+
+extern "C" TZ_API int tz_target_buffer_append(tz_handle* h, size_t count, const tz_state_t* env, const float* value,
+                                              const float* ube, const int* n, const uint64_t* offset,
+                                              const tz_move_t* moves, const float* probs, size_t n_policy) {
+    CHECK_H(h);
+    TzTargetRing& R = h->ring;
+    if (!R.env) return fail(TZ_EINVAL, "no target buffer: tz_target_buffer first");
+    if (count == 0) return TZ_OK;
+    if (!env || !value || !ube || !n || !offset) return fail(TZ_EINVAL, "null target array");
+    if (n_policy > 0 && (!moves || !probs)) return fail(TZ_EINVAL, "null policy array");
+    if (count > (size_t)INT32_MAX) return fail(TZ_EINVAL, "count %zu is too large for one call", count);
+    const int M = h->d.M, N = h->d.n;
+    std::vector<uint8_t> seen(1 << 16, 0);
+    for (size_t i = 0; i < count; i++) {
+        if (n[i] < 0 || n[i] > M) return fail(TZ_EINVAL, "target %zu: n = %d is outside 0..%d (move_stride)", i, n[i], M);
+        if (offset[i] > n_policy || (uint64_t)n[i] > n_policy - offset[i])
+            return fail(TZ_EINVAL, "target %zu: entries %llu..%llu are outside the %zu policy entries", i,
+                        (unsigned long long)offset[i], (unsigned long long)offset[i] + (unsigned long long)n[i],
+                        n_policy);
+        const tz_move_t* mv = moves + offset[i];
+        for (int j = 0; j < n[i]; j++)
+            if (!move_has_index(N, mv[j]))
+                return fail(TZ_EINVAL, "target %zu: move 0x%04x has no move_index on a %dx%d board", i,
+                            (unsigned)mv[j], N, N);
+        bool dup = false;  // two entries of one move would scatter to one policy index
+        for (int j = 0; j < n[i]; j++) {
+            dup = dup || seen[mv[j]];
+            seen[mv[j]] = 1;
+        }
+        for (int j = 0; j < n[i]; j++) seen[mv[j]] = 0;
+        if (dup) return fail(TZ_EINVAL, "target %zu lists a move twice", i);
+    }
+    CHECK_STATES(env, (int)count, nullptr);
+    Scratch s;
+    TzState* d_env;
+    float *d_value, *d_ube, *d_probs;
+    int* d_n;
+    unsigned long long* d_off;
+    uint16_t* d_moves;
+    CU(s.get(&d_env, count));
+    CU(s.get(&d_value, count));
+    CU(s.get(&d_ube, count));
+    CU(s.get(&d_n, count));
+    CU(s.get(&d_off, count));
+    CU(s.get(&d_moves, n_policy));
+    CU(s.get(&d_probs, n_policy));
+    const unsigned long long range[2] = {0ull, (unsigned long long)count};
+    CU(cudaMemcpyAsync(d_env, env, count * sizeof(TzState), cudaMemcpyHostToDevice, h->stream));
+    CU(cudaMemcpyAsync(d_value, value, count * sizeof(float), cudaMemcpyHostToDevice, h->stream));
+    CU(cudaMemcpyAsync(d_ube, ube, count * sizeof(float), cudaMemcpyHostToDevice, h->stream));
+    CU(cudaMemcpyAsync(d_n, n, count * sizeof(int), cudaMemcpyHostToDevice, h->stream));
+    CU(cudaMemcpyAsync(d_off, offset, count * sizeof(uint64_t), cudaMemcpyHostToDevice, h->stream));
+    if (n_policy > 0) {
+        CU(cudaMemcpyAsync(d_moves, moves, n_policy * sizeof(uint16_t), cudaMemcpyHostToDevice, h->stream));
+        CU(cudaMemcpyAsync(d_probs, probs, n_policy * sizeof(float), cudaMemcpyHostToDevice, h->stream));
+    }
+    CU(cudaMemcpyAsync(R.range, range, sizeof(range), cudaMemcpyHostToDevice, h->stream));
+    launch_target_append(R, d_env, d_value, d_ube, d_n, d_off, d_moves, d_probs, count, h->stream);
+    h->launches += 1;
+    CU(cudaStreamSynchronize(h->stream));
+    CU(cudaGetLastError());
+    return TZ_OK;
+}
+
+// an output of tz_training_batch: NULL, or 4-byte aligned (`align`) device memory of the handle's device
+static int check_device_output(tz_handle* h, const void* p, size_t align, const char* name) {
+    if (!p) return TZ_OK;
+    if ((uintptr_t)p % align) return fail(TZ_EINVAL, "%s is not %zu-byte aligned", name, align);
+    cudaPointerAttributes a;
+    if (cudaPointerGetAttributes(&a, p) != cudaSuccess) {
+        cudaGetLastError();
+        return fail(TZ_EINVAL, "%s is not device memory", name);
+    }
+    if (a.type != cudaMemoryTypeDevice || a.device != h->device)
+        return fail(TZ_EINVAL, "%s is not device memory of device %d", name, h->device);
+    return TZ_OK;
+}
+
+extern "C" TZ_API int tz_training_batch(tz_handle* h, const tz_training_batch_t* p) {
+    CHECK_H(h);
+    if (!p) return fail(TZ_EINVAL, "null parameters");
+    TzTargetRing& R = h->ring;
+    if (!R.env) return fail(TZ_EINVAL, "no target buffer: tz_target_buffer first");
+    if (p->batch <= 0) return fail(TZ_EINVAL, "batch must be > 0");
+    int rc;
+    if ((rc = check_device_output(h, p->planes, 4, "planes")) || (rc = check_device_output(h, p->policy, 4, "policy")) ||
+        (rc = check_device_output(h, p->mask, 1, "mask")) || (rc = check_device_output(h, p->value, 4, "value")) ||
+        (rc = check_device_output(h, p->ube, 4, "ube")) || (rc = check_device_output(h, p->out_index, 4, "out_index")) ||
+        (rc = check_device_output(h, p->out_symmetry, 4, "out_symmetry")))
+        return rc;
+    unsigned long long appended = 0;
+    if ((rc = ring_appended(h, &appended))) return rc;
+    const unsigned long long size = std::min<unsigned long long>(appended, R.cap);
+    if (size == 0) return fail(TZ_EINVAL, "the target buffer is empty");
+    const size_t B = (size_t)p->batch;
+    if (p->indices)
+        for (size_t i = 0; i < B; i++)
+            if (p->indices[i] >= size)
+                return fail(TZ_EINVAL, "indices[%zu] = %llu is not below the size %llu", i,
+                            (unsigned long long)p->indices[i], size);
+    if (p->symmetry)
+        for (size_t i = 0; i < B; i++)
+            if (p->symmetry[i] < 0 || p->symmetry[i] > 7)
+                return fail(TZ_EINVAL, "symmetry[%zu] = %d is not 0..7", i, p->symmetry[i]);
+    if ((p->indices || p->symmetry) && B > h->batch_cap) {  // the stream is idle (ring_appended waited)
+        if (h->batch_idx) cudaFree(h->batch_idx);
+        if (h->batch_sym) cudaFree(h->batch_sym);
+        h->batch_idx = nullptr;
+        h->batch_sym = nullptr;
+        h->batch_cap = 0;
+        CU(cudaMalloc(&h->batch_idx, B * sizeof(unsigned long long)));
+        CU(cudaMalloc(&h->batch_sym, B * sizeof(int)));
+        h->batch_cap = B;
+    }
+    if (p->indices)
+        CU(cudaMemcpyAsync(h->batch_idx, p->indices, B * sizeof(uint64_t), cudaMemcpyHostToDevice, h->stream));
+    if (p->symmetry)
+        CU(cudaMemcpyAsync(h->batch_sym, p->symmetry, B * sizeof(int), cudaMemcpyHostToDevice, h->stream));
+    const TzBatchOut o = {p->planes, p->policy, p->mask, p->value, p->ube, p->out_index, p->out_symmetry};
+    const unsigned long long first = (appended - size) % R.cap;
+    launch_training_batch(R, h->d.n, h->d.half_komi, p->batch, p->indices ? h->batch_idx : nullptr,
+                          p->symmetry ? h->batch_sym : nullptr, p->augment, p->seed, size, first, o, h->stream);
+    h->launches += 1;
+    CU(cudaGetLastError());
+    return TZ_OK;
+}
 
 extern "C" TZ_API int tz_stage_positions(tz_handle* h, const tz_state_t* states, size_t count) {
     CHECK_H(h);

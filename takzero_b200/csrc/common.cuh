@@ -173,3 +173,19 @@ struct TzRecorder {
     unsigned long long* g_count;  // [G][TZ_Q_KINDS] what each finished game emits
     unsigned long long* g_base;   // [G][TZ_Q_KINDS] where it goes; g_base[g][0] = ~0 when it does not fit
 };
+
+// Target buffer (tz_target_buffer): a ring of `cap` slots with a fixed stride.  Target number k ever appended lives in
+// slot k % cap; the ones kept are the last min(appended, cap).
+struct TzTargetRing {
+    TzState* env;      // [cap]
+    float* value;      // [cap]
+    float* ube;        // [cap]
+    int* n;            // [cap] entries
+    uint16_t* moves;   // [cap][stride]
+    float* probs;      // [cap][stride]
+    unsigned long long cap;
+    int stride;
+    unsigned long long* appended;  // [1] targets ever appended
+    unsigned long long* range;     // [2] source entries [lo, hi) of the append in flight
+    unsigned int* ticket;          // [1] blocks of k_target_append done (the last one advances `appended`)
+};

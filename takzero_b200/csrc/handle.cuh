@@ -64,6 +64,13 @@ struct tz_handle {
     TzRecorder rec{};
     std::vector<void*> rec_allocs;
     bool rec_stale = false;  // positions were moved or replaced since the last recording move: drop pending records
+    // target buffer of training batches (tz_target_buffer); ring.env == nullptr: none
+    TzTargetRing ring{};
+    std::vector<void*> ring_allocs;
+    bool ring_from_selfplay = false;
+    unsigned long long* batch_idx = nullptr;  // device staging of tz_training_batch's host indices / symmetries
+    int* batch_sym = nullptr;
+    size_t batch_cap = 0;
     // bookkeeping
     unsigned long long move_counter = 0;
     unsigned long long opening_counter = 0;

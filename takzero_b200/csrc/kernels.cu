@@ -14,6 +14,7 @@
 //   k_select_actions node/mod.rs:132-207
 #include "encode.cuh"
 #include "kernels.cuh"
+#include "planes.cuh"
 #include "rules.cuh"
 #include "tree.cuh"
 
@@ -1800,6 +1801,152 @@ __global__ void __launch_bounds__(32 * WPB) k_emit_write(TzDev d, TzRecorder r, 
     }
 }
 
+// ---- training batches from the target buffer (the data side of `learn`) ------------------------------------
+
+// Append source entries [range[0], range[1]) -- targets in the layout of tz_selfplay_read: env / value / ube / n per
+// target, its entries moves / probs [off, off + n) -- to the ring: entry lo + k goes to slot (appended + k) % cap.  When
+// more than cap arrive at once only the last cap are written.  The last block to finish advances `appended`.
+__global__ void __launch_bounds__(32 * WPB) k_target_append(TzTargetRing R, const TzState* env, const float* value,
+                                                            const float* ube, const int* n,
+                                                            const unsigned long long* off, const uint16_t* moves,
+                                                            const float* probs) {
+    const int lane = threadIdx.x & 31;
+    const unsigned long long lo = R.range[0], hi = R.range[1], base = *R.appended;
+    const unsigned long long count = hi - lo, skip = count > R.cap ? count - R.cap : 0ull;
+    const unsigned long long nw = (unsigned long long)gridDim.x * WPB;
+    for (unsigned long long k = skip + blockIdx.x * WPB + (threadIdx.x >> 5); k < count; k += nw) {
+        const unsigned long long q = lo + k, slot = (base + k) % R.cap;
+        if (lane < 24)
+            reinterpret_cast<uint4*>(&R.env[slot])[lane] = reinterpret_cast<const uint4*>(&env[q])[lane];
+        const int cnt = n[q];
+        const unsigned long long po = off[q];
+        if (lane == 0) {
+            R.value[slot] = value[q];
+            R.ube[slot] = ube[q];
+            R.n[slot] = cnt;
+        }
+        uint16_t* dm = R.moves + (size_t)slot * R.stride;
+        float* dp = R.probs + (size_t)slot * R.stride;
+        for (int i = lane; i < cnt; i += 32) {
+            dm[i] = moves[po + i];
+            dp[i] = probs[po + i];
+        }
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        __threadfence();
+        if (atomicAdd(R.ticket, 1u) == gridDim.x - 1) {
+            *R.appended = base + count;
+            *R.ticket = 0;
+        }
+    }
+}
+
+// symmetry t of the board (tz_training_batch): bit 0 mirrors the column, bit 1 the row, bit 2 swaps them, in this order
+__device__ __forceinline__ void sym_square(int t, int n, int* row, int* col) {
+    if (t & 1) *col = n - 1 - *col;
+    if (t & 2) *row = n - 1 - *row;
+    if (t & 4) {
+        const int tmp = *col;
+        *col = *row;
+        *row = tmp;
+    }
+}
+
+// the same on a move: the square as above, a spread's direction (0 '+', 1 '-', 2 '<', 3 '>') alike, the pattern kept
+__device__ __forceinline__ uint16_t sym_move(int t, int n, uint16_t m) {
+    int col = m & 7, row = (m >> 3) & 7, kd = (m >> 6) & 3;
+    const int pat = m >> 8;
+    sym_square(t, n, &row, &col);
+    if (pat) {
+        if ((t & 1) && kd >= 2) kd ^= 1;  // '<' <-> '>'
+        if ((t & 2) && kd < 2) kd ^= 1;   // '+' <-> '-'
+        if (t & 4) kd = 3 - kd;           // '+' <-> '>', '-' <-> '<'
+    }
+    return (uint16_t)(col | (row << 3) | (kd << 6) | (pat << 8));
+}
+
+// k_training_batch: blocks of 8 warps; each example is written by a team of `team` warps (1, 2, 4 or 8).  A 6x6
+// example writes about 50 KB of policy and mask, so a small batch needs several warps per example to keep enough
+// stores in flight, while a large one is fastest with a warp per example (no team waits for its leader's planes).
+#define TB_THREADS 256
+
+// `nthreads` threads zero `bytes` bytes at p: byte stores up to the first 16-byte boundary, 16-byte stores, byte
+// stores for the tail (rows of 5x5 and 6x6 masks, and of 5x5 policies, do not start 16-byte aligned)
+__device__ __forceinline__ void team_zero_bytes(uint8_t* p, size_t bytes, int tid, int nthreads) {
+    size_t head = (16 - ((uintptr_t)p & 15)) & 15;
+    if (head > bytes) head = bytes;
+    if ((size_t)tid < head) p[tid] = 0;
+    const size_t nvec = (bytes - head) >> 4;
+    uint4* q = reinterpret_cast<uint4*>(p + head);
+    for (size_t i = tid; i < nvec; i += nthreads) q[i] = make_uint4(0u, 0u, 0u, 0u);
+    const size_t done = head + (nvec << 4);
+    if ((size_t)tid < bytes - done) p[done + tid] = 0;
+}
+
+// Example b = target `first + index` of the ring under symmetry t -> the planes of the transformed position (the
+// team's first warp), the dense policy / mask rows of the transformed moves (zeroed by the team, then scattered after
+// a barrier), value and UBE.
+__global__ void __launch_bounds__(TB_THREADS) k_training_batch(TzTargetRing R, int n, int half_komi, int batch,
+                                                               const unsigned long long* indices, const int* symmetry,
+                                                               int augment, unsigned long long seed,
+                                                               unsigned long long size, unsigned long long first,
+                                                               int team, TzBatchOut o) {
+    __shared__ TzState s_src[TB_THREADS / 32], s_dst[TB_THREADS / 32];
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int e = warp / team, team_threads = team * 32, ttid = threadIdx.x - e * team_threads;
+    const int b = blockIdx.x * (TB_THREADS / 32 / team) + e;
+    const bool valid = b < batch;
+    const unsigned long long idx =
+        !valid ? 0ull : indices ? indices[b] : __umul64hi(rng_hash(seed, (uint64_t)b, 0, 0), size);
+    const int t = !valid ? 0 : symmetry ? symmetry[b] : augment ? (int)(rng_hash(seed, (uint64_t)b, 1, 0) & 7) : 0;
+    const unsigned long long slot = (first + idx) % R.cap;
+    const int nn = n * n;
+    const size_t row_len = (size_t)(3 + 4 * ((1 << n) - 2)) * nn;
+    float* prow = valid && o.policy ? o.policy + (size_t)b * row_len : nullptr;
+    uint8_t* mrow = valid && o.mask ? o.mask + (size_t)b * row_len : nullptr;
+    if (valid && ttid < 32) {
+        TzState* src = &s_src[e];
+        TzState* dst = &s_dst[e];
+        warp_load_state(src, &R.env[slot], lane);
+        warp_load_state(dst, src, lane);
+        for (int sq = lane; sq < nn; sq += 32) {
+            int row = sq / n, col = sq - row * n;
+            sym_square(t, n, &row, &col);
+            const int to = row * n + col;
+            dst->stack[to] = src->stack[sq];
+            dst->height[to] = src->height[sq];
+            dst->top[to] = src->top[sq];
+        }
+        __syncwarp();
+        if (o.planes) warp_encode_planes(dst, n, half_komi, o.planes + (size_t)b * (2 * (2 * n + 5) + 2) * nn, lane);
+        if (lane == 0) {
+            if (o.value) o.value[b] = R.value[slot];
+            if (o.ube) o.ube[b] = R.ube[slot];
+            if (o.out_index) o.out_index[b] = (int)idx;
+            if (o.out_symmetry) o.out_symmetry[b] = t;
+        }
+    }
+    if (prow) team_zero_bytes(reinterpret_cast<uint8_t*>(prow), row_len * sizeof(float), ttid, team_threads);
+    if (mrow) team_zero_bytes(mrow, row_len, ttid, team_threads);
+    // the zeroes land before the scatter overwrites them (team is uniform over the block)
+    if (team == 1)
+        __syncwarp();
+    else
+        __syncthreads();
+    if (prow || mrow) {
+        const int cnt = R.n[slot];
+        const uint16_t* mv = R.moves + (size_t)slot * R.stride;
+        const float* pr = R.probs + (size_t)slot * R.stride;
+        for (int i = ttid; i < cnt; i += team_threads) {
+            const uint16_t m = sym_move(t, n, mv[i]);
+            const int at = enc::move_channel(n, m) * nn + ((m >> 3) & 7) * n + (m & 7);
+            if (prow) prow[at] = pr[i];
+            if (mrow) mrow[at] = 1;
+        }
+    }
+}
+
 // ---- launchers -------------------------------------------------------------------------------
 
 static inline int blocks_for(int items) { return (items + WPB - 1) / WPB; }
@@ -1917,4 +2064,27 @@ void launch_rules_probe(const TzDev& d, const TzState* states, int count, int st
 void launch_apply_moves(const TzDev& d, TzState* states, const uint16_t* moves, int count, int* out_ok,
                         cudaStream_t st) {
     k_apply_moves<<<blocks_for(count), 32 * WPB, 0, st>>>(d, states, moves, count, out_ok);
+}
+
+// blocks of the ring appends: the self-play append does not know its count on the host, so it covers any count with
+// a grid-stride loop over this many warps
+static const int TZ_APPEND_BLOCKS = 592;
+
+void launch_target_append(const TzTargetRing& R, const TzState* env, const float* value, const float* ube, const int* n,
+                          const unsigned long long* off, const uint16_t* moves, const float* probs, size_t count_hint,
+                          cudaStream_t st) {
+    int blocks = TZ_APPEND_BLOCKS;
+    if (count_hint > 0 && count_hint < (size_t)TZ_APPEND_BLOCKS * WPB) blocks = blocks_for((int)count_hint);
+    k_target_append<<<blocks, 32 * WPB, 0, st>>>(R, env, value, ube, n, off, moves, probs);
+}
+void launch_training_batch(const TzTargetRing& R, int n, int half_komi, int batch, const unsigned long long* indices,
+                           const int* symmetry, int augment, unsigned long long seed, unsigned long long size,
+                           unsigned long long first, const TzBatchOut& o, cudaStream_t st) {
+    // warps per example: 8 up to 512 examples, halving as the batch doubles, 1 from 4096 on
+    int team = 8;
+    while (team > 1 && (long long)batch * team > 4096) team >>= 1;
+    const int per_block = TB_THREADS / 32 / team;
+    k_training_batch<<<(batch + per_block - 1) / per_block, TB_THREADS, 0, st>>>(R, n, half_komi, batch, indices,
+                                                                                 symmetry, augment, seed, size, first,
+                                                                                 team, o);
 }

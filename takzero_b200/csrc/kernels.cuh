@@ -31,6 +31,23 @@ void launch_record(const TzDev& d, const TzRecorder& r, const float* policy, con
                    cudaStream_t st);
 void launch_emit(const TzDev& d, const TzRecorder& r, const int* terminal, const int* fin_len, const TzState* fin_start,
                  const uint16_t* fin_replay, int weighted_random_plies, int exploration_games, cudaStream_t st);
+// target buffer: append source entries [R.range[0], R.range[1]) (count_hint: that count when the host knows it, else
+// 0), and one training batch (tz_training_batch)
+void launch_target_append(const TzTargetRing& R, const TzState* env, const float* value, const float* ube, const int* n,
+                          const unsigned long long* off, const uint16_t* moves, const float* probs, size_t count_hint,
+                          cudaStream_t st);
+struct TzBatchOut {
+    float* planes;
+    float* policy;
+    uint8_t* mask;
+    float* value;
+    float* ube;
+    int* out_index;
+    int* out_symmetry;
+};
+void launch_training_batch(const TzTargetRing& R, int n, int half_komi, int batch, const unsigned long long* indices,
+                           const int* symmetry, int augment, unsigned long long seed, unsigned long long size,
+                           unsigned long long first, const TzBatchOut& o, cudaStream_t st);
 void launch_root_table(const TzDev& d, int stride, int* out_n, uint16_t* moves, uint32_t* visits, uint32_t* eval_tag,
                        uint32_t* eval_bits, float* logit, float* prob, float* std_dev, cudaStream_t st);
 void launch_root_stats(const TzDev& d, uint32_t* out, cudaStream_t st);

@@ -137,42 +137,8 @@ __global__ void __launch_bounds__(32 * WPB) k_encode(const TzState* states, int 
     if (q >= count) return;
     TzState* st = &s_state[warp];
     warp_load_state(st, &states[q], lane);
-    const int nn = n * n, ss = 2 * n + 3, C = 2 * (ss + 2) + 2;
-    const int me = st->to_move, other = me ^ 1;
-    const TzBoards b = warp_boards(st, nn, lane);
-    const int s0 = n == 3 ? 10 : n == 4 ? 15 : n == 5 ? 21 : 30;
-    const int c0 = n >= 5 ? 1 : 0;
-    const float my_stones = __fdiv_rn((float)st->stones[me], (float)s0);
-    const float my_caps = c0 ? __fdiv_rn((float)st->caps[me], (float)c0) : 0.0f;
-    const float op_stones = __fdiv_rn((float)st->stones[other], (float)s0);
-    const float op_caps = c0 ? __fdiv_rn((float)st->caps[other], (float)c0) : 0.0f;
-    const float fcd = __fsub_rn((float)(__popcll(b.flat[0]) - __popcll(b.flat[1])), __fdiv_rn((float)half_komi, 2.0f));
-    const float fcd_sq = __fdiv_rn(fcd, (float)nn);
-    const float side = me == 1 ? 1.0f : 0.0f;
-    for (int sq = lane; sq < nn; sq += 32) {
-        float v[CIN_PAD];
-#pragma unroll
-        for (int c = 0; c < CIN_PAD; c++) v[c] = 0.0f;
-        const int h = st->height[sq];
-        if (h > 0) {
-            const uint64_t stack = st->stack[sq];
-            const int top_col = (int)((stack >> (h - 1)) & 1ull);
-            v[st->top[sq] + (top_col != me ? ss : 0)] = 1.0f;
-            for (int i = 0; i < ss - 3 && h - 2 - i >= 0; i++) {
-                const int col = (int)((stack >> (h - 2 - i)) & 1ull);
-                v[3 + i + (col != me ? ss : 0)] = 1.0f;
-            }
-        }
-        const int base = 2 * ss;
-        v[base] = my_stones;
-        v[base + 1] = my_caps;
-        v[base + 2] = op_stones;
-        v[base + 3] = op_caps;
-        v[base + 4] = side;
-        v[base + 5] = fcd_sq;
-        float* o = out_f32 + (size_t)q * C * nn + sq;
-        for (int c = 0; c < C; c++) o[(size_t)c * nn] = v[c];
-    }
+    const int C = 2 * (2 * n + 5) + 2;
+    warp_encode_planes(st, n, half_komi, out_f32 + (size_t)q * C * n * n, lane);
 }
 
 // parity hook for the 16-bit planes the first convolution's A producer builds (same device function): one thread

@@ -2,12 +2,14 @@
 k = 16, 256 simulations, fp16, bench's weights).  One command alternates, `--rounds` times:
   (a) tz_selfplay_move without recording;
   (b) tz_selfplay_move with recording and a tz_selfplay_read after every move;
+  (d) as (b) with a target buffer of --buffer targets fed by self-play (tz_target_buffer from_selfplay = 1);
   (c) the `selfplay` binary without and with --resident, in moves per second of wall clock (process start, model load
       and the first move included, so compare the two with each other, not with (a) / (b)).
-Prints one JSON object: simulations/s of (a) and (b), read time and bytes per move, the per-game high-water mark of
+Prints one JSON object: simulations/s of (a), (b) and (d), read time and bytes per move, the per-game high-water mark of
 the record regions, the binary's rates, and the card's name and power limit read in the same run.
 
-    python tools/selfplay_rate.py [--moves 6] [--rounds 3] [--games 8192] [--binary-moves 6] [--out FILE]"""
+    python tools/selfplay_rate.py [--moves 6] [--rounds 3] [--games 8192] [--binary-moves 6] [--buffer 1000000]
+                                  [--out FILE]"""
 import argparse
 import json
 import os
@@ -78,6 +80,7 @@ def main():
     ap.add_argument("--games", type=int, default=WORKLOADS["6x6_selfplay"]["games"])
     ap.add_argument("--binary-moves", type=int, default=6)
     ap.add_argument("--warmup", type=int, default=2)
+    ap.add_argument("--buffer", type=int, default=1_000_000)
     ap.add_argument("--out", default=None)
     args = ap.parse_args()
 
@@ -106,6 +109,12 @@ def main():
             m.selfplay_record(True)
             r["b_record_read"] = timed_moves(m, sp, args.moves, True)
             m.selfplay_record(False)
+            m.target_buffer(args.buffer, from_selfplay=True)
+            m.selfplay_record(True)
+            r["d_record_read_buffer"] = timed_moves(m, sp, args.moves, True)
+            r["d_record_read_buffer"]["buffer_appended"] = m.target_buffer_info()[1]
+            m.selfplay_record(False)
+            m.target_buffer(0)
             r["c_binary_host"] = binary_rate(exe, wpath, args, False)
             r["c_binary_resident"] = binary_rate(exe, wpath, args, True)
             res["rounds"].append(r)
@@ -114,8 +123,9 @@ def main():
     rounds = res["rounds"]
     a = sum(r["a_off"]["sims_per_s"] for r in rounds) / len(rounds)
     b = sum(r["b_record_read"]["sims_per_s"] for r in rounds) / len(rounds)
+    dd = sum(r["d_record_read_buffer"]["sims_per_s"] for r in rounds) / len(rounds)
     res["summary"] = {
-        "a_sims_per_s": a, "b_sims_per_s": b, "b_over_a": b / a,
+        "a_sims_per_s": a, "b_sims_per_s": b, "b_over_a": b / a, "d_sims_per_s": dd, "d_over_b": dd / b,
         "read_ms_per_move": sum(r["b_record_read"]["read_ms_per_move"] for r in rounds) / len(rounds),
         "read_bytes_per_move": sum(r["b_record_read"]["read_bytes_per_move"] for r in rounds) / len(rounds),
         "high_water_bytes_per_game": max(r["b_record_read"]["high_water_bytes"] for r in rounds),
