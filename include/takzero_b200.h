@@ -86,7 +86,7 @@ typedef struct tz_config_t {
     int half_komi;         /* e.g. 4 for Game<6,4> */
     int n_games;           /* BATCH_SIZE of BatchedMCTS, dynamic here */
     int device;            /* CUDA ordinal */
-    int game_base;         /* global id of game 0 (sharding: RNG streams are keyed by global id) */
+    int game_base;         /* global id of game 0 (sharding: RNG streams are keyed by global id); 0..INT_MAX - n_games */
     int reversible_limit;  /* reversible-ply draw threshold; 0 = default 100 (unpinned, see DESIGN.md) */
     int move_stride;       /* row stride of per-game move/logit tables; 0 = default for board_n */
     uint32_t arena_slots;  /* node slots per game per arena half; 0 = sized from free HBM */
@@ -155,6 +155,24 @@ TZ_API int tz_result(tz_handle* h, const tz_state_t* states, int count, int* out
 /* Game::result in absolute terms (the suffix of a Replay line, target.rs:226-230):
  * 0 ongoing, 1 "R-0", 2 "0-R", 3 "F-0", 4 "0-F", 5 "1/2-1/2" */
 TZ_API int tz_game_result(tz_handle* h, const tz_state_t* states, int count, int* out_result);
+
+/* ---- device draws ----------------------------------------------------------------------- */
+/* Where a call takes NULL for its randomness, it draws on the device h = rng_hash(seed, a, b, c) (stated at
+ * tz_training_batch) with a = game_base + g, the global game id, so sharded handles draw what one handle would:
+ *   Gumbel noise (tz_gumbel_sequential_halving, tz_selfplay_move, tz_reanalyze_batch), child i of game g:
+ *     b = move counter, c = i; u = ((float)(h >> 41) + 0.5f) * 2^-23, exactly (x + 1/2) * 2^-23 for the 23-bit x,
+ *     in [2^-24, 1 - 2^-24]; noise = -logf(-logf(u)) in float32, finite
+ *   self-play sample (tz_select_selfplay, tz_selfplay_move): b = move counter, c = 0x5e1ec; the first child whose
+ *     cumulative weight exceeds h mod (total weight)
+ *   opening (tz_new_openings, tz_restart_terminal, the restart of tz_selfplay_move): b = opening counter,
+ *     c = 0x0fe11; sym = h & 7, adj = (h >> 3) & 1
+ *   random step (tz_random_steps): b = the ply before the step, c = 0x57e95; the move h mod count of
+ *     tz_legal_moves' list
+ * Counters of a handle, both 0 at tz_create: the move counter goes up by one at the end of every search of
+ * tz_gumbel_sequential_halving, tz_selfplay_move and tz_reanalyze_batch.  A search's noise uses the counter before it;
+ * tz_select_selfplay uses the current one, so after a search the one after it; tz_selfplay_move samples with the
+ * counter after its search (noise c, sample c + 1).  The opening counter goes up by one on every tz_new_openings and
+ * every restart (tz_restart_terminal and inside tz_selfplay_move), whether or not a game finished. */
 
 /* ---- positions ------------------------------------------------------------------------- */
 /* BatchedMCTS::from_envs / nodes_and_envs_mut writes (reanalyze/src/main.rs:159-165); roots reset */

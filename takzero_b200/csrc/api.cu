@@ -2,6 +2,7 @@
 // memory, host <-> device staging and the lock-step drivers of
 // BatchedMCTS::{simulate, gumbel_sequential_halving, step, restart_terminal_envs}
 // (takzero/src/search/node/batched.rs:63-409) on top of the kernels in kernels.cu / nn.cu.
+#include <limits.h>
 #include <math.h>
 #include <stdarg.h>
 #include <stdio.h>
@@ -105,6 +106,9 @@ extern "C" TZ_API int tz_create(const tz_config_t* cfg, tz_handle** out) {
     if (!cfg || !out) return fail(TZ_EINVAL, "null argument");
     if (cfg->board_n < 3 || cfg->board_n > 6) return fail(TZ_EINVAL, "board_n must be 3..6");
     if (cfg->n_games <= 0) return fail(TZ_EINVAL, "n_games must be positive");
+    // game ids game_base + g are int, and they key every device draw
+    if (cfg->game_base < 0 || cfg->game_base > INT_MAX - cfg->n_games)
+        return fail(TZ_EINVAL, "game_base must be 0..%d for %d games", INT_MAX - cfg->n_games, cfg->n_games);
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
         return fail(TZ_ECUDA, "no CUDA device: takzero_b200 has no CPU fallback");

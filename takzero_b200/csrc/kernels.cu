@@ -812,7 +812,9 @@ __global__ void k_gumbel_noise(TzDev d, float* out, int stride, unsigned long lo
     if (idx >= (size_t)d.G * stride) return;
     const int g = (int)(idx / stride), i = (int)(idx % stride);
     const uint64_t h = rng_hash(seed, (uint64_t)(d.game_base + g), counter, (uint64_t)i);
-    const float u = ((float)(h >> 40) + 0.5f) * (1.0f / 16777216.0f);  // (0,1)
+    // 23 bits: x + 0.5 is exact in float below 2^23, so u = (x + 0.5) * 2^-23 is exact, distinct for every x and at
+    // most 1 - 2^-24.  A 24-bit field would round x + 0.5 to even above 2^23 and reach u = 1.0f: +inf noise.
+    const float u = ((float)(h >> 41) + 0.5f) * (1.0f / 8388608.0f);
     out[idx] = -logf(-logf(u));
 }
 

@@ -240,6 +240,11 @@ def test_argument_errors():
     with pytest.raises(capi.TakzeroError, match="tz_set_weights"):
         m.set_agent(capi.AGENT_NETWORK)
     m.close()
+    # game ids game_base + g key every device draw and must fit an int
+    for base in (-1, 2**31 - 4, 2**31 - 1):
+        with pytest.raises(capi.TakzeroError, match="game_base"):
+            capi.BatchedMCTS(4, 4, 4, game_base=base, arena_slots=4096)
+    capi.BatchedMCTS(4, 4, 4, game_base=2**31 - 5, arena_slots=4096).close()
 
 
 def test_arena_overflow_is_reported():

@@ -6,9 +6,9 @@ row and column.  A spread keeps its pattern byte and maps its direction (0 '+', 
 import numpy as np
 import pytest
 
+from draws import rng_hash
 from oracle import oracle as O
 
-MASK64 = (1 << 64) - 1
 REVERSIBLE_LIMIT = 100
 
 
@@ -46,22 +46,6 @@ def sym_state(t: int, n: int, rec: np.ndarray) -> np.ndarray:
         to = r * n + c
         o_stack[to], o_height[to], o_top[to] = stack[sq], height[sq], top[sq]
     return out
-
-
-def mix64(x: int) -> int:
-    x ^= x >> 33
-    x = (x * 0xFF51AFD7ED558CCD) & MASK64
-    x ^= x >> 33
-    x = (x * 0xC4CEB9FE1A85EC53) & MASK64
-    x ^= x >> 33
-    return x
-
-
-def rng_hash(seed: int, a: int, b: int, c: int) -> int:
-    h = mix64((seed ^ 0x9E3779B97F4A7C15) & MASK64)
-    h = mix64(h ^ ((a * 0xBF58476D1CE4E5B9) & MASK64))
-    h = mix64(h ^ ((b * 0x94D049BB133111EB) & MASK64))
-    return mix64(h ^ ((c * 0xD6E8FEB86659FD93) & MASK64))
 
 
 def draw_index(seed: int, i: int, size: int) -> int:
