@@ -209,6 +209,7 @@ extern "C" {
     pub fn tz_target_buffer_append(h: *mut tz_handle, count: usize, env: *const tz_state_t, value: *const f32, ube: *const f32, n: *const c_int, offset: *const u64, moves: *const tz_move_t, probs: *const f32, n_policy: usize) -> c_int;
     pub fn tz_target_buffer_info(h: *mut tz_handle, size: *mut usize, appended: *mut u64) -> c_int;
     pub fn tz_training_batch(h: *mut tz_handle, params: *const tz_training_batch_t) -> c_int;
+    pub fn tz_update_counts_buffer(h: *mut tz_handle, params: *const tz_training_batch_t) -> c_int;
     pub fn tz_stage_positions(h: *mut tz_handle, states: *const tz_state_t, count: usize) -> c_int;
     pub fn tz_reanalyze_batch(h: *mut tz_handle, pool_indices: *const u32, params: *const tz_reanalyze_t) -> c_int;
     pub fn tz_reanalyze_read(h: *mut tz_handle, stride: c_int, out_policy: *mut f32, out_ube: *mut f32, out_value: *mut f32, out_n: *mut c_int, out_moves: *mut tz_move_t) -> c_int;
@@ -228,6 +229,7 @@ extern "C" {
     pub fn tz_comm_init(h: *mut tz_handle, id128: *const c_void, nranks: c_int, rank: c_int) -> c_int;
     pub fn tz_comm_destroy(h: *mut tz_handle) -> c_int;
     pub fn tz_broadcast_weights(h: *mut tz_handle, tensors: *const tz_tensor_t, count: c_int, res_blocks: c_int, root: c_int) -> c_int;
+    pub fn tz_broadcast_novelty_set(h: *mut tz_handle, bitset: *const u8, root: c_int) -> c_int;
     pub fn tz_weight_generation(h: *mut tz_handle, out_generation: *mut u64, out_ms: *mut f64) -> c_int;
     pub fn tz_allreduce_sum(h: *mut tz_handle, values: *mut u64, count: c_int) -> c_int;
     pub fn tz_load_model(h: *mut tz_handle, path: *const c_char) -> c_int;

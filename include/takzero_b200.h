@@ -358,6 +358,19 @@ typedef struct tz_training_batch_t {
     int* out_symmetry;
 } tz_training_batch_t;
 TZ_API int tz_training_batch(tz_handle* h, const tz_training_batch_t* params);
+/* `update_counts` (net6_simhash.rs:236-241) for a batch that stays on the device: reads only batch, indices, symmetry,
+ * augment and seed of `params` (the outputs are ignored), resolves example i's target index and symmetry exactly as
+ * tz_training_batch does (explicit arrays or the rng_hash draws above), and marks, in the handle's novelty set, the
+ * hash index (the hash set last: SimHash or LCG) of that target's position under that symmetry.  A learner passes the
+ * params of the batch it just trained on.  Which form the reference's `learn` marks -- the augmented position it
+ * trained on or the position as stored -- was not checked against the reference: the caller chooses, through
+ * symmetry / augment; augment = 0 (or all-zero symmetries) marks the positions as stored.
+ * Validation and codes as tz_training_batch (waits for the stream, then TZ_EINVAL for an empty buffer, batch <= 0, an
+ * index at or past the size or a symmetry above 7, nothing marked); TZ_ENOWEIGHTS without tz_set_simhash /
+ * tz_set_lcghash.  A set that is still the empty one of a fresh network becomes a real, zeroed one first (as in
+ * tz_update_counts).  Asynchronous: one kernel on the handle's stream, so on a self-play handle the marks land between
+ * the moves enqueued before and after the call. */
+TZ_API int tz_update_counts_buffer(tz_handle* h, const tz_training_batch_t* params);
 
 /* The loop body of `reanalyze` (reanalyze/src/main.rs:147-235) without per-batch host buffers.  tz_stage_positions
  * uploads the positions of the replay buffer once (position_buffer, main.rs:60-75); tz_reanalyze_batch makes the
@@ -448,6 +461,26 @@ TZ_API int tz_comm_destroy(tz_handle* h);
  * root takes it from its tensors as tz_set_weights does (a model without it switches it off), the other ranks keep
  * the one they had. */
 TZ_API int tz_broadcast_weights(tz_handle* h, const tz_tensor_t* tensors, int count, int res_blocks, int root);
+/* One novelty-set GENERATION on every rank of the communicator (collective; without one, or with nranks == 1, a set
+ * generation on one GPU): the 512 MiB set travels like the weight image of tz_broadcast_weights -- written into the
+ * inactive one of two sets on the same side stream, ncclBroadcast to the inactive set of every other rank, swapped for
+ * the launches each rank enqueues afterwards; launches already enqueued keep reading the old set.  The second set is
+ * allocated by the first call (a handle that never calls this holds one set).  Every rank needs a network
+ * (TZ_ENOWEIGHTS otherwise).  The root's `bitset`:
+ *   a host image in the bitvec.bin layout (2^29 bytes, LSB-first) in pinned memory (tz_host_alloc): uploaded from
+ *     where it is, asynchronously; leave it unchanged until tz_sync
+ *   a host image in pageable memory: copied before the call returns, through a 16 MiB pinned staging buffer of the
+ *     handle (the call then waits until the readers of the set it overwrites, the launches enqueued before the last
+ *     swap, have run)
+ *   NULL: the root's own current set, marks of tz_update_counts / tz_update_counts_buffer enqueued before the call
+ *     included (the copy waits for them on the device)
+ * The other ranks pass NULL.  The root needs a hash (tz_set_simhash / tz_set_lcghash, else TZ_ENOWEIGHTS); the
+ * broadcast carries its hash kind and board size, and a rank whose hash differs, or that has none, raises
+ * TZ_STATUS_WEIGHTS_MISMATCH on the device and keeps its old set.  The SimHash matrix / LCG multipliers are not
+ * broadcast: they come with the model (tz_set_simhash, tz_set_lcghash, tz_load_model), as before.  TZ_EINVAL, nothing
+ * changed, for a root out of range or a non-NULL bitset on another rank.  Sets are not OR-reduced over ranks: the
+ * root's set is the set (one learner). */
+TZ_API int tz_broadcast_novelty_set(tz_handle* h, const uint8_t* bitset, int root);
 /* number of generations so far and the device time of the last one (upload + fold + broadcast); waits for it */
 TZ_API int tz_weight_generation(tz_handle* h, uint64_t* out_generation, double* out_ms);
 /* in-place sum over all ranks of up to 64 counters (simulations, positions, targets, finished games ...) */

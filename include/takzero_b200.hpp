@@ -486,6 +486,11 @@ class BatchedMCTS {
             t[i] = tz_tensor_t{w->names[i].c_str(), w->data[i].data(), w->shapes[i].data(), (int)w->shapes[i].size()};
         check(tz_broadcast_weights(h_, t.data(), (int)t.size(), res_blocks, root));
     }
+    // The novelty set that goes with a model, as ONE collective: the root passes a bitvec.bin image (2^29 bytes) or
+    // nullptr for its own set, the others nullptr; all ranks swap sets between moves (see tz_broadcast_novelty_set).
+    void broadcast_novelty_set(const uint8_t* bitset = nullptr, int root = 0) {
+        check(tz_broadcast_novelty_set(h_, bitset, root));
+    }
     std::vector<uint64_t> allreduce_sum(std::vector<uint64_t> values) {
         check(tz_allreduce_sum(h_, values.data(), (int)values.size()));
         return values;
@@ -626,6 +631,8 @@ class BatchedMCTS {
     }
     // one batch into caller-owned device memory (see tz_training_batch); asynchronous, sync() waits
     void training_batch(const tz_training_batch_t& params) { check(tz_training_batch(h_, &params)); }
+    // mark the examples of that batch in the novelty set (see tz_update_counts_buffer); asynchronous
+    void update_counts_buffer(const tz_training_batch_t& params) { check(tz_update_counts_buffer(h_, &params)); }
     void set_agent(int kind, tz_agent_fn fn = nullptr, void* ctx = nullptr) { check(tz_set_agent(h_, kind, fn, ctx)); }
     void new_openings(uint64_t seed) { check(tz_new_openings(h_, nullptr, nullptr, nullptr, seed)); }
     void set_positions(const std::vector<tz_state_t>& envs) { check(tz_set_positions(h_, envs.data(), nullptr)); }

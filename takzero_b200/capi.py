@@ -214,6 +214,7 @@ def lib():
         "tz_target_buffer_append": ([vp, C.c_size_t, vp, vp, vp, vp, vp, vp, vp, C.c_size_t], i32),
         "tz_target_buffer_info": ([vp, P(C.c_size_t), P(u64)], i32),
         "tz_training_batch": ([vp, P(TrainingBatchParams)], i32),
+        "tz_update_counts_buffer": ([vp, P(TrainingBatchParams)], i32),
         "tz_stage_positions": ([vp, vp, C.c_size_t], i32),
         "tz_reanalyze_batch": ([vp, vp, P(ReanalyzeParams)], i32),
         "tz_reanalyze_read": ([vp, i32, vp, vp, vp, vp, vp], i32),
@@ -627,6 +628,15 @@ class BatchedMCTS:
         _check(lib().tz_training_batch(self._h, C.byref(p)))
         self.sync()
         return out
+
+    def update_counts_buffer(self, batch: int, seed: int, augment: bool = True, indices=None, symmetry=None) -> None:
+        """Mark the examples of a training batch in the novelty set (tz_update_counts_buffer): the same arguments as
+        training_batch resolve the same targets and symmetries, and each one's transformed position is marked.
+        augment=False (or zero symmetries) marks the positions as stored.  Asynchronous on the handle's stream."""
+        idx = None if indices is None else _arr(indices, np.uint64, (batch,))
+        sym = None if symmetry is None else _arr(symmetry, np.int32, (batch,))
+        p = TrainingBatchParams(batch, _ptr(idx), _ptr(sym), 1 if augment else 0, seed)
+        _check(lib().tz_update_counts_buffer(self._h, C.byref(p)))
 
     # ---- reanalyze (reanalyze/src/main.rs:147-235) ---------------------------------------------------------
     def stage_positions(self, states: np.ndarray) -> None:

@@ -924,6 +924,13 @@ extern "C" TZ_API int tz_broadcast_weights(tz_handle* h, const tz_tensor_t* tens
     return TZ_OK;
 }
 
+extern "C" TZ_API int tz_broadcast_novelty_set(tz_handle* h, const uint8_t* bitset, int root) {
+    CHECK_H(h);
+    const int rc = nn_broadcast_novelty_set(h, bitset, root);
+    if (rc) return fail(rc, "tz_broadcast_novelty_set: %s", nn_last_error());
+    return TZ_OK;
+}
+
 extern "C" TZ_API int tz_weight_generation(tz_handle* h, uint64_t* out_generation, double* out_ms) {
     CHECK_H(h);
     double ms = 0.0;
@@ -1433,19 +1440,14 @@ static int check_device_output(tz_handle* h, const void* p, size_t align, const 
     return TZ_OK;
 }
 
-extern "C" TZ_API int tz_training_batch(tz_handle* h, const tz_training_batch_t* p) {
-    CHECK_H(h);
-    if (!p) return fail(TZ_EINVAL, "null parameters");
+// The examples of a batch (tz_training_batch, tz_update_counts_buffer): waits for the stream (queued self-play appends
+// land first), validates the host indices / symmetries against the buffer's size and stages them on the device.
+// *size = targets kept, *first = ring slot of the oldest one.
+static int stage_batch_examples(tz_handle* h, const tz_training_batch_t* p, unsigned long long* size_out,
+                                unsigned long long* first_out) {
     TzTargetRing& R = h->ring;
-    if (!R.env) return fail(TZ_EINVAL, "no target buffer: tz_target_buffer first");
-    if (p->batch <= 0) return fail(TZ_EINVAL, "batch must be > 0");
-    int rc;
-    if ((rc = check_device_output(h, p->planes, 4, "planes")) || (rc = check_device_output(h, p->policy, 4, "policy")) ||
-        (rc = check_device_output(h, p->mask, 1, "mask")) || (rc = check_device_output(h, p->value, 4, "value")) ||
-        (rc = check_device_output(h, p->ube, 4, "ube")) || (rc = check_device_output(h, p->out_index, 4, "out_index")) ||
-        (rc = check_device_output(h, p->out_symmetry, 4, "out_symmetry")))
-        return rc;
     unsigned long long appended = 0;
+    int rc;
     if ((rc = ring_appended(h, &appended))) return rc;
     const unsigned long long size = std::min<unsigned long long>(appended, R.cap);
     if (size == 0) return fail(TZ_EINVAL, "the target buffer is empty");
@@ -1473,12 +1475,47 @@ extern "C" TZ_API int tz_training_batch(tz_handle* h, const tz_training_batch_t*
         CU(cudaMemcpyAsync(h->batch_idx, p->indices, B * sizeof(uint64_t), cudaMemcpyHostToDevice, h->stream));
     if (p->symmetry)
         CU(cudaMemcpyAsync(h->batch_sym, p->symmetry, B * sizeof(int), cudaMemcpyHostToDevice, h->stream));
+    *size_out = size;
+    *first_out = (appended - size) % R.cap;
+    return TZ_OK;
+}
+
+extern "C" TZ_API int tz_training_batch(tz_handle* h, const tz_training_batch_t* p) {
+    CHECK_H(h);
+    if (!p) return fail(TZ_EINVAL, "null parameters");
+    TzTargetRing& R = h->ring;
+    if (!R.env) return fail(TZ_EINVAL, "no target buffer: tz_target_buffer first");
+    if (p->batch <= 0) return fail(TZ_EINVAL, "batch must be > 0");
+    int rc;
+    if ((rc = check_device_output(h, p->planes, 4, "planes")) || (rc = check_device_output(h, p->policy, 4, "policy")) ||
+        (rc = check_device_output(h, p->mask, 1, "mask")) || (rc = check_device_output(h, p->value, 4, "value")) ||
+        (rc = check_device_output(h, p->ube, 4, "ube")) || (rc = check_device_output(h, p->out_index, 4, "out_index")) ||
+        (rc = check_device_output(h, p->out_symmetry, 4, "out_symmetry")))
+        return rc;
+    unsigned long long size = 0, first = 0;
+    if ((rc = stage_batch_examples(h, p, &size, &first))) return rc;
     const TzBatchOut o = {p->planes, p->policy, p->mask, p->value, p->ube, p->out_index, p->out_symmetry};
-    const unsigned long long first = (appended - size) % R.cap;
     launch_training_batch(R, h->d.n, h->d.half_komi, p->batch, p->indices ? h->batch_idx : nullptr,
                           p->symmetry ? h->batch_sym : nullptr, p->augment, p->seed, size, first, o, h->stream);
     h->launches += 1;
     CU(cudaGetLastError());
+    return TZ_OK;
+}
+
+extern "C" TZ_API int tz_update_counts_buffer(tz_handle* h, const tz_training_batch_t* p) {
+    CHECK_H(h);
+    if (!p) return fail(TZ_EINVAL, "null parameters");
+    TzTargetRing& R = h->ring;
+    if (!R.env) return fail(TZ_EINVAL, "no target buffer: tz_target_buffer first");
+    if (p->batch <= 0) return fail(TZ_EINVAL, "batch must be > 0");
+    if (nn_hash_kind(h) == 0)
+        return fail(TZ_ENOWEIGHTS, "tz_update_counts_buffer needs tz_set_simhash / tz_set_lcghash first (the set takes 512 MiB of HBM)");
+    unsigned long long size = 0, first = 0;
+    int rc;
+    if ((rc = stage_batch_examples(h, p, &size, &first))) return rc;
+    rc = nn_update_counts_buffer(h, R, p->batch, p->indices ? h->batch_idx : nullptr, p->symmetry ? h->batch_sym : nullptr,
+                                 p->augment, p->seed, size, first);
+    if (rc) return fail(rc, "tz_update_counts_buffer: %s", rc == TZ_ENOMEM ? "cudaMalloc of the 512 MiB set failed" : "launch failed");
     return TZ_OK;
 }
 

@@ -796,12 +796,7 @@ __global__ void __launch_bounds__(32 * TREE_WARPS) k_tree_backward(TzDev d, int 
 
 // ---- Gumbel top-k and sequential halving -----------------------------------------------
 
-__device__ __forceinline__ uint64_t rng_hash(uint64_t seed, uint64_t a, uint64_t b, uint64_t c) {
-    uint64_t h = tz_mix64(seed ^ 0x9e3779b97f4a7c15ULL);
-    h = tz_mix64(h ^ (a * 0xbf58476d1ce4e5b9ULL));
-    h = tz_mix64(h ^ (b * 0x94d049bb133111ebULL));
-    return tz_mix64(h ^ (c * 0xd6e8feb86659fd93ULL));
-}
+// rng_hash: rules.cuh
 
 // Gumbel(0,1) noise for every (game, child index): the reference draws from `rand`
 // (batched.rs:226-227), whose stream is not pinned, so this is our own counter-based
@@ -1844,18 +1839,8 @@ __global__ void __launch_bounds__(32 * WPB) k_target_append(TzTargetRing R, cons
     }
 }
 
-// symmetry t of the board (tz_training_batch): bit 0 mirrors the column, bit 1 the row, bit 2 swaps them, in this order
-__device__ __forceinline__ void sym_square(int t, int n, int* row, int* col) {
-    if (t & 1) *col = n - 1 - *col;
-    if (t & 2) *row = n - 1 - *row;
-    if (t & 4) {
-        const int tmp = *col;
-        *col = *row;
-        *row = tmp;
-    }
-}
-
-// the same on a move: the square as above, a spread's direction (0 '+', 1 '-', 2 '<', 3 '>') alike, the pattern kept
+// symmetry t of the board (rules.cuh `sym_square`) on a move: the square as there, a spread's direction (0 '+', 1 '-',
+// 2 '<', 3 '>') alike, the pattern kept
 __device__ __forceinline__ uint16_t sym_move(int t, int n, uint16_t m) {
     int col = m & 7, row = (m >> 3) & 7, kd = (m >> 6) & 3;
     const int pat = m >> 8;
@@ -1899,9 +1884,9 @@ __global__ void __launch_bounds__(TB_THREADS) k_training_batch(TzTargetRing R, i
     const int e = warp / team, team_threads = team * 32, ttid = threadIdx.x - e * team_threads;
     const int b = blockIdx.x * (TB_THREADS / 32 / team) + e;
     const bool valid = b < batch;
-    const unsigned long long idx =
-        !valid ? 0ull : indices ? indices[b] : __umul64hi(rng_hash(seed, (uint64_t)b, 0, 0), size);
-    const int t = !valid ? 0 : symmetry ? symmetry[b] : augment ? (int)(rng_hash(seed, (uint64_t)b, 1, 0) & 7) : 0;
+    unsigned long long idx = 0;
+    int t = 0;
+    if (valid) batch_example(indices, symmetry, augment, seed, size, b, &idx, &t);
     const unsigned long long slot = (first + idx) % R.cap;
     const int nn = n * n;
     const size_t row_len = (size_t)(3 + 4 * ((1 << n) - 2)) * nn;
@@ -1911,16 +1896,7 @@ __global__ void __launch_bounds__(TB_THREADS) k_training_batch(TzTargetRing R, i
         TzState* src = &s_src[e];
         TzState* dst = &s_dst[e];
         warp_load_state(src, &R.env[slot], lane);
-        warp_load_state(dst, src, lane);
-        for (int sq = lane; sq < nn; sq += 32) {
-            int row = sq / n, col = sq - row * n;
-            sym_square(t, n, &row, &col);
-            const int to = row * n + col;
-            dst->stack[to] = src->stack[sq];
-            dst->height[to] = src->height[sq];
-            dst->top[to] = src->top[sq];
-        }
-        __syncwarp();
+        warp_symmetric_state(dst, src, t, n, lane);
         if (o.planes) warp_encode_planes(dst, n, half_komi, o.planes + (size_t)b * (2 * (2 * n + 5) + 2) * nn, lane);
         if (lane == 0) {
             if (o.value) o.value[b] = R.value[slot];

@@ -15,6 +15,7 @@
 
 #include <string>
 #include <type_traits>
+#include <utility>
 #include <vector>
 
 #include "comm.cuh"
@@ -30,6 +31,9 @@
 #define CIN_PAD 64
 #define SET_HEADER_BYTES 256
 #define SET_MAGIC 0x53575a54u  // "TZWS"
+#define NOVELTY_BYTES ((size_t)1 << 29)        // the 2^32-bit novelty set (bitvec.bin)
+#define NOVELTY_STAGE_BYTES ((size_t)8 << 20)  // each of the two pinned chunks a pageable set image goes through
+#define NOVELTY_MAGIC 0x53535a54u              // "TZSS": header of a broadcast novelty set
 
 // Byte offsets inside one weight set (a single device allocation, so that a generation travels as ONE broadcast):
 // [header 256 B][per convolution: blocks in the shared-memory image the tensor core reads, then 256 f32 biases]
@@ -92,6 +96,15 @@ struct NnState {
     uint32_t* simhash_set = nullptr;  // 2^32-bit set (bitvec.bin), optional; absent = empty set
     uint32_t* simhash_set_alloc = nullptr;
     uint32_t* simhash_idx = nullptr;  // [max_positions] hash index of each queued position
+    // set generations (tz_broadcast_novelty_set), all created by the first one: the inactive set the next generation
+    // is written into (swapped with simhash_set_alloc), the broadcast header ([0..3] magic, hash kind, board size;
+    // [4] this rank's mismatch flag), the pinned chunks of pageable images and their events
+    uint32_t* set_spare = nullptr;
+    uint32_t* set_hdr = nullptr;
+    unsigned char* set_pin = nullptr;
+    cudaEvent_t ev_stage[2] = {nullptr, nullptr};  // wstream: chunk k of set_pin has been read
+    bool stage_used[2] = {false, false};
+    cudaEvent_t ev_marks = nullptr;  // search stream: the marks a generation copies (or keeps) have landed
     size_t progress_len = 0;
     unsigned* progress = nullptr;     // [chunks][pair tiles] tile-completion counters of the fused launch, then
                                       // [chunks] chunk-completion counters
@@ -112,7 +125,9 @@ void nn_free(tz_handle* h) {
     for (void* p : s->allocs) cudaFree(p);
     if (s->raw_pin) cudaFreeHost(s->raw_pin);
     if (s->head_pin) cudaFreeHost(s->head_pin);
-    for (cudaEvent_t e : {s->ev_ready, s->ev_swap, s->ev_h2d, s->ev_gen[0], s->ev_gen[1]})
+    if (s->set_pin) cudaFreeHost(s->set_pin);
+    for (cudaEvent_t e : {s->ev_ready, s->ev_swap, s->ev_h2d, s->ev_gen[0], s->ev_gen[1], s->ev_stage[0], s->ev_stage[1],
+                          s->ev_marks})
         if (e) cudaEventDestroy(e);
     if (s->wstream) cudaStreamDestroy(s->wstream);
     delete s;
@@ -167,48 +182,28 @@ __global__ void k_encode16(const TzState* states, int count, int n, int f16, flo
 
 // ---- SimHash novelty index (net6_simhash.rs:203-234 `get_indices`) ---------------------------------
 
-// One warp per position, lane = hash bit: dot of the f32 planes (side-to-move plane zeroed) with column
-// `lane` of the [C*N*N][32] matrix; bit set when the dot is >= 0; index = sum of 2^bit.
-__global__ void __launch_bounds__(32 * WPB) k_simhash(const TzState* states, const int* count_ptr, int count_max, int n,
-                                                       int half_komi, const float* matrix, uint32_t* out_idx) {
-    __shared__ TzState s_state[WPB];
-    __shared__ float s_planes[WPB][36 * 36];
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int q = blockIdx.x * WPB + warp;
-    const int count = count_ptr ? *count_ptr : count_max;
-    if (q >= count) return;
-    TzState* st = &s_state[warp];
-    warp_load_state(st, &states[q], lane);
+// One warp, lane = hash bit: dot of the f32 planes (side-to-move plane zeroed, built in x) with column `lane` of the
+// [C*N*N][32] matrix; bit set when the dot is >= 0; index = sum of 2^bit, in every lane.
+__device__ __forceinline__ uint32_t warp_simhash(const TzState* st, int n, int half_komi, const float* matrix, float* x,
+                                                 int lane) {
     const int nn = n * n, C = 2 * (2 * n + 3 + 2) + 2;
-    float* x = s_planes[warp];
     warp_fill_planes(x, st, n, half_komi, lane, true);
     float dot = 0.0f;
     const int total = C * nn;
     for (int j = 0; j < total; j++) dot = fmaf(x[j], matrix[(size_t)j * 32 + lane], dot);
-    const uint32_t bits = __ballot_sync(0xffffffffu, !(dot < 0.0f));
-    if (lane == 0) out_idx[q] = bits;
+    return __ballot_sync(0xffffffffu, !(dot < 0.0f));
 }
 
 // ---- LCG-hash novelty index (net4_lcghash.rs:203-241 `get_indices`) -------------------------------------
 // planes * lcghash_init (f32, elementwise) reinterpreted as i32, folded with the 64-bit LCG
 // acc = acc * 6364136223846793005 + 1 + v  along the columns, then the rows, then the channels (wrapping i64);
-// index = |acc| >> 31.  Integer work: bit-exact.  One warp per position.
-__global__ void __launch_bounds__(32 * WPB) k_lcghash(const TzState* states, const int* count_ptr, int count_max, int n,
-                                                       int half_komi, const float* init, uint32_t* out_idx) {
-    __shared__ TzState s_state[WPB];
-    __shared__ float s_planes[WPB][36 * 36];
-    __shared__ unsigned long long s_rows[WPB][36 * 6];
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int q = blockIdx.x * WPB + warp;
-    const int count = count_ptr ? *count_ptr : count_max;
-    if (q >= count) return;
-    TzState* st = &s_state[warp];
-    warp_load_state(st, &states[q], lane);
+// index = |acc| >> 31.  Integer work: bit-exact.  One warp (x: the planes, rows: C * N folds); the index is valid in
+// lane 0.
+__device__ __forceinline__ uint32_t warp_lcghash(const TzState* st, int n, int half_komi, const float* init, float* x,
+                                                 unsigned long long* rows, int lane) {
     const int C = 2 * (2 * n + 3 + 2) + 2;
-    float* x = s_planes[warp];
     warp_fill_planes(x, st, n, half_komi, lane, false);
     const unsigned long long MUL = 6364136223846793005ull;
-    unsigned long long* rows = s_rows[warp];
     for (int cr = lane; cr < C * n; cr += 32) {  // (channel, row): fold the columns
         unsigned long long acc = 0;
         for (int j = 0; j < n; j++) {
@@ -226,13 +221,70 @@ __global__ void __launch_bounds__(32 * WPB) k_lcghash(const TzState* states, con
         rows[c * n] = acc;
     }
     __syncwarp();
+    uint32_t index = 0;
     if (lane == 0) {
         unsigned long long acc = 0;
         for (int c = 0; c < C; c++) acc = acc * MUL + 1ull + rows[c * n];
         long long sacc = (long long)acc;
         if (sacc < 0) sacc = -sacc;  // i64::MIN stays negative, as a wrapping abs does
-        out_idx[q] = (uint32_t)((unsigned long long)sacc >> 31);
+        index = (uint32_t)((unsigned long long)sacc >> 31);
     }
+    return index;
+}
+
+// One warp per position: the hash index of every position.
+__global__ void __launch_bounds__(32 * WPB) k_simhash(const TzState* states, const int* count_ptr, int count_max, int n,
+                                                       int half_komi, const float* matrix, uint32_t* out_idx) {
+    __shared__ TzState s_state[WPB];
+    __shared__ float s_planes[WPB][36 * 36];
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int q = blockIdx.x * WPB + warp;
+    const int count = count_ptr ? *count_ptr : count_max;
+    if (q >= count) return;
+    TzState* st = &s_state[warp];
+    warp_load_state(st, &states[q], lane);
+    const uint32_t bits = warp_simhash(st, n, half_komi, matrix, s_planes[warp], lane);
+    if (lane == 0) out_idx[q] = bits;
+}
+
+__global__ void __launch_bounds__(32 * WPB) k_lcghash(const TzState* states, const int* count_ptr, int count_max, int n,
+                                                       int half_komi, const float* init, uint32_t* out_idx) {
+    __shared__ TzState s_state[WPB];
+    __shared__ float s_planes[WPB][36 * 36];
+    __shared__ unsigned long long s_rows[WPB][36 * 6];
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int q = blockIdx.x * WPB + warp;
+    const int count = count_ptr ? *count_ptr : count_max;
+    if (q >= count) return;
+    TzState* st = &s_state[warp];
+    warp_load_state(st, &states[q], lane);
+    const uint32_t index = warp_lcghash(st, n, half_komi, init, s_planes[warp], s_rows[warp], lane);
+    if (lane == 0) out_idx[q] = index;
+}
+
+// tz_update_counts_buffer: one warp per example of a training batch.  The example's target (resolved as
+// k_training_batch does) is read from the ring, transformed by its symmetry, hashed with the handle's hash
+// (kind 1 SimHash: w = matrix, 2 LCG: w = multipliers) and its bit ORed into the set.
+__global__ void __launch_bounds__(32 * WPB) k_mark_batch(TzTargetRing R, int n, int half_komi, int batch,
+                                                          const unsigned long long* indices, const int* symmetry,
+                                                          int augment, unsigned long long seed, unsigned long long size,
+                                                          unsigned long long first, int kind, const float* w,
+                                                          uint32_t* set) {
+    __shared__ TzState s_src[WPB], s_dst[WPB];
+    __shared__ float s_planes[WPB][36 * 36];
+    __shared__ unsigned long long s_rows[WPB][36 * 6];
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int b = blockIdx.x * WPB + warp;
+    if (b >= batch) return;
+    unsigned long long idx;
+    int t;
+    batch_example(indices, symmetry, augment, seed, size, b, &idx, &t);
+    const unsigned long long slot = (first + idx) % R.cap;
+    warp_load_state(&s_src[warp], &R.env[slot], lane);
+    warp_symmetric_state(&s_dst[warp], &s_src[warp], t, n, lane);
+    const uint32_t index = kind == 2 ? warp_lcghash(&s_dst[warp], n, half_komi, w, s_planes[warp], s_rows[warp], lane)
+                                     : warp_simhash(&s_dst[warp], n, half_komi, w, s_planes[warp], lane);
+    if (lane == 0) atomicOr(&set[index >> 5], 1u << (index & 31));
 }
 
 // ---- host-supplied positions (tz_evaluate): what k_select provides for queued leaves ------------------------
@@ -740,20 +792,30 @@ static int upload_and_fold(tz_handle* h, int target) {
     return TZ_OK;
 }
 
-// The new set is complete on wstream: launches enqueued from now on read it (after waiting for it), and the event
-// recorded here on the search stream marks the end of the old set's readers.
+// The new set (weights or novelty) is complete on wstream: launches enqueued from now on wait for it
+static bool search_waits_for_wstream(tz_handle* h) {
+    NnState* s = h->nn;
+    return cudaEventRecord(s->ev_ready, s->wstream) == cudaSuccess && cudaStreamWaitEvent(h->stream, s->ev_ready, 0) == cudaSuccess;
+}
+// after a swap: the event recorded on the search stream marks the end of the swapped-out set's readers, which every
+// later generation waits for before it writes into an inactive set
+static void record_swap(tz_handle* h) {
+    NnState* s = h->nn;
+    cudaEventRecord(s->ev_swap, h->stream);
+    s->swap_recorded = true;
+    bind_search(h);
+}
+
+// The new weight set is complete on wstream: launches enqueued from now on read it
 static int publish(tz_handle* h, int target) {
     NnState* s = h->nn;
     cudaEventRecord(s->ev_gen[1], s->wstream);
     s->gen_timed = true;
-    if (cudaEventRecord(s->ev_ready, s->wstream) != cudaSuccess || cudaStreamWaitEvent(h->stream, s->ev_ready, 0) != cudaSuccess)
-        NN_FAIL(TZ_ECUDA, "publishing the weight set failed");
+    if (!search_waits_for_wstream(h)) NN_FAIL(TZ_ECUDA, "publishing the weight set failed");
     s->set_f16[target] = h->nn_f16;
     s->active = target;
     s->generation++;
-    cudaEventRecord(s->ev_swap, h->stream);
-    s->swap_recorded = true;
-    bind_search(h);
+    record_swap(h);
     return TZ_OK;
 }
 
@@ -1264,19 +1326,27 @@ __global__ void k_set_bits(const uint32_t* __restrict__ idx, int count, uint32_t
     if (i < count) atomicOr(&set[idx[i] >> 5], 1u << (idx[i] & 31));
 }
 
-int nn_update_counts(tz_handle* h, const TzState* states_dev, int count, uint32_t* idx_dev) {
+// the empty set of a fresh network becomes a real, zeroed one before it is marked
+static int ensure_marked_set(tz_handle* h) {
     NnState* s = h->nn;
-    if (!s || s->novelty == 0) return TZ_ENOWEIGHTS;
-    const size_t bytes = (size_t)1 << 29;
     if (!s->simhash_set_alloc) {
-        if (cudaMalloc((void**)&s->simhash_set_alloc, bytes) != cudaSuccess) return TZ_ENOMEM;
+        if (cudaMalloc((void**)&s->simhash_set_alloc, NOVELTY_BYTES) != cudaSuccess) return TZ_ENOMEM;
         s->allocs.push_back(s->simhash_set_alloc);
     }
-    if (!s->simhash_set) {  // the empty set of a fresh network becomes a real one
-        if (cudaMemsetAsync(s->simhash_set_alloc, 0, bytes, h->stream) != cudaSuccess) return TZ_ECUDA;
+    if (!s->simhash_set) {
+        if (cudaMemsetAsync(s->simhash_set_alloc, 0, NOVELTY_BYTES, h->stream) != cudaSuccess) return TZ_ECUDA;
         s->simhash_set = s->simhash_set_alloc;
         bind_search(h);
     }
+    return TZ_OK;
+}
+
+int nn_hash_kind(const tz_handle* h) { return h->nn ? h->nn->novelty : 0; }
+
+int nn_update_counts(tz_handle* h, const TzState* states_dev, int count, uint32_t* idx_dev) {
+    NnState* s = h->nn;
+    if (!s || s->novelty == 0) return TZ_ENOWEIGHTS;
+    if (const int erc = ensure_marked_set(h)) return erc;
     const int rc = s->novelty == 2 ? nn_lcghash_indices(h, states_dev, count, idx_dev)
                                    : nn_simhash_indices(h, states_dev, count, idx_dev);
     if (rc) return rc;
@@ -1295,4 +1365,133 @@ int nn_read_novelty_set(tz_handle* h, unsigned char* out_host) {
         return TZ_OK;
     }
     return cudaMemcpy(out_host, s->simhash_set, bytes, cudaMemcpyDeviceToHost) == cudaSuccess ? TZ_OK : TZ_ECUDA;
+}
+
+// tz_update_counts_buffer: mark the examples of a training batch (k_mark_batch) on the search stream
+int nn_update_counts_buffer(tz_handle* h, const TzTargetRing& R, int batch, const unsigned long long* indices,
+                            const int* symmetry, int augment, unsigned long long seed, unsigned long long size,
+                            unsigned long long first) {
+    NnState* s = h->nn;
+    if (!s || s->novelty == 0) return TZ_ENOWEIGHTS;
+    if (const int rc = ensure_marked_set(h)) return rc;
+    const float* w = s->novelty == 2 ? s->lcghash_init : s->simhash_matrix;
+    k_mark_batch<<<(batch + WPB - 1) / WPB, 32 * WPB, 0, h->stream>>>(R, h->d.n, h->d.half_komi, batch, indices, symmetry,
+                                                                      augment, seed, size, first, s->novelty, w,
+                                                                      s->simhash_set);
+    h->launches += 1;
+    return cudaGetLastError() == cudaSuccess ? TZ_OK : TZ_ECUDA;
+}
+
+// ---- novelty-set generations (tz_broadcast_novelty_set) ------------------------------------------------------
+
+__global__ void k_novelty_header(uint32_t* hdr, uint32_t kind, uint32_t n) {
+    hdr[0] = NOVELTY_MAGIC;
+    hdr[1] = kind;
+    hdr[2] = n;
+    hdr[3] = 0;
+}
+
+// after a broadcast: the set that arrived must be indexed by this rank's hash (kind and board size); hdr[4] says
+// whether it is not
+__global__ void k_check_novelty(uint32_t* hdr, uint32_t kind, uint32_t n, uint32_t* status) {
+    const bool bad = hdr[0] != NOVELTY_MAGIC || hdr[1] != kind || hdr[2] != n;
+    hdr[4] = bad ? 1u : 0u;
+    if (bad) atomicOr(status, TZ_ERR_WEIGHTS_MISMATCH);
+}
+
+// a rank whose check failed keeps its old set: the received one is overwritten with it (zeroes for the empty set)
+// before the swap; nothing to do otherwise
+__global__ void k_keep_novelty(const uint32_t* hdr, uint4* dst, const uint4* src, size_t count) {
+    if (!hdr[4]) return;
+    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < count; i += (size_t)gridDim.x * blockDim.x)
+        dst[i] = src ? src[i] : make_uint4(0u, 0u, 0u, 0u);
+}
+
+// One set generation on every rank of the handle's communicator, on the weight stream beside the search: the root
+// writes the new set into its inactive set (from a host image, or bitset = NULL: its own current set, marks enqueued
+// before the call included), ncclBroadcast sends the hash kind and the set into every other rank's inactive set, and
+// every rank swaps for the launches it enqueues afterwards.  The inactive set is written only after the readers of the
+// last swap (ev_swap), as for the weights.
+int nn_broadcast_novelty_set(tz_handle* h, const unsigned char* bitset, int root) {
+    cudaSetDevice(h->device);
+    const int nranks = comm_nranks(h), rank = comm_rank(h);
+    if (root < 0 || root >= nranks) NN_FAIL(TZ_EINVAL, "root %d of %d ranks", root, nranks);
+    if (rank != root && bitset) NN_FAIL(TZ_EINVAL, "rank %d is not the root (%d): only the root passes a set", rank, root);
+    NnState* s = h->nn;
+    if (!s || s->active < 0) NN_FAIL(TZ_ENOWEIGHTS, "no network: tz_set_weights / tz_broadcast_weights first");
+    if (rank == root && s->novelty == 0) NN_FAIL(TZ_ENOWEIGHTS, "the root has no hash: tz_set_simhash / tz_set_lcghash first");
+    if (!s->set_spare) {
+        if (cudaMalloc((void**)&s->set_spare, NOVELTY_BYTES) != cudaSuccess) {
+            cudaGetLastError();
+            NN_FAIL(TZ_ENOMEM, "cudaMalloc of the second 512 MiB novelty set failed");
+        }
+        s->allocs.push_back(s->set_spare);
+    }
+    if (!s->set_hdr) {
+        if (cudaMalloc((void**)&s->set_hdr, 8 * sizeof(uint32_t)) != cudaSuccess) NN_FAIL(TZ_ENOMEM, "cudaMalloc failed");
+        s->allocs.push_back(s->set_hdr);
+    }
+    if (!s->ev_marks) {
+        bool ok = true;
+        for (cudaEvent_t* e : {&s->ev_marks, &s->ev_stage[0], &s->ev_stage[1]})
+            ok = ok && cudaEventCreateWithFlags(e, cudaEventDisableTiming) == cudaSuccess;
+        if (!ok) NN_FAIL(TZ_ECUDA, "event creation failed");
+    }
+    uint32_t* target = s->set_spare;
+    if (s->swap_recorded && cudaStreamWaitEvent(s->wstream, s->ev_swap, 0) != cudaSuccess) NN_FAIL(TZ_ECUDA, "cudaStreamWaitEvent");
+    if (cudaEventRecord(s->ev_marks, h->stream) != cudaSuccess) NN_FAIL(TZ_ECUDA, "cudaEventRecord");
+    cudaError_t e = cudaSuccess;
+    if (rank == root) {
+        if (!bitset) {
+            // the root's own set, once the marks enqueued before this call have landed
+            e = cudaStreamWaitEvent(s->wstream, s->ev_marks, 0);
+            if (e == cudaSuccess)
+                e = s->simhash_set ? cudaMemcpyAsync(target, s->simhash_set, NOVELTY_BYTES, cudaMemcpyDeviceToDevice, s->wstream)
+                                   : cudaMemsetAsync(target, 0, NOVELTY_BYTES, s->wstream);
+        } else if (is_pinned(bitset)) {
+            e = cudaMemcpyAsync(target, bitset, NOVELTY_BYTES, cudaMemcpyHostToDevice, s->wstream);
+        } else {
+            // pageable: through two pinned chunks in turn, so that the caller's image has been read when the call returns
+            if (!s->set_pin && cudaHostAlloc((void**)&s->set_pin, 2 * NOVELTY_STAGE_BYTES, cudaHostAllocDefault) != cudaSuccess) {
+                cudaGetLastError();
+                s->set_pin = nullptr;
+                NN_FAIL(TZ_ENOMEM, "cudaHostAlloc of the %zu MiB set staging failed", 2 * NOVELTY_STAGE_BYTES >> 20);
+            }
+            for (size_t off = 0, i = 0; off < NOVELTY_BYTES && e == cudaSuccess; off += NOVELTY_STAGE_BYTES, i++) {
+                const int k = (int)(i & 1);
+                unsigned char* pin = s->set_pin + k * NOVELTY_STAGE_BYTES;
+                if (s->stage_used[k] && (e = cudaEventSynchronize(s->ev_stage[k])) != cudaSuccess) break;
+                memcpy(pin, bitset + off, NOVELTY_STAGE_BYTES);
+                e = cudaMemcpyAsync(reinterpret_cast<unsigned char*>(target) + off, pin, NOVELTY_STAGE_BYTES,
+                                    cudaMemcpyHostToDevice, s->wstream);
+                if (e == cudaSuccess) e = cudaEventRecord(s->ev_stage[k], s->wstream);
+                s->stage_used[k] = true;
+            }
+        }
+        if (e == cudaSuccess) k_novelty_header<<<1, 1, 0, s->wstream>>>(s->set_hdr, (uint32_t)s->novelty, (uint32_t)s->n);
+    }
+    if (e != cudaSuccess) NN_FAIL(TZ_ECUDA, "set upload failed: %s", cudaGetErrorString(e));
+    int rc;
+    if ((rc = comm_broadcast(h, s->set_hdr, 4 * sizeof(uint32_t), root, s->wstream)) != TZ_OK ||
+        (rc = comm_broadcast(h, target, NOVELTY_BYTES, root, s->wstream)) != TZ_OK)
+        NN_FAIL(rc, "%s", comm_last_error());
+    if (rank != root) {
+        k_check_novelty<<<1, 1, 0, s->wstream>>>(s->set_hdr, (uint32_t)s->novelty, (uint32_t)s->n, h->d.status);
+        if (s->novelty) {
+            // the old set as it stands after the marks enqueued before this call
+            cudaStreamWaitEvent(s->wstream, s->ev_marks, 0);
+            k_keep_novelty<<<4 * s->sm_count, 256, 0, s->wstream>>>(s->set_hdr, reinterpret_cast<uint4*>(target),
+                                                                    reinterpret_cast<const uint4*>(s->simhash_set),
+                                                                    NOVELTY_BYTES / sizeof(uint4));
+        }
+    }
+    if (cudaGetLastError() != cudaSuccess) NN_FAIL(TZ_ECUDA, "set generation launch failed");
+    if (!search_waits_for_wstream(h)) NN_FAIL(TZ_ECUDA, "publishing the novelty set failed");
+    // a rank without a hash keeps having none (k_check_novelty raised the mismatch)
+    if (s->novelty) {
+        std::swap(s->simhash_set_alloc, s->set_spare);
+        s->simhash_set = s->simhash_set_alloc;
+    }
+    record_swap(h);
+    return TZ_OK;
 }

@@ -31,3 +31,11 @@ int nn_set_lcghash(tz_handle* h, const float* init, const unsigned char* bitset)
 int nn_lcghash_indices(tz_handle* h, const TzState* states, int count, uint32_t* out_dev);
 int nn_update_counts(tz_handle* h, const TzState* states_dev, int count, uint32_t* idx_dev);
 int nn_read_novelty_set(tz_handle* h, unsigned char* out_host);
+// 0 no hash yet, 1 SimHash, 2 LCG hash
+int nn_hash_kind(const tz_handle* h);
+// tz_update_counts_buffer: the examples of a validated training batch (explicit arrays already on the device)
+int nn_update_counts_buffer(tz_handle* h, const TzTargetRing& R, int batch, const unsigned long long* indices,
+                            const int* symmetry, int augment, unsigned long long seed, unsigned long long size,
+                            unsigned long long first);
+// tz_broadcast_novelty_set
+int nn_broadcast_novelty_set(tz_handle* h, const unsigned char* bitset, int root);

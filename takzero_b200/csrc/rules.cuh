@@ -392,3 +392,48 @@ __device__ __forceinline__ uint64_t warp_state_hash(const TzState* s, int nn, in
     for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(FULL_MASK, acc, o);
     return tz_mix64(acc + (0x9e3779b97f4a7c15ULL ^ (uint64_t)s->to_move));
 }
+
+// the library's counter-based generator (stated at tz_training_batch in the header)
+__device__ __forceinline__ uint64_t rng_hash(uint64_t seed, uint64_t a, uint64_t b, uint64_t c) {
+    uint64_t h = tz_mix64(seed ^ 0x9e3779b97f4a7c15ULL);
+    h = tz_mix64(h ^ (a * 0xbf58476d1ce4e5b9ULL));
+    h = tz_mix64(h ^ (b * 0x94d049bb133111ebULL));
+    return tz_mix64(h ^ (c * 0xd6e8feb86659fd93ULL));
+}
+
+// ---- board symmetries of the training batches (tz_training_batch, tz_update_counts_buffer) -----------
+
+// symmetry t of the board: bit 0 mirrors the column, bit 1 the row, bit 2 swaps them, in this order
+__device__ __forceinline__ void sym_square(int t, int n, int* row, int* col) {
+    if (t & 1) *col = n - 1 - *col;
+    if (t & 2) *row = n - 1 - *row;
+    if (t & 4) {
+        const int tmp = *col;
+        *col = *row;
+        *row = tmp;
+    }
+}
+
+// example b of a batch: target `index` (counted from the oldest kept one of `size`) under symmetry `t`, explicit or
+// drawn as the header states at tz_training_batch
+__device__ __forceinline__ void batch_example(const unsigned long long* indices, const int* symmetry, int augment,
+                                              unsigned long long seed, unsigned long long size, int b,
+                                              unsigned long long* index, int* t) {
+    *index = indices ? indices[b] : __umul64hi(rng_hash(seed, (uint64_t)b, 0, 0), size);
+    *t = symmetry ? symmetry[b] : augment ? (int)(rng_hash(seed, (uint64_t)b, 1, 0) & 7) : 0;
+}
+
+// dst = src under symmetry t (shared memory, one warp): the squares move, reserves, side to move and plies are kept
+__device__ __forceinline__ void warp_symmetric_state(TzState* dst, const TzState* src, int t, int n, int lane) {
+    warp_load_state(dst, src, lane);
+    const int nn = n * n;
+    for (int sq = lane; sq < nn; sq += 32) {
+        int row = sq / n, col = sq - row * n;
+        sym_square(t, n, &row, &col);
+        const int to = row * n + col;
+        dst->stack[to] = src->stack[sq];
+        dst->height[to] = src->height[sq];
+        dst->top[to] = src->top[sq];
+    }
+    __syncwarp();
+}

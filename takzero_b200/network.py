@@ -49,6 +49,7 @@ def _declare():
     capi.declare("tz_comm_init", [vp, vp, i32, i32], i32)
     capi.declare("tz_comm_destroy", [vp], i32)
     capi.declare("tz_broadcast_weights", [vp, C.POINTER(_Tensor), i32, i32, i32], i32)
+    capi.declare("tz_broadcast_novelty_set", [vp, vp, i32], i32)
     capi.declare("tz_weight_generation", [vp, C.POINTER(C.c_uint64), C.POINTER(C.c_double)], i32)
     capi.declare("tz_allreduce_sum", [vp, vp, i32], i32)
     capi.declare("tz_read_model_file", [C.c_char_p, _MODEL_TENSOR_FN, vp], i32)
@@ -93,6 +94,19 @@ def broadcast_weights(mcts: capi.BatchedMCTS, tensors: Dict[str, np.ndarray] | N
     else:
         arr, _keep = _tensor_array(tensors)
         capi._check(capi.lib().tz_broadcast_weights(mcts.handle, arr, len(tensors), res_blocks, root))
+
+
+def broadcast_novelty_set(mcts: capi.BatchedMCTS, bitset: np.ndarray | None = None, root: int = 0) -> None:
+    """One novelty-set generation on every rank of the handle's communicator (`tz_broadcast_novelty_set`,
+    collective): the root passes a `bitvec.bin` image (2^29 uint8; from capi.pinned_array it is uploaded in place and
+    must stay unchanged until mcts.sync()) or None for its own current set; the other ranks pass None.  Every rank
+    swaps to the new set for the launches it enqueues afterwards."""
+    _declare()
+    b = None
+    if bitset is not None:
+        b = np.ascontiguousarray(bitset, dtype=np.uint8)
+        assert b.size == 1 << 29
+    capi._check(capi.lib().tz_broadcast_novelty_set(mcts.handle, capi._ptr(b), root))
 
 
 def weight_generation(mcts: capi.BatchedMCTS):
